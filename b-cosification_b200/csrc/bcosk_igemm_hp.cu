@@ -658,13 +658,15 @@ bcosk_igemm_hp_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_c
                 sq_acc += maxout_fwd_tail<T, 8>(p, v, inv_norm, ri.m, yrow, cg, 8);
                 continue;
               }
+              // (the operation order of hp_fwd_fast wherever both forms apply: |lin| * (alpha * inv_norm), then the residual planes
+              //  added one at a time, so that the packed and the generic epilogue write the same bits)
               float t[8];
               const float4 a0 = *reinterpret_cast<const float4*>(s_alpha + jj * 32 + g * 8);
               const float4 a1 = *reinterpret_cast<const float4*>(s_alpha + jj * 32 + g * 8 + 4);
               const float al[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
               if (p.scale_mode == BCOSK_SCALE_B2) {
 #pragma unroll
-                for (int i = 0; i < 8; ++i) t[i] = fabsf(v[i]) * inv_norm * al[i];
+                for (int i = 0; i < 8; ++i) t[i] = fabsf(v[i]) * (al[i] * inv_norm);
               } else if (p.scale_mode == BCOSK_SCALE_POW) {
                 const float e = p.b_exp - 1.f;
 #pragma unroll
@@ -679,18 +681,13 @@ bcosk_igemm_hp_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_c
 #pragma unroll
               for (int i = 0; i < 8; ++i) v[i] = fmaf(v[i], t[i], be[i]);
               if (p.res != nullptr) {
-                float r[8];
-#pragma unroll
-                for (int i = 0; i < 8; ++i) r[i] = 0.f;
                 if (aux.in16_planes) {
-                  for (int pl = 0; pl < aux.in16_planes; ++pl) add8<T>(lds128(tile_ptr(r_in16 + pl * PLANE_BYTES, row, jj, g)), r);
+                  for (int pl = 0; pl < aux.in16_planes; ++pl) add8<T>(lds128(tile_ptr(r_in16 + pl * PLANE_BYTES, row, jj, g)), v);
                 } else {
                   const T* rp = reinterpret_cast<const T*>(p.res) + (size_t)ri.m * p.res_ld + cg;
                   for (int pl = 0; pl < p.res_planes; ++pl)
-                    add8<T>(__ldg(reinterpret_cast<const uint4*>(rp + (size_t)pl * p.res_plane_stride)), r);
+                    add8<T>(__ldg(reinterpret_cast<const uint4*>(rp + (size_t)pl * p.res_plane_stride)), v);
                 }
-#pragma unroll
-                for (int i = 0; i < 8; ++i) v[i] += r[i];
               }
               if (p.relu) {
 #pragma unroll
@@ -1044,7 +1041,8 @@ extern "C" int bcosk_set_hp_chunk(int32_t stages) {
 }
 
 extern "C" int bcosk_set_hp_boxes(int32_t enabled) {
-  const int prev = bcosk::g_hp_stage_boxes | (bcosk::g_hp_early_iters << 8);
+  // the previous setting in the encoding the argument uses (bits 8.. = 1 + threshold), so that passing it back restores it
+  const int prev = bcosk::g_hp_stage_boxes | ((bcosk::g_hp_early_iters + 1) << 8);
   bcosk::g_hp_stage_boxes = enabled & 7;        // bit 0: boxes, bit 1: generic arithmetic, bit 2: no paired stages
   if (enabled >> 8) bcosk::g_hp_early_iters = (enabled >> 8) - 1;   // bits 8..: 1 + K stages up to which input boxes are fetched early
   return prev;

@@ -188,11 +188,15 @@ int bcosk_igemm(const bcosk_igemm_params* p, void* stream);
 
 /* Parity-mode (hp_accum) launches: default for bcosk_igemm_params.hp_chunk == 0 (>= 1).  Returns the previous setting. */
 int bcosk_set_hp_chunk(int32_t stages);
-/* Parity-mode launches, A/B measurement switches (results are identical).  Bit 0 (default 1): epilogue tensors move as TMA
+/* Parity-mode launches, A/B measurement switches.  Bit 0 (default 1): epilogue tensors move as TMA
  * boxes through shared memory instead of per-row 16-byte accesses.  Bit 1 (default 0): the generic epilogue arithmetic runs
  * even where the packed two-plane form applies.  Bit 2 (default 0): no paired stages (every segment fetches its own A plane).
  * Bits 8..: when non-zero, 1 + the number of K stages up to which the input
- * boxes are fetched at kernel start (default 4) instead of after the last MMA.  Returns the previous setting. */
+ * boxes are fetched at kernel start (default 4) instead of after the last MMA.  Returns the previous setting in the same
+ * encoding (passing it back restores it).  Bits 0, 1 and 8.. leave y planes, gains and mask bits bit-identical (sums of squares
+ * are regrouped).  Bit 2 is not bit-identical: unpaired stages accumulate the cross terms in another order (a0 b1 over all of K,
+ * then a1 b0, instead of both per stage; with bf16 planes also in chunks), which moves the last bit of fp32 within the same error
+ * bound (tests/test_contract_gemm_fp64_gpu.py). */
 int bcosk_set_hp_boxes(int32_t enabled);
 
 /* Scheduling switch for A/B measurements: 1 = launches with block_n 64 (the bandwidth-bound ones) run on the persistent
