@@ -524,3 +524,32 @@ def agc_adamw(w, g, gidx, m, v, units, cols, grad_scale, lr, beta1, beta2, eps, 
     check(load().bcosk_agc_adamw(_p(w), _p(g), _p(gidx), _p(m), _p(v), units, cols, C.c_float(grad_scale), C.c_float(lr),
                                  C.c_float(beta1), C.c_float(beta2), C.c_float(eps), C.c_float(weight_decay), C.c_float(clip_factor),
                                  C.c_float(agc_eps), step, _stream()), "bcosk_agc_adamw")
+
+
+# ---- DenseNet fine-tuning step (csrc/bcosk_dense_train.cu)
+def dense_slice_stats(F, rows, ld, col0, c, eps, partials, mean, var, rstd, dtype) -> None:
+    """partials: [nblk, 2c] fp32 scratch; mean / var / rstd: the block's [C_total] arrays, channels [col0, col0 + c) written"""
+    check(load().bcosk_dense_slice_stats(_p(F), C.c_int64(rows), ld, col0, c, C.c_float(eps), _p(partials), partials.shape[0], _p(mean),
+                                         _p(var), _p(rstd), dtype, _stream()), "bcosk_dense_slice_stats")
+
+
+def dense_consumer_finalize(var, rstd, weight, c, momentum, running_var, alpha) -> None:
+    check(load().bcosk_dense_consumer_finalize(_p(var), _p(rstd), _p(weight), c, C.c_float(momentum), _p(running_var), _p(alpha), _stream()),
+          "bcosk_dense_consumer_finalize")
+
+
+def dense_consumer_bwd(g_t, t, gnt, alpha, F, ld, rows, c, G, accumulate, partials, dtype) -> None:
+    """partials: [nblk, c] fp32 (one row per launched block, summed in order by dense_consumer_bwd_finalize)"""
+    import torch
+    check(load().bcosk_dense_consumer_bwd(_p(g_t), int(g_t.dtype == torch.float32), _p(t), _p(gnt), _p(alpha), _p(F), ld, C.c_int64(rows), c,
+                                          _p(G), int(accumulate), _p(partials), partials.shape[0], dtype, _stream()), "bcosk_dense_consumer_bwd")
+
+
+def dense_consumer_bwd_finalize(partials, rstd, weight, rows, c, accumulate, K, g_weight) -> None:
+    check(load().bcosk_dense_consumer_bwd_finalize(_p(partials), partials.shape[0], _p(rstd), _p(weight), C.c_int64(rows), c, int(accumulate),
+                                                   _p(K), _p(g_weight), _stream()), "bcosk_dense_consumer_bwd_finalize")
+
+
+def dense_slice_bwd(G, F, ld, col0, rows, c, mean, K, scale, inv_norm, out, gnt, dtype) -> None:
+    check(load().bcosk_dense_slice_bwd(_p(G), _p(F), ld, col0, C.c_int64(rows), c, _p(mean), _p(K), _p(scale), _p(inv_norm), _p(out), _p(gnt),
+                                       dtype, _stream()), "bcosk_dense_slice_bwd")

@@ -20,7 +20,7 @@ LIB = os.path.join(PKG, "libbcosk.so")
 STAMP = os.path.join(PKG, ".libbcosk.stamp")
 
 SOURCES = ["bcosk_api.cu", "bcosk_igemm.cu", "bcosk_igemm_hp.cu", "bcosk_wgrad.cu", "bcosk_train.cu", "bcosk_elementwise.cu", "bcosk_layout.cu", "bcosk_tokens.cu",
-           "bcosk_rgba.cu", "bcosk_norms.cu", "bcosk_vit.cu", "bcosk_vit_attn.cu", "bcosk_dense.cu", "bcosk_head.cu"]
+           "bcosk_rgba.cu", "bcosk_norms.cu", "bcosk_vit.cu", "bcosk_vit_attn.cu", "bcosk_dense.cu", "bcosk_dense_train.cu", "bcosk_head.cu"]
 HEADERS = ["bcosk_common.cuh", "bcosk_host.h", "bcosk_igemm_epi.cuh", os.path.join(ROOT, "include", "bcosk.h")]
 OBJDIR = os.path.join(PKG, "build")
 

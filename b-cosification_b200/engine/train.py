@@ -1,5 +1,6 @@
-"""Fine-tuning step of a B-cosified ResNet (SURVEY 8f row 2, BASELINE config 5): forward in train mode, loss, full backward,
-gradient all-reduce, adaptive gradient clipping + AdamW - one process per GPU, batch sharded, NCCL for the gradients.
+"""Fine-tuning step of a B-cosified ResNet or DenseNet (SURVEY 8f row 2, BASELINE config 5): forward in train mode, loss, full
+backward, gradient all-reduce, adaptive gradient clipping + AdamW - one process per GPU, batch sharded, NCCL for the gradients.
+`ResNetTrainPlan` and `DenseNetTrainPlan` share `TrainPlanBase`; the DenseNet's own kernels are described at its class.
 
 Reference: `training_step` bcos/training/trainer.py:666-784 (outputs = model(images); loss = criterion(outputs, labels)),
 autograd backward through `BcosifyConv2d.forward_impl` (bcosifyconv2d.py:50-102, scale NOT detached) and
@@ -104,8 +105,10 @@ class TrainLayer:
     need_dgrad: bool = True
 
 
-class ResNetTrainPlan(PlanBase):
-    """One fine-tuning step of `BcosifyNetwork(ResNetBcos(...))` on `batch` images per rank."""
+class TrainPlanBase(PlanBase):
+    """What the fine-tuning plans share: fp32 master weights with refreshable packed operands, the flat gradient buffer in
+    backward order and its all-reduce buckets, the conv + batch-statistics BN emission and its backward, AGC + AdamW of the
+    whole model, CUDA-graph capture.  Subclasses emit the network (`_build`)."""
 
     parity_dgrad = True          # strided 3x3 data gradients as parity classes over the dense gradient
     flat_3x3 = False             # the flat-window variants keep their weights resident: not refreshable per step here
@@ -121,7 +124,6 @@ class ResNetTrainPlan(PlanBase):
                  world_size: int = 1, bucket_mb: float = 25.0, input_u8: bool = True, loss_scale: float = 1.0):
         super().__init__(batch, planes=1, dtype=dtype, device=device, explain=True, b=2.0, bn_eps=bn_eps, state_dict=state_dict)
         self.arch = arch
-        self.kind, self.nblocks = RESNET_ARCH[arch]
         self.size, self.input_u8 = image_size, input_u8
         self.mean, self.inv_std = tuple(mean), tuple(1.0 / s for s in std)
         self.logit_bias = 0.0 if logit_bias is None else float(logit_bias)
@@ -138,7 +140,10 @@ class ResNetTrainPlan(PlanBase):
         self.packs: List[Tuple[Tensor, Tensor]] = []          # (packed operand, int32 source index into w_flat)
         self._cur_w_off = 0
         self._w_items: List[Tuple[str, Tensor, int]] = []     # (state-dict key, fp32 tensor, offset)
+        self.norm_units: List[Tuple[int, int, int]] = []      # (master offset, gradient offset, c) of BN weights not owned by a TrainLayer
         self.opt_ops: List = []
+        self.running_var: Dict[str, Tensor] = {}
+        self.w_flat = None                    # allocated after all weights are registered (closures read self.w_flat late)
         self._build()
 
     # ------------------------------------------------------------------ master weights and packing
@@ -163,16 +168,20 @@ class ResNetTrainPlan(PlanBase):
     # ------------------------------------------------------------------ forward
     def _conv_bn(self, name: str, x: Act, wkey: str, stride: int, pad: int, bn: Optional[str], relu: bool, res: Optional[Tensor] = None,
                  w_standin: Optional[Tensor] = None, w_off: Optional[int] = None, w_numel: Optional[int] = None,
-                 pad_hi: Optional[int] = None, kch: int = 64, sq_geom=None, y_f32: bool = False, want_z_sq: bool = True) -> TrainLayer:
+                 pad_hi: Optional[int] = None, kch: int = 64, sq_geom=None, y_f32: bool = False, want_z_sq: bool = True,
+                 y_buf: Optional[Tensor] = None, y_col: int = 0) -> TrainLayer:
+        """Conv launch (+ batch-statistics BN `bn`, residual, ReLU).  `y_buf`: the conv writes columns [y_col, y_col + o) of that
+        wider tensor (a DenseNet feature tensor); `out` is then a strided view."""
         if w_standin is None:
             w_standin, w_off = self._register_weight(wkey)
             w_numel = w_standin.numel()
         self._pack_off = w_off
         y, rec = self._conv_fwd(name, x, w_standin, stride, pad, pad if pad_hi is None else pad_hi, bn=None, relu=False,
-                                want_sq=False, want_inv=True, kch=kch, sq_geom=sq_geom, y_f32=y_f32)
+                                want_sq=False, want_inv=True, kch=kch, sq_geom=sq_geom, y_f32=y_f32, y_buf=y_buf, y_col=y_col)
         fwd = self.fwd_ops[-1]
         M, o = fwd.M, fwd.n
-        lay = TrainLayer(name, rec, fwd, x, y.t.view(M, o), bn, relu, res=res, w_off=w_off, w_numel=w_numel)
+        out = y.t.view(M, o) if y_buf is None else y_buf.view(M, -1)[:, y_col:y_col + o]
+        lay = TrainLayer(name, rec, fwd, x, out, bn, relu, res=res, w_off=w_off, w_numel=w_numel)
         lay.gnT = self._empty(M, dtype=torch.float32)
         if bn is not None:
             f32 = dict(dtype=torch.float32)
@@ -197,11 +206,9 @@ class ResNetTrainPlan(PlanBase):
         self.layers.append(lay)
         return lay
 
-    def _build(self) -> None:
+    def _stem(self, conv_key: str, bn_key: str, pool_sq: bool) -> Act:
+        """Input prep, the stem conv + batch-statistics BN + ReLU, the 3x3/2 average pool; returns the pooled activation."""
         nb, S = self.nb, self.size
-        sd = self.sd
-        self.running_var: Dict[str, Tensor] = {}
-        self.w_flat = None                    # allocated after all weights are registered (closures read self.w_flat late)
         self.x_in = self._empty(nb, 3, S, S, dtype=torch.uint8) if self.input_u8 else self._empty(nb, 6, S, S, dtype=torch.float32)
         self.labels = self._zeros(nb, dtype=torch.int32)
         h2 = S // 2
@@ -211,41 +218,23 @@ class ResNetTrainPlan(PlanBase):
         self.fwd_ops.append(O.InputPrepOp("input_prep", self.x_in, self.mean, self.inv_std, a0, cp, 1, self.dt_code, sq0))
         # stem: the 7x7/2 conv as a 4x4/1 conv on the 2x2 space-to-depth input (engine/pack.py stem_s2d_weight); the stand-in goes
         # through the same linear map, so its operand elements point back at the 7x7 master weights
-        w7, off7 = self._register_weight("model.conv1.linear.weight")
+        w7, off7 = self._register_weight(conv_key)
         w4 = P.stem_s2d_weight(w7, cp)                                        # unmapped entries stay 0 -> index -1
-        stem = self._conv_bn("stem", Act(a0, cp, sq0, 1), "", 1, 2, "model.bn1", True, w_standin=w4, w_off=off7, w_numel=w7.numel(),
+        stem = self._conv_bn("stem", Act(a0, cp, sq0, 1), "", 1, 2, bn_key, True, w_standin=w4, w_off=off7, w_numel=w7.numel(),
                              pad_hi=1, kch=32, sq_geom=(S, S, 7, 2, 3), want_z_sq=False)
         stem.need_dgrad = False
         self.stem = stem
+        o = stem.fwd.n
         hp = (h2 + 2 - 3) // 2 + 1
-        p1 = self._empty(nb, hp, hp, 64)
-        sqp = self._empty(1, nb * hp * hp, dtype=torch.float32)
-        self.fwd_ops.append(O.AvgPoolFwdOp("pool", stem.z.t, 64, 1, 3, 2, 1, p1, self.dt_code, sqp))
-        self.pool_out = Act(p1, 64, sqp, 1)
-        x = self.pool_out
-        self.blocks: List[dict] = []
-        for li, (width, nblocks) in enumerate(zip([64, 128, 256, 512], self.nblocks), start=1):
-            for bi in range(nblocks):
-                stride = 2 if (li > 1 and bi == 0) else 1
-                pfx = f"model.layer{li}.{bi}"
-                ds = None
-                idn = x.t
-                if (pfx + ".downsample.0.linear.weight") in sd:
-                    ds = self._conv_bn(pfx + ".downsample", x, pfx + ".downsample.0.linear.weight", stride, 0, pfx + ".downsample.1", False,
-                                       want_z_sq=False)
-                    idn = ds.z.t
-                if self.kind == "basic":
-                    c1 = self._conv_bn(pfx + ".conv1", x, pfx + ".conv1.linear.weight", stride, 1, pfx + ".bn1", True)
-                    c2 = self._conv_bn(pfx + ".conv2", c1.z, pfx + ".conv2.linear.weight", 1, 1, pfx + ".bn2", True, res=idn)
-                    convs = [c1, c2]
-                else:
-                    c1 = self._conv_bn(pfx + ".conv1", x, pfx + ".conv1.linear.weight", 1, 0, pfx + ".bn1", True)
-                    c2 = self._conv_bn(pfx + ".conv2", c1.z, pfx + ".conv2.linear.weight", stride, 1, pfx + ".bn2", True)
-                    c3 = self._conv_bn(pfx + ".conv3", c2.z, pfx + ".conv3.linear.weight", 1, 0, pfx + ".bn3", True, res=idn)
-                    convs = [c1, c2, c3]
-                self.blocks.append(dict(name=pfx, convs=convs, ds=ds, x=x, y=convs[-1].z))
-                x = convs[-1].z
-        fc = self._conv_bn("fc", x, "model.fc.linear.weight", 1, 0, None, False, y_f32=True)
+        p1 = self._empty(nb, hp, hp, o)
+        sqp = self._empty(1, nb * hp * hp, dtype=torch.float32) if pool_sq else None
+        self.fwd_ops.append(O.AvgPoolFwdOp("pool", stem.z.t, o, 1, 3, 2, 1, p1, self.dt_code, sqp))
+        return Act(p1, o, sqp, 1)
+
+    def _head(self, name: str, x: Act, wkey: str) -> None:
+        """Classifier per position (fp32 output), global average + logit layer, UniformOffLabelsBCE and its gradient g_fc."""
+        nb = self.nb
+        fc = self._conv_bn(name, x, wkey, 1, 0, None, False, y_f32=True)
         self.fc = fc
         self.ncls = fc.fwd.n
         self.npix = x.hw[0] * x.hw[1]
@@ -258,21 +247,32 @@ class ResNetTrainPlan(PlanBase):
         self.fwd_ops.append(FnOp("loss.zero", self.loss.zero_))
         self.fwd_ops.append(FnOp("loss", lambda: L.bce_uniform_off(self.logits, self.labels, nb, self.ncls, off, self.inv_temp, self.npix, self.loss_scale,
                                                                   self.loss, self.g_fc, None, self.dt_code)))
-        # ---- flat fp32 master weights / optimizer state
-        n_w = self._cur_w_off
-        self.w_flat = self._empty(n_w, dtype=torch.float32)
-        for key, w, o in self._w_items:
-            self.w_flat[o:o + w.numel()].copy_(w.reshape(-1))
-        self.m_flat = self._zeros(n_w, dtype=torch.float32)
-        self.v_flat = self._zeros(n_w, dtype=torch.float32)
-        self._build_backward()
-        if self.device.type == "cuda":
-            self.refresh_operands()
 
     # ------------------------------------------------------------------ backward
+    def _alloc_grads(self, order: List) -> None:
+        """Gradient slots in backward order (`order`: TrainLayers, and norm records with `c` / `gbn_off` for BN weights that no
+        TrainLayer owns), the flat gradient buffer, its zeroing launch and the bucket state."""
+        g_off = 0
+        for lay in order:
+            if isinstance(lay, TrainLayer):
+                lay.g_off = g_off
+                g_off += lay.fwd.n * lay.fwd.ktot
+                if lay.bn is not None:
+                    lay.gbn_off = g_off
+                    g_off += lay.fwd.n
+            else:
+                lay.gbn_off = g_off
+                g_off += lay.c
+        self.g_flat = self._zeros(g_off, dtype=torch.float32)
+        self.buckets: List[Tuple[int, int]] = []
+        self._bucket_begin = self._bucket_end = 0
+        self.comm_stream = torch.cuda.Stream(self.device) if self.device.type == "cuda" else None
+        self.bwd_ops.append(FnOp("grad.zero", self.g_flat.zero_))
+
     def _layer_bwd(self, lay: TrainLayer, ga: Tensor, gb: Optional[Tensor], tn: Optional[Tensor], ga_f32: bool = False,
-                   want_gy: bool = False) -> Optional[Tensor]:
-        """Emit: norm / ReLU / B-cos backward of `lay`, its weight gradient, its data gradient, its patch-norm vector."""
+                   want_gy: bool = False, gx32: Optional[Tensor] = None) -> Optional[Tensor]:
+        """Emit: norm / ReLU / B-cos backward of `lay`, its weight gradient, its data gradient, its patch-norm vector.
+        `gx32`: the data gradient goes to this fp32 buffer instead of a fresh 16-bit one."""
         M, o = lay.out.shape
         dtc = self.dt_code
         relu = lay.relu
@@ -289,12 +289,23 @@ class ResNetTrainPlan(PlanBase):
         self.bwd_ops.append(FnOp(lay.name + ".bwd.apply", lambda: L.train_bwd_apply(
             ga, ga_f32, gb, xpost, tn, relu, lay.out, out_f32, lay.rec.gain, lay.alpha, lay.kcoef, lay.mean, lay.rec.inv, M, o, glin, lay.gnT,
             gy, dtc)))
+        self._wgrad_dgrad(lay, glin, gx32)
+        return gy
+
+    def _wgrad_dgrad(self, lay: TrainLayer, glin: Tensor, gx32: Optional[Tensor] = None) -> None:
+        """Weight gradient of `lay` from g_lin (into its slot of the flat buffer), then its data gradient."""
+        o = lay.fwd.n
         self.bwd_ops.append(WgradOp(lay.name + ".wgrad", lay.fwd, glin, self.g_flat[lay.g_off:lay.g_off + o * lay.fwd.ktot]))
         self._grad_ready(lay)
         if lay.need_dgrad:
             self._pack_off = lay.w_off
             h, w = lay.rec.in_hw
             cin = lay.rec.cin_phys
+            if gx32 is not None:
+                assert lay.rec.stride == 1 and lay.rec.k == 1
+                lay.gx = gx32
+                self._dgrad(lay.rec, y=gx32, y_f32=True)
+                return
             lay.gx = self._zeros(self.nb, h, w, cin)
             if lay.rec.stride > 1 and lay.rec.k == 1:
                 # strided 1x1: the dense GEMM at output resolution lands on the sampled pixels of a zeroed full-resolution tensor
@@ -302,7 +313,6 @@ class ResNetTrainPlan(PlanBase):
                 self._dgrad(lay.rec, y=lay.gx, y_map=(0, h * w, s * w, s))
             else:
                 self._dgrad(lay.rec, y=lay.gx)
-        return gy
 
     def _norm_path(self, lay: TrainLayer, tn: Tensor, accumulate: bool) -> None:
         """tn[input pixel] (+)= sum of lay.gnT over the windows that cover it (d ||patch|| / d x = x / ||patch||)."""
@@ -312,10 +322,13 @@ class ResNetTrainPlan(PlanBase):
         self.bwd_ops.append(FnOp(lay.name + ".normpath", lambda: L.sumpool_transpose(lay.gnT, self.nb, h, w, k, s, pad, oh, ow, accumulate, tn)))
 
     def _grad_ready(self, lay: TrainLayer) -> None:
-        """Bucketed all-reduce: once the gradients up to this layer (backward order) fill a bucket, a side stream reduces it."""
         end = lay.g_off + lay.fwd.n * lay.fwd.ktot
         if lay.gbn_off >= 0:
             end = max(end, lay.gbn_off + lay.fwd.n)
+        self._grad_ready_to(end)
+
+    def _grad_ready_to(self, end: int) -> None:
+        """Bucketed all-reduce: once the gradients up to `end` (backward order) fill a bucket, a side stream reduces it."""
         self._bucket_end = max(self._bucket_end, end)
         if (self._bucket_end - self._bucket_begin) * 4 >= self.bucket_bytes:
             self._close_bucket()
@@ -342,58 +355,16 @@ class ResNetTrainPlan(PlanBase):
             self.comm_stream.wait_event(ev)
             dist.all_reduce(self.g_flat[a:b])
 
-    def _build_backward(self) -> None:
-        nb = self.nb
-        # gradient buffer in BACKWARD order: classifier first, stem last, so that finished buckets are contiguous
-        order = [self.fc]
-        for blk in reversed(self.blocks):
-            order += list(reversed(blk["convs"]))
-            if blk["ds"] is not None:
-                order.append(blk["ds"])
-        order.append(self.stem)
-        g_off = 0
-        for lay in order:
-            lay.g_off = g_off
-            g_off += lay.fwd.n * lay.fwd.ktot
-            if lay.bn is not None:
-                lay.gbn_off = g_off
-                g_off += lay.fwd.n
-        self.g_flat = self._zeros(g_off, dtype=torch.float32)
-        self.buckets: List[Tuple[int, int]] = []
-        self._bucket_begin = self._bucket_end = 0
-        self.comm_stream = torch.cuda.Stream(self.device) if self.device.type == "cuda" else None
-        self.bwd_ops.append(FnOp("grad.zero", self.g_flat.zero_))
-        # ---- classifier
-        self._layer_bwd(self.fc, self.g_fc, None, None)
-        ga, gb = self.fc.gx.view(-1, self.fc.rec.cin_phys), None
-        tn = self.fc.gnT                                # 1x1 stride 1: the patch-norm vector is gnT itself
-        # ---- blocks in reverse
-        for bi in range(len(self.blocks) - 1, -1, -1):
-            blk = self.blocks[bi]
-            convs, ds = blk["convs"], blk["ds"]
-            last = convs[-1]
-            gy = self._layer_bwd(last, ga, gb, tn, want_gy=True)          # g_y also flows into the identity / downsample branch
-            for j in range(len(convs) - 2, -1, -1):
-                nxt, cur = convs[j + 1], convs[j]
-                t_in = self._norm_vec(nxt)
-                self._layer_bwd(cur, nxt.gx.view(-1, nxt.rec.cin_phys), None, t_in)
-            first = convs[0]
-            t_blk = self._norm_vec(first)
-            if ds is not None:
-                self._layer_bwd(ds, gy, None, None)
-                self._norm_path(ds, t_blk, accumulate=True)
-                gb = ds.gx.view(-1, ds.rec.cin_phys)
-            else:
-                gb = gy
-            ga, tn = first.gx.view(-1, first.rec.cin_phys), t_blk
-        # ---- pooled stem: g = ga + gb + x_pool * T, average-pool backward, stem layer
-        M_pool = self.pool_out.t.shape[0] * self.pool_out.t.shape[1] * self.pool_out.t.shape[2]
-        g_pool = self._empty(*self.pool_out.t.shape)
-        self.bwd_ops.append(FnOp("pool.grad", lambda: L.grad_combine(ga, gb, self.pool_out.t, tn, M_pool, 64, g_pool, self.dt_code)))
-        g_stem = self._empty(*self.stem.z.t.shape)
-        self.bwd_ops.append(O.AvgPoolBwdMulOp("pool.bwd", g_pool, 64, 1, 3, 2, 1, None, g_stem, self.dt_code))
-        self._layer_bwd(self.stem, g_stem.view(-1, 64), None, None)
-        self._close_bucket()
+    def _alloc_master(self) -> None:
+        """flat fp32 master weights / optimizer state"""
+        n_w = self._cur_w_off
+        self.w_flat = self._empty(n_w, dtype=torch.float32)
+        for key, w, o in self._w_items:
+            self.w_flat[o:o + w.numel()].copy_(w.reshape(-1))
+        self.m_flat = self._zeros(n_w, dtype=torch.float32)
+        self.v_flat = self._zeros(n_w, dtype=torch.float32)
+
+    def _build_optimizer(self) -> None:
         # ---- optimizer: gradient index of every master element (the weight-gradient kernel writes the packed layout)
         gidx = torch.full((self._cur_w_off,), -1, dtype=torch.int64)
         for lay in self.layers:
@@ -404,6 +375,8 @@ class ResNetTrainPlan(PlanBase):
             if lay.bn is not None:
                 o = lay.fwd.n
                 gidx[lay.bnw_off:lay.bnw_off + o] = lay.gbn_off + torch.arange(o)
+        for w_off, g_off, c in self.norm_units:
+            gidx[w_off:w_off + c] = g_off + torch.arange(c)
         assert int((gidx < 0).sum()) == 0, "a master weight without a gradient slot"
         self.gidx = gidx.to(torch.int32).to(self.device)
         # ---- AGC + AdamW of the WHOLE model in one launch: one unit = one output row of a conv / the whole BN weight vector
@@ -417,6 +390,9 @@ class ResNetTrainPlan(PlanBase):
             if lay.bn is not None:
                 u_off.append(lay.bnw_off)
                 u_cols.append(o)
+        for w_off, _, c in self.norm_units:
+            u_off.append(w_off)
+            u_cols.append(c)
         self.unit_off = torch.tensor(u_off, dtype=torch.int64, device=self.device)
         self.unit_cols = torch.tensor(u_cols, dtype=torch.int32, device=self.device)
         self.adam_state = self._zeros(3, dtype=torch.float32)          # {step, 1 - beta1^step, 1 - beta2^step}
@@ -552,3 +528,285 @@ class ResNetTrainPlan(PlanBase):
         """2*MAC of forward + data gradient + weight gradient (the data gradient of the stem is not needed)."""
         f = sum(l.fwd.algo_flops for l in self.layers)
         return 3.0 * f - self.stem.fwd.algo_flops
+
+
+class ResNetTrainPlan(TrainPlanBase):
+    """One fine-tuning step of `BcosifyNetwork(ResNetBcos(...))` on `batch` images per rank."""
+
+    def __init__(self, arch: str, state_dict: Dict[str, Tensor], batch: int, **kw):
+        self.kind, self.nblocks = RESNET_ARCH[arch]
+        super().__init__(arch, state_dict, batch, **kw)
+
+    def _build(self) -> None:
+        sd = self.sd
+        self.pool_out = self._stem("model.conv1.linear.weight", "model.bn1", pool_sq=True)
+        x = self.pool_out
+        self.blocks: List[dict] = []
+        for li, (width, nblocks) in enumerate(zip([64, 128, 256, 512], self.nblocks), start=1):
+            for bi in range(nblocks):
+                stride = 2 if (li > 1 and bi == 0) else 1
+                pfx = f"model.layer{li}.{bi}"
+                ds = None
+                idn = x.t
+                if (pfx + ".downsample.0.linear.weight") in sd:
+                    ds = self._conv_bn(pfx + ".downsample", x, pfx + ".downsample.0.linear.weight", stride, 0, pfx + ".downsample.1", False,
+                                       want_z_sq=False)
+                    idn = ds.z.t
+                if self.kind == "basic":
+                    c1 = self._conv_bn(pfx + ".conv1", x, pfx + ".conv1.linear.weight", stride, 1, pfx + ".bn1", True)
+                    c2 = self._conv_bn(pfx + ".conv2", c1.z, pfx + ".conv2.linear.weight", 1, 1, pfx + ".bn2", True, res=idn)
+                    convs = [c1, c2]
+                else:
+                    c1 = self._conv_bn(pfx + ".conv1", x, pfx + ".conv1.linear.weight", 1, 0, pfx + ".bn1", True)
+                    c2 = self._conv_bn(pfx + ".conv2", c1.z, pfx + ".conv2.linear.weight", stride, 1, pfx + ".bn2", True)
+                    c3 = self._conv_bn(pfx + ".conv3", c2.z, pfx + ".conv3.linear.weight", 1, 0, pfx + ".bn3", True, res=idn)
+                    convs = [c1, c2, c3]
+                self.blocks.append(dict(name=pfx, convs=convs, ds=ds, x=x, y=convs[-1].z))
+                x = convs[-1].z
+        self._head("fc", x, "model.fc.linear.weight")
+        self._alloc_master()
+        self._build_backward()
+        if self.device.type == "cuda":
+            self.refresh_operands()
+
+    def _build_backward(self) -> None:
+        # gradient buffer in BACKWARD order: classifier first, stem last, so that finished buckets are contiguous
+        order = [self.fc]
+        for blk in reversed(self.blocks):
+            order += list(reversed(blk["convs"]))
+            if blk["ds"] is not None:
+                order.append(blk["ds"])
+        order.append(self.stem)
+        self._alloc_grads(order)
+        # ---- classifier
+        self._layer_bwd(self.fc, self.g_fc, None, None)
+        ga, gb = self.fc.gx.view(-1, self.fc.rec.cin_phys), None
+        tn = self.fc.gnT                                # 1x1 stride 1: the patch-norm vector is gnT itself
+        # ---- blocks in reverse
+        for bi in range(len(self.blocks) - 1, -1, -1):
+            blk = self.blocks[bi]
+            convs, ds = blk["convs"], blk["ds"]
+            last = convs[-1]
+            gy = self._layer_bwd(last, ga, gb, tn, want_gy=True)          # g_y also flows into the identity / downsample branch
+            for j in range(len(convs) - 2, -1, -1):
+                nxt, cur = convs[j + 1], convs[j]
+                t_in = self._norm_vec(nxt)
+                self._layer_bwd(cur, nxt.gx.view(-1, nxt.rec.cin_phys), None, t_in)
+            first = convs[0]
+            t_blk = self._norm_vec(first)
+            if ds is not None:
+                self._layer_bwd(ds, gy, None, None)
+                self._norm_path(ds, t_blk, accumulate=True)
+                gb = ds.gx.view(-1, ds.rec.cin_phys)
+            else:
+                gb = gy
+            ga, tn = first.gx.view(-1, first.rec.cin_phys), t_blk
+        # ---- pooled stem: g = ga + gb + x_pool * T, average-pool backward, stem layer
+        M_pool = self.pool_out.t.shape[0] * self.pool_out.t.shape[1] * self.pool_out.t.shape[2]
+        g_pool = self._empty(*self.pool_out.t.shape)
+        self.bwd_ops.append(FnOp("pool.grad", lambda: L.grad_combine(ga, gb, self.pool_out.t, tn, M_pool, 64, g_pool, self.dt_code)))
+        g_stem = self._empty(*self.stem.z.t.shape)
+        self.bwd_ops.append(O.AvgPoolBwdMulOp("pool.bwd", g_pool, 64, 1, 3, 2, 1, None, g_stem, self.dt_code))
+        self._layer_bwd(self.stem, g_stem.view(-1, 64), None, None)
+        self._close_bucket()
+        self._build_optimizer()
+
+
+@dataclass
+class DenseNorm:
+    """A consumer's batch-statistics BN + ReLU over the prefix F[:, :c] of a dense block's feature tensor (dense-layer norm1, a
+    transition's norm, norm5).  Its statistics are the block's per-channel ones; it owns alpha, its running_var and its BN weight."""
+    name: str
+    blk: "DenseTrainBlock"
+    c: int
+    t: Act                                   # relu(F[:, :c] * alpha), the input of the 1x1 conv that follows
+    alpha: Tensor
+    bnw_off: int
+    gbn_off: int = -1
+    conv: Optional[TrainLayer] = None        # the 1x1 B-cos conv that reads t (its gnT is the patch-norm path of t)
+
+
+@dataclass
+class DenseTrainBlock:
+    name: str
+    F: Tensor                                # [nb, h, w, c_total] 16-bit feature tensor
+    c_total: int
+    c_in: int
+    M: int
+    mean: Tensor                             # [c_total] fp32 batch statistics of every channel of F
+    var: Tensor
+    rstd: Tensor
+    K: Tensor                                # [c_total] fp32: sum over the consumers of their batch-statistics coefficients k_l
+    G: Tensor                                # [M, c_total] fp32 gradient wrt F (the consumers' direct terms)
+    layers: List[Tuple[DenseNorm, TrainLayer, TrainLayer]] = field(default_factory=list)     # (norm1, conv1, conv2)
+    t_norm: Optional[DenseNorm] = None       # transition behind the block
+    t_conv: Optional[TrainLayer] = None
+
+
+class DenseNetTrainPlan(TrainPlanBase):
+    """One fine-tuning step of `BcosifyNetwork(DenseNetBcos(...))` (DenseNet-121 / -169 / -201) on `batch` images per rank.
+
+    Same launches as the ResNet plan for the stem, the convs (+ norm2 of every dense layer) and the head.  What is DenseNet's own is
+    the batch-statistics BN + ReLU every consumer applies to a prefix of its block's feature tensor F (csrc/bcosk_dense_train.cu):
+      forward   dense_slice_stats after the block-input copy and after every 3x3 launch (statistics of a channel do not depend on the
+                consumer: computed once), then per consumer dense_consumer_finalize -> dense_bn_relu_fwd -> its 1x1 conv
+      backward  per consumer ONE pass dense_consumer_bwd (G[:, :C_l] += g_y alpha_l, S_l) + finalize (BN weight gradient, K += k_l);
+                the batch-statistics terms of all consumers, (F - mean) K, are applied once by dense_slice_bwd when the slice's
+                producer (a 3x3 conv, or the block input) runs its backward."""
+
+    def __init__(self, arch: str, state_dict: Dict[str, Tensor], batch: int, **kw):
+        from .densenet import DENSENET_ARCH
+        self.growth, self.block_cfg, self.init_c = DENSENET_ARCH[arch]
+        super().__init__(arch, state_dict, batch, **kw)
+
+    # ------------------------------------------------------------------ forward
+    def _slice_stats(self, blk: DenseTrainBlock, col0: int, c: int, name: str) -> None:
+        part = self.stat_part[:self.red_blocks * 2 * c].view(self.red_blocks, 2 * c)
+        self.fwd_ops.append(FnOp(name, lambda: L.dense_slice_stats(blk.F, blk.M, blk.c_total, col0, c, self.bn_eps, part, blk.mean, blk.var,
+                                                                    blk.rstd, self.dt_code)))
+
+    def _consumer(self, bn: str, blk: DenseTrainBlock, c: int) -> DenseNorm:
+        nb = self.nb
+        h, w = blk.F.shape[1], blk.F.shape[2]
+        alpha = self._empty(c, dtype=torch.float32)
+        off = self._cur_w_off
+        self._w_items.append((bn + ".weight", self.sd[bn + ".weight"], off))
+        self._cur_w_off += c
+        rv = self._dev(self.sd[bn + ".running_var"])
+        self.running_var[bn] = rv
+        self.fwd_ops.append(FnOp(bn + ".finalize", lambda: L.dense_consumer_finalize(blk.var, blk.rstd, self.w_flat[off:off + c], c, self.momentum,
+                                                                                     rv, alpha)))
+        t = self._empty(nb, h, w, c)
+        sq = self._empty(1, nb * h * w, dtype=torch.float32)
+        self.fwd_ops.append(O.DenseBnReluFwdOp(bn + ".apply", blk.F, c, 1, alpha, True, t, sq, None, self.dt_code))
+        return DenseNorm(bn, blk, c, Act(t, c, sq, 1), alpha, off)
+
+    def _build(self) -> None:
+        from .densenet import dn_names
+        nb = self.nb
+        nm = dn_names(len(self.block_cfg))
+        f32 = dict(dtype=torch.float32)
+        pooled = self._stem(nm["conv0"] + ".linear.weight", nm["norm0"], pool_sq=False).t
+        hw = (pooled.shape[1], pooled.shape[2])
+        c = self.init_c
+        # per-block partial sums, shared by the launches (one stream): statistics [blocks][2 c], consumer reductions [blocks][c]
+        c_max = max(ci + self.growth * n for ci, n in zip(self._block_inputs(), self.block_cfg))
+        self.stat_part = self._empty(self.red_blocks * 2 * c_max, **f32)
+        self.cons_part = self._empty(self.red_blocks * c_max, **f32)
+        self.blocks: List[DenseTrainBlock] = []
+        self.norms: List[DenseNorm] = []
+        for bi, nlayers in enumerate(self.block_cfg, start=1):
+            c_total = c + self.growth * nlayers
+            M = nb * hw[0] * hw[1]
+            F = self._zeros(nb, hw[0], hw[1], c_total)
+            blk = DenseTrainBlock(f"denseblock{bi}", F, c_total, c, M, *(self._zeros(c_total, **f32) for _ in range(4)),
+                                  G=self._empty(M, c_total, **f32))
+            self.blocks.append(blk)
+            self.fwd_ops.append(O.CopyChannelsOp(f"denseblock{bi}.input", pooled, c, 1, F, 0))
+            self._slice_stats(blk, 0, c, f"denseblock{bi}.input.stats")
+            cl = c
+            for li in range(1, nlayers + 1):
+                p = nm[f"denseblock{bi}"] + f".denselayer{li}"
+                n1 = self._consumer(p + ".norm1", blk, cl)
+                c1 = self._conv_bn(p + ".conv1", n1.t, p + ".conv1.linear.weight", 1, 0, p + ".norm2", True)
+                n1.conv = c1
+                c2 = self._conv_bn(p + ".conv2", c1.z, p + ".conv2.linear.weight", 1, 1, None, False, y_buf=F, y_col=cl)
+                self._slice_stats(blk, cl, self.growth, p + ".conv2.stats")
+                blk.layers.append((n1, c1, c2))
+                self.norms.append(n1)
+                cl += self.growth
+            c = c_total
+            if bi != len(self.block_cfg):
+                tn = self._consumer(nm[f"transition{bi}.norm"], blk, c)
+                tc = self._conv_bn(nm[f"transition{bi}.conv"], tn.t, nm[f"transition{bi}.conv"] + ".linear.weight", 1, 0, None, False)
+                tn.conv = tc
+                blk.t_norm, blk.t_conv = tn, tc
+                self.norms.append(tn)
+                c //= 2
+                y = tc.out.view(nb, hw[0], hw[1], c)
+                hw = (hw[0] // 2, hw[1] // 2)
+                pooled = self._empty(nb, hw[0], hw[1], c)
+                self.fwd_ops.append(O.AvgPoolFwdOp(f"transition{bi}.pool", y, c, 1, 2, 2, 0, pooled, self.dt_code, None))
+        n5 = self._consumer(nm["norm5"], self.blocks[-1], c)
+        self.norms.append(n5)
+        self.norm5 = n5
+        self._head("classifier", n5.t, "model.classifier.linear.weight")
+        n5.conv = self.fc
+        self._alloc_master()
+        self._build_backward()
+        if self.device.type == "cuda":
+            self.refresh_operands()
+
+    def _block_inputs(self) -> List[int]:
+        c, out = self.init_c, []
+        for bi, n in enumerate(self.block_cfg):
+            out.append(c)
+            c = (c + self.growth * n) // 2
+        return out
+
+    # ------------------------------------------------------------------ backward
+    def _consumer_bwd(self, n: DenseNorm, accumulate: bool) -> None:
+        """g_t (the consumer conv's fp32 data gradient) -> G[:, :c] and the partials of S, then the BN weight gradient and K += k."""
+        blk, c, M, dtc = n.blk, n.c, n.blk.M, self.dt_code
+        g_t = n.conv.gx.view(M, c)
+        part = self.cons_part[:self.red_blocks * c].view(self.red_blocks, c)
+        self.bwd_ops.append(FnOp(n.name + ".bwd", lambda: L.dense_consumer_bwd(g_t, n.t.t, n.conv.gnT, n.alpha, blk.F, blk.c_total, M, c, blk.G,
+                                                                             accumulate, part, dtc)))
+        self.bwd_ops.append(FnOp(n.name + ".bwd.finalize", lambda: L.dense_consumer_bwd_finalize(
+            part, blk.rstd, self.w_flat[n.bnw_off:n.bnw_off + c], M, c, accumulate, blk.K, self.g_flat[n.gbn_off:n.gbn_off + c])))
+        self._grad_ready_to(n.gbn_off + c)
+
+    def _consumer_conv_bwd(self, lay: TrainLayer, ga: Tensor, n: DenseNorm, scratch: Tensor, accumulate: bool) -> None:
+        """A consumer's 1x1 conv without a norm behind it (transition, classifier): B-cos backward, weight gradient, fp32 data
+        gradient into `scratch`, then the consumer's own backward."""
+        self._layer_bwd(lay, ga, None, None, gx32=scratch[:n.blk.M * n.c].view(self.nb, *n.t.hw, n.c))
+        self._consumer_bwd(n, accumulate)
+
+    def _build_backward(self) -> None:
+        nb, dtc = self.nb, self.dt_code
+        order: List = [self.fc, self.norm5]
+        for blk in reversed(self.blocks):
+            for n1, c1, c2 in reversed(blk.layers):
+                order += [c2, c1, n1]
+            prev = self.blocks.index(blk) - 1
+            if prev >= 0:
+                order += [self.blocks[prev].t_conv, self.blocks[prev].t_norm]
+        order.append(self.stem)
+        self._alloc_grads(order)
+        self.norm_units = [(n.bnw_off, n.gbn_off, n.c) for n in self.norms]
+        scratch = self._empty(max(b.M * b.c_total for b in self.blocks), dtype=torch.float32)   # fp32 data gradients of the 1x1 convs
+        # ---- head: classifier, then norm5 (the first consumer of the last block: it writes G and K)
+        self._consumer_conv_bwd(self.fc, self.g_fc, self.norm5, scratch, accumulate=False)
+        for bi in range(len(self.blocks) - 1, -1, -1):
+            blk = self.blocks[bi]
+            M = blk.M
+            for n1, c1, c2 in reversed(blk.layers):
+                # 3x3 slice: g_out = G + (F - mean) K -> g_lin, gnT; weight and data gradient
+                self._alloc_ghat(c2.rec, classes=True)
+                glin = c2.rec.ghat.view(M, self.growth)
+                col = n1.c
+                self.bwd_ops.append(FnOp(c2.name + ".bwd.slice", lambda blk=blk, c2=c2, glin=glin, col=col: L.dense_slice_bwd(
+                    blk.G, blk.F, blk.c_total, col, blk.M, self.growth, blk.mean, blk.K, c2.rec.gain, c2.rec.inv, glin, c2.gnT, dtc)))
+                self._wgrad_dgrad(c2, glin)
+                # conv1 + norm2 (+ ReLU) with the 3x3's patch-norm path, its data gradient in fp32, then norm1's one pass
+                self._layer_bwd(c1, c2.gx.view(-1, c2.rec.cin_phys), None, self._norm_vec(c2),
+                                gx32=scratch[:M * n1.c].view(nb, *n1.t.hw, n1.c))
+                self._consumer_bwd(n1, accumulate=True)
+            # ---- the block's input channels: g = G[:, :c_in] + (F - mean) K, through the pool in front of the block
+            g_in = self._empty(nb, *blk.F.shape[1:3], blk.c_in)
+            self.bwd_ops.append(FnOp(blk.name + ".input.bwd", lambda blk=blk, g_in=g_in: L.dense_slice_bwd(
+                blk.G, blk.F, blk.c_total, 0, blk.M, blk.c_in, blk.mean, blk.K, None, None, g_in, None, dtc)))
+            if bi > 0:
+                prev = self.blocks[bi - 1]
+                tc = prev.t_conv
+                g_y = self._empty(*tc.out.shape)
+                h, w = prev.F.shape[1], prev.F.shape[2]
+                self.bwd_ops.append(O.AvgPoolBwdMulOp(f"transition{bi}.pool.bwd", g_in, blk.c_in, 1, 2, 2, 0, None, g_y.view(nb, h, w, blk.c_in),
+                                                      dtc))
+                self._consumer_conv_bwd(tc, g_y, prev.t_norm, scratch, accumulate=False)
+            else:
+                g_stem = self._empty(*self.stem.z.t.shape)
+                self.bwd_ops.append(O.AvgPoolBwdMulOp("pool.bwd", g_in, blk.c_in, 1, 3, 2, 1, None, g_stem, dtc))
+                self._layer_bwd(self.stem, g_stem.view(-1, blk.c_in), None, None)
+        self._close_bucket()
+        self._build_optimizer()

@@ -505,6 +505,34 @@ int bcosk_dense_slice_cast(const float* G, int32_t g_ld, int32_t col0, int64_t r
 int bcosk_copy_rows_2d(void* dst, int64_t dst_pitch_bytes, const void* src, int64_t src_pitch_bytes, int64_t width_bytes,
                        int64_t rows, void* stream);
 
+/* DenseNet fine-tuning step (engine/train.py DenseNetTrainPlan, csrc/bcosk_dense_train.cu).  In train mode consumer l normalises
+ * F[:, :C_l] with the batch statistics of those channels, which do not depend on the consumer: they are computed ONCE per slice
+ * of F, when the slice is written.  In the backward pass consumer l's batch-statistics term for channel c is
+ * (F[:, c] - mean[c]) * k_l[c], k_l = -rstd^3 w_l S_l / rows, S_l[c] = sum_m g_y * F: linear in (F - mean), so the block keeps
+ * ONE accumulator K = sum_l k_l, applied when the producer of the slice runs its backward (all consumers of a slice run before
+ * it in reverse order).  16-bit rows of `dtype`, fp32 arithmetic; every reduction is a fixed-order sum of per-block partials
+ * (no atomics: bit-reproducible).  F / G rows have pitch ld (= C_total) elements; c <= 2048, c % 8 == 0, col0 % 8 == 0.
+ * slice_stats:  mean / var (centred, biased) / rstd = 1/sqrt(var + eps) of F[:, col0 : col0 + c] -> mean, var, rstd [col0 ..
+ *               col0 + c) (arrays of the whole block); partials [nblk][2c] fp32 scratch.
+ * consumer_finalize:  alpha[:c] = weight * rstd;  running_var[:c] = (1 - momentum) running_var + momentum var  (this consumer's buffer).
+ * consumer_bwd (one pass over the prefix; the consumer is a 1x1 B-cos conv, so its patch-norm vector is its own gnt):
+ *               g_y = (g_t + t * gnt[row]) * [t > 0];  G[:, :c] = (accumulate ? G[:, :c] : 0) + g_y * alpha;
+ *               partials[b][c] = sum over block b's rows of g_y * F      (g_t fp32 or 16-bit [rows][c], t 16-bit [rows][c])
+ * consumer_bwd_finalize:  S = sum_b partials[b];  g_weight = S * rstd;  K[:c] = (accumulate ? K[:c] : 0) + k_l.
+ * slice_bwd:    g_out = G[:, slice] + (F[:, slice] - mean) * K.  scale != NULL (the slice is a B-cos conv's output F = lin |lin| / n,
+ *               scale = |lin| / n [rows][c]): out = 2 * scale * g_out and gnt[row] = -sum_c g_out * F * inv_norm[row]^2;
+ *               scale == NULL (a block's input channels): out = g_out.  out [rows][c] dense 16-bit. */
+int bcosk_dense_slice_stats(const void* F, int64_t rows, int32_t ld, int32_t col0, int32_t c, float eps, float* partials, int32_t nblk,
+                            float* mean, float* var, float* rstd, int32_t dtype, void* stream);
+int bcosk_dense_consumer_finalize(const float* var, const float* rstd, const float* weight, int32_t c, float momentum, float* running_var,
+                                  float* alpha, void* stream);
+int bcosk_dense_consumer_bwd(const void* g_t, int32_t g_t_f32, const void* t, const float* gnt, const float* alpha, const void* F, int32_t ld,
+                             int64_t rows, int32_t c, float* G, int32_t accumulate, float* partials, int32_t nblk, int32_t dtype, void* stream);
+int bcosk_dense_consumer_bwd_finalize(const float* partials, int32_t nblk, const float* rstd, const float* weight, int64_t rows, int32_t c,
+                                      int32_t accumulate, float* K, float* g_weight, void* stream);
+int bcosk_dense_slice_bwd(const float* G, const void* F, int32_t ld, int32_t col0, int64_t rows, int32_t c, const float* mean, const float* K,
+                          const void* scale, const float* inv_norm, void* out, float* gnt, int32_t dtype, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Attention-pool head of the CLIP ResNet encoders inside the fused plan (BcosAttentionPool2d.forward bcosattnpool.py:34-59, pooled
  * mode; csrc/bcosk_head.cu).  Only the mean token's output is kept, so projections commute with the pooling: scores

@@ -1,30 +1,35 @@
-"""2+ ranks (torchrun): the bucketed NCCL all-reduce inside ResNetTrainPlan gives the SUM of the ranks' local gradients, the
-ranks end a step with identical weights, and the timing of a step with / without the collective.
-  python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29517 scripts/exp_train_ddp.py"""
-import os, sys, json
+"""2+ ranks (torchrun): the bucketed NCCL all-reduce inside ResNetTrainPlan (DenseNetTrainPlan with --arch densenet121) gives the
+SUM of the ranks' local gradients, the ranks end a step with identical weights, and the timing of a step with / without the collective.
+  python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29517 scripts/exp_train_ddp.py [--arch A]"""
+import argparse, os, sys, json
 import torch, torch.distributed as dist
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import bcos_b200  # noqa
-from bcos_b200.engine import ResNetTrainPlan
-from bcos_b200.models import resnet_state_shapes
+from bcos_b200.engine import DenseNetTrainPlan, ResNetTrainPlan
+from bcos_b200.models import densenet_state_shapes, resnet_state_shapes
 from bcos_b200.utils import synth, dist as D
+
+ap = argparse.ArgumentParser()
+ap.add_argument("--arch", default="resnet50", help="resnet18/34/50 or densenet121/169/201")
+arch = ap.parse_args().arch
+Plan, shapes = (DenseNetTrainPlan, densenet_state_shapes) if arch.startswith("densenet") else (ResNetTrainPlan, resnet_state_shapes)
 
 rank, local, world = D.env_rank()
 torch.cuda.set_device(local)
 D.init("nccl")
 dev = f"cuda:{local}"
-arch, B = "resnet50", 32
-sd = synth.synthetic_checkpoint(arch, resnet_state_shapes(arch))
+B = 32
+sd = synth.synthetic_checkpoint(arch, shapes(arch))
 imgs = torch.from_numpy(synth.synth_images_u8(B, 224, 500 + rank)).to(dev)
 labels = ((torch.arange(B) * 13 + rank * 7) % 1000).to(dev)
-local_plan = ResNetTrainPlan(arch, sd, B, device=dev, world_size=1)
+local_plan = Plan(arch, sd, B, device=dev, world_size=1)
 local_plan.load_batch(imgs, labels)
 local_plan.forward_backward()
 g_own = local_plan.g_flat.clone()
 g_local = g_own.clone()
 dist.all_reduce(g_local)
-plan = ResNetTrainPlan(arch, sd, B, device=dev, world_size=world, bucket_mb=25.0)
+plan = Plan(arch, sd, B, device=dev, world_size=world, bucket_mb=25.0)
 plan.load_batch(imgs, labels)
 plan.forward_backward()
 torch.cuda.synchronize()
