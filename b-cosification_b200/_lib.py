@@ -138,6 +138,15 @@ def igemm(p: IgemmParams) -> None:
     check(load().bcosk_igemm(C.byref(p), _stream()), "bcosk_igemm")
 
 
+def igemm_hp_config(p: IgemmParams) -> Tuple[int, ...]:
+    """(CTAs per SM the kernel is built for, threads, dynamic shared memory bytes, CTAs per SM the occupancy API reports,
+    registers per thread, local memory bytes per thread) of a parity-mode launch, without launching it (include/bcosk.h
+    bcosk_igemm_hp_config)."""
+    info = (C.c_int32 * 6)()
+    check(load().bcosk_igemm_hp_config(C.byref(p), info), "bcosk_igemm_hp_config")
+    return tuple(int(v) for v in info)
+
+
 def debug_a_tile(p: IgemmParams, tile_m: int, chunk: int, out) -> None:
     check(load().bcosk_debug_a_tile(C.byref(p), tile_m, chunk, _p(out), _stream()), "bcosk_debug_a_tile")
 

@@ -19,7 +19,8 @@
 //     fetched at kernel start into memory next to the ring when the K loop is short (bandwidth-bound launches), or after
 //     the last MMA into ring space when it is long (their lines are pulled into L2 by TMA prefetches meanwhile).
 //   * 320 threads: TMA producer warp, MMA warp, 8 epilogue warps (TMEM lane quadrant x 32-column half each, 32
-//     accumulator registers per thread), two CTAs per SM (128 TMEM columns and <= 113 KB of shared memory each).
+//     accumulator registers per thread), two CTAs per SM (256 TMEM columns and <= 113 KB of shared memory each).  64-wide
+//     forward launches may instead run 192 threads, three CTAs per SM (hp::Cfg<64, 3>, bcosk_igemm_params.sched = 3).
 //   * The common case (two planes, B = 2, everything boxed) runs a packed-fp32 epilogue (FMUL2 / FFMA2 / FADD2);
 //     anything else falls back, per tensor, to a generic form with per-row 16-byte accesses.
 #include <cuda.h>
@@ -38,27 +39,38 @@ constexpr int BM = 128;
 constexpr int STAGE_K = 64;
 constexpr int A_BYTES = BM * STAGE_K * 2;      // 16 KB
 constexpr int BOX_BYTES = BM * 128;            // one [128 rows][128 bytes] swizzled box
-constexpr int THREADS = 320;
 constexpr int MAX_STAGES = 8;
 // Tile width.  64: two CTAs per SM (<= 113 KB of shared memory, 256 TMEM columns each).  128 (forward launches with the packed
 // epilogue only): one CTA per SM, 64 KB paired stages - 98 instead of 65 FLOP per byte of L2 -> shared-memory fill, which is what
 // bounds the K >= 1024 launches (DESIGN.md 3.6); every epilogue warp then owns two 32-column groups.
-template <int BN_>
+// CTAS_ = 3 (64-wide forward launches with the packed epilogue only, `sched` 3): three CTAs per SM - more independent tiles in
+// flight for the latency-bound short-K launches.  128 TMEM columns (ONE partial accumulator + the cross-term accumulator: the MMA
+// warp waits for the epilogue to drain the partial before the next chunk), 6 warps (4 epilogue warps, each walks both 32-column
+// groups of its lane quadrant), one paired stage as the ring, <= 75 KB of shared memory.  CTAS_ = 4 (`sched` 4): the same kernel
+// for launches whose leading segment is one accumulation (no stash), <= 56 KB of shared memory and <= 80 registers.
+template <int BN_, int CTAS_ = (BN_ == 64 ? 2 : 1)>
 struct Cfg {
   static constexpr int BN = BN_;
+  static constexpr bool SLIM = CTAS_ >= 3;                  // one partial accumulator, four epilogue warps
+  static constexpr bool ONE_DRAIN = CTAS_ >= 4;             // launches whose leading segment is one accumulation (no stash)
+  static constexpr int EPI_WARPS = SLIM ? 4 : 8;
+  static constexpr int THREADS = 64 + 32 * EPI_WARPS;       // TMA producer, MMA issuer, epilogue warps
+  static constexpr int GS = EPI_WARPS / 4;                  // epilogue warps per lane quadrant: warp j owns groups jj = j + GS h
   static constexpr int NB = BN_ / 64;                       // 64-column boxes per plane of a 16-bit tensor
-  static constexpr int NG = BN_ / 64;                       // 32-column groups per epilogue warp (group jj = j + 2 h)
+  static constexpr int NG = BN_ / (32 * GS);                // 32-column groups per epilogue warp
+  static constexpr int NACC = SLIM ? 1 : 2;                 // partial accumulators of the leading segment
   static constexpr int B_BYTES = BN_ * STAGE_K * 2;         // 8 / 16 KB
   static constexpr int SLOT_BYTES = A_BYTES + B_BYTES;      // 24 / 32 KB
   static constexpr int PAIR_BYTES = 2 * A_BYTES + 2 * B_BYTES;   // paired stage: [A plane 0 | A plane 1 | B plane 0 | B plane 1] = 48 / 64 KB
   static constexpr int PLANE_BYTES = NB * BOX_BYTES;        // boxes of one plane lie back to back
-  static constexpr int TMEM_COLS = 4 * BN_;                 // two ping-pong partial accumulators + the cross-term accumulator (power of two)
+  static constexpr int TMEM_COLS = SLIM ? 2 * BN_ : 4 * BN_;    // partial accumulator(s) + the cross-term accumulator (power of two)
   static constexpr int TAIL_BYTES = 256 + 2 * BN_ * 4 + BM * 4;   // barriers | alpha, beta | sum-of-squares exchange
-  static constexpr int MAX_SMEM = BN_ == 64 ? 115712 : 230400;    // two CTAs per SM: (228 KB - 2 x 1 KB reserved) / 2; one: 225 KB
+  // (228 KB - CTAS x 1 KB reserved) / CTAS; one CTA: 225 KB
+  static constexpr int MAX_SMEM = CTAS_ == 1 ? 230400 : (233472 - CTAS_ * 1024) / CTAS_ / 128 * 128;
   static constexpr int MIN_SMEM = BN_ == 64 ? 0 : 118784;   // wide tiles allocate all of TMEM: keep a second CTA off the SM
-  static constexpr int MIN_BLOCKS = BN_ == 64 ? 2 : 1;
-  static constexpr int MAX_RING_PAIRED = BN_ == 64 ? 2 : 3;
-  static constexpr int MAX_RING = BN_ == 64 ? 4 : 6;
+  static constexpr int MIN_BLOCKS = CTAS_;
+  static constexpr int MAX_RING_PAIRED = SLIM ? 1 : (BN_ == 64 ? 2 : 3);
+  static constexpr int MAX_RING = SLIM ? 2 : (BN_ == 64 ? 4 : 6);
 };
 }  // namespace hp
 
@@ -78,6 +90,7 @@ struct HpAux {
   int fast;          // the packed two-plane epilogue applies
   uint32_t off_in16, off_in32;     // byte offsets of the box regions from the start of shared memory
   uint32_t off_out1, off_out2;
+  uint32_t off_stash;              // three-CTA kernel with more than one drain: running sums of the groups after the first (fp32 boxes)
   uint32_t tail;                   // barriers etc. (after the ring and the extra input area)
 };
 
@@ -139,7 +152,7 @@ __device__ __forceinline__ void split_pair(const float2 y, uint32_t& w0, uint32_
 // Packed forward epilogue of one row x 32 columns (two planes, B = 2 scale, everything boxed).
 //   t = |lin| * inv_norm * alpha;  y = lin * t + beta + res;  ReLU;  y -> two planes, gain = t (0 where clamped), sum y^2
 template <typename T>
-__device__ __forceinline__ void hp_fwd_fast(const float (&acc)[32], float inv_norm, uint32_t ab /* smem: alpha[32] of this group, beta at + 4 BN bytes */,
+__device__ __forceinline__ void hp_fwd_fast(const float* acc /* [32] */, float inv_norm, uint32_t ab /* smem: alpha[32] of this group, beta at + 4 BN bytes */,
                                             uint32_t res0 /* plane-0 box or 0 */, uint32_t y0, uint32_t gbox /* fp32 gain box or 0 */,
                                             uint32_t g16 /* 16-bit gain box or 0 */, int row, int j, bool relu, float& sq_acc,
                                             uint32_t& mbits, bool plain /* scale mode NONE: multiplier = alpha */,
@@ -197,7 +210,7 @@ __device__ __forceinline__ void hp_fwd_fast(const float (&acc)[32], float inv_no
 // Packed explain epilogue of one row x 32 columns (two planes, everything boxed except the optional fp32 mul2).
 //   tot = D + add;  out2 = tot * mul2 * mask2 bit;  y = tot * mul1
 template <typename T>
-__device__ __forceinline__ void hp_explain_fast(const float (&acc)[32], uint32_t add0 /* plane-0 box or 0 */, uint32_t gbox /* fp32 mul1 box or 0 */,
+__device__ __forceinline__ void hp_explain_fast(const float* acc /* [32] */, uint32_t add0 /* plane-0 box or 0 */, uint32_t gbox /* fp32 mul1 box or 0 */,
                                                 uint32_t y0, uint32_t o20 /* out2 plane-0 box or 0 */, const float* mul2_row /* global or null */,
                                                 uint32_t mb2, int row, int j, uint32_t pstep) {
   using namespace hp;
@@ -242,15 +255,16 @@ __device__ __forceinline__ void hp_explain_fast(const float (&acc)[32], uint32_t
   }
 }
 
-template <int MODE, typename T, int BN_>
-__global__ void __launch_bounds__(hp::THREADS, hp::Cfg<BN_>::MIN_BLOCKS)
+template <int MODE, typename T, int BN_, int CTAS_>
+__global__ void __launch_bounds__(hp::Cfg<BN_, CTAS_>::THREADS, hp::Cfg<BN_, CTAS_>::MIN_BLOCKS)
 bcosk_igemm_hp_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                       const __grid_constant__ CUtensorMap tmap_in16, const __grid_constant__ CUtensorMap tmap_in32,
                       const __grid_constant__ CUtensorMap tmap_out1, const __grid_constant__ CUtensorMap tmap_out2,
                       const __grid_constant__ bcosk_igemm_params p, const HpAux aux) {
   using namespace hp;
-  using C = Cfg<BN_>;
-  constexpr int BN = C::BN, NB = C::NB, NG = C::NG;
+  using C = Cfg<BN_, CTAS_>;
+  constexpr int BN = C::BN, NB = C::NB, NG = C::NG, GS = C::GS, NACC = C::NACC, EPI_THREADS = 32 * C::EPI_WARPS;
+  static_assert(!C::SLIM || MODE == BCOSK_MODE_FWD, "the three- and four-CTA kernels run forward launches only");
   constexpr int B_BYTES = C::B_BYTES, SLOT_BYTES = C::SLOT_BYTES, PAIR_BYTES = C::PAIR_BYTES, PLANE_BYTES = C::PLANE_BYTES;
   constexpr int TMEM_COLS = C::TMEM_COLS;
   extern __shared__ __align__(1024) uint8_t smem[];   // no static shared memory: the dynamic window starts 1024-byte aligned
@@ -292,9 +306,9 @@ bcosk_igemm_hp_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_c
       mbar_init(&full_bar[s], 1);
       mbar_init(&empty_bar[s], 1);
     }
-    for (int s = 0; s < 2; ++s) {
+    for (int s = 0; s < NACC; ++s) {
       mbar_init(&acc_full_bar[s], 1);
-      mbar_init(&acc_empty_bar[s], 8);   // one arrival per epilogue warp
+      mbar_init(&acc_empty_bar[s], C::EPI_WARPS);   // one arrival per epilogue warp
     }
     mbar_init(&acc_full_bar[2], 1);
     mbar_init(mma_done_bar, 1);
@@ -402,13 +416,13 @@ bcosk_igemm_hp_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_c
       int d = 0;                        // accumulation (drain) index
       if (aux.paired) {
         const uint64_t pair16 = PAIR_BYTES >> 4;
-        const uint32_t tmem_x = tmem_base + 2 * BN;      // cross-term accumulator
+        const uint32_t tmem_x = tmem_base + NACC * BN;   // cross-term accumulator
         for (int it = 0; it < num_iters; ++it) {
           const bool first = it % aux.chunk == 0;
           const bool last = it % aux.chunk == aux.chunk - 1 || it == num_iters - 1;
-          const uint32_t buf = (uint32_t)d & 1u;
+          const uint32_t buf = (uint32_t)d % NACC;
           if (first) {
-            mbar_wait(&acc_empty_bar[buf], (((uint32_t)d >> 1) & 1u) ^ 1u);
+            mbar_wait(&acc_empty_bar[buf], (((uint32_t)d / NACC) & 1u) ^ 1u);
             tc_fence_after();
           }
           const uint32_t tmem_d = tmem_base + buf * BN;
@@ -449,9 +463,9 @@ bcosk_igemm_hp_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_c
         const bool first = it < seg_iters ? (it % aux.chunk == 0) : (xi % aux.xchunk == 0);
         const bool last = it < seg_iters ? (it % aux.chunk == aux.chunk - 1 || it == seg_iters - 1)
                                          : (xi % aux.xchunk == aux.xchunk - 1 || it == num_iters - 1);
-        const uint32_t buf = (uint32_t)d & 1u;
+        const uint32_t buf = (uint32_t)d % NACC;
         if (first) {
-          mbar_wait(&acc_empty_bar[buf], (((uint32_t)d >> 1) & 1u) ^ 1u);
+          mbar_wait(&acc_empty_bar[buf], (((uint32_t)d / NACC) & 1u) ^ 1u);
           tc_fence_after();
           accumulate = 0;
         }
@@ -488,18 +502,18 @@ bcosk_igemm_hp_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_c
       }
     }
   } else {
-    // ===================== epilogue (warps 2..9) =====================
+    // ===================== epilogue (warps 2 .. 2 + EPI_WARPS - 1) =====================
     const int quad = warp & 3;                 // TMEM lane quadrant this warp may read
-    const int j = (warp - 2) >> 2;             // this warp owns the 32-column groups jj = j + 2 h, h < NG (warp-uniform)
+    const int j = (warp - 2) >> 2;             // this warp owns the 32-column groups jj = j + GS h, h < NG (warp-uniform)
     const int row = quad * 32 + lane;
-    const int et = threadIdx.x - 64;           // 0..255
+    const int et = threadIdx.x - 64;           // 0 .. EPI_THREADS - 1
     if (MODE == BCOSK_MODE_FWD) {
       if (et < BN) {
         const int c = n0 + et;
         s_alpha[et] = (p.alpha != nullptr && c < p.n) ? __ldg(p.alpha + c) : 1.f;
         s_beta[et] = (p.beta != nullptr && c < p.n) ? __ldg(p.beta + c) : 0.f;
       }
-      asm volatile("bar.sync 1, 256;" ::: "memory");
+      asm volatile("bar.sync 1, %0;" ::"n"(EPI_THREADS) : "memory");
     }
     RowInfo ri;
     ri.m = m0 + row;
@@ -545,14 +559,14 @@ bcosk_igemm_hp_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_c
     uint32_t mb2s[NG];
 #pragma unroll
     for (int h = 0; h < NG; ++h) {
-      const int c0 = n0 + (j + 2 * h) * 32;
+      const int c0 = n0 + (j + GS * h) * 32;
       mb2s[h] = 0xffffffffu;
       if (MODE == BCOSK_MODE_EXPLAIN && p.mask2 != nullptr && ri.valid && c0 < p.n) mb2s[h] = __ldg(p.mask2 + (size_t)ri.m * p.mask2_ld + (c0 >> 5));
     }
     // side tensors read with per-row loads after the last drain: pull their lines into L2 now
 #pragma unroll
     for (int h = 0; h < NG; ++h) {
-      const int c0 = n0 + (j + 2 * h) * 32;
+      const int c0 = n0 + (j + GS * h) * 32;
       if (!(ri.valid && c0 < p.n)) continue;
       const int ncols_pf = min(32, p.n - c0);
       auto prefetch_row = [&](const void* base, size_t elem_off, int elem_bytes) {
@@ -573,41 +587,80 @@ bcosk_igemm_hp_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_c
       }
     }
 
-    // ---- sum the partial accumulators of this thread's 32-column groups (round-to-nearest fp32 adds)
-    const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(j * 32);     // group h: + 64 h columns
-    float acc[NG][32];
+    // ---- sum the partial accumulators of this thread's 32-column groups (round-to-nearest fp32 adds, in drain order, then
+    //      the cross-term accumulator)
+    const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(j * 32);     // group h: + 32 GS h columns
+    constexpr int NGR = C::SLIM ? 1 : NG;      // groups whose sums live in registers across the drains
+    float acc[NGR][32];
 #pragma unroll
-    for (int h = 0; h < NG; ++h)
+    for (int h = 0; h < NGR; ++h)
 #pragma unroll
       for (int i = 0; i < 32; ++i) acc[h][i] = 0.f;
-    for (int d = 0; d < num_drains; ++d) {
-      const uint32_t buf = (uint32_t)d & 1u;
-      mbar_wait(&acc_full_bar[buf], ((uint32_t)d >> 1) & 1u);
+    if constexpr (!C::SLIM) {
+      for (int d = 0; d < num_drains; ++d) {
+        const uint32_t buf = (uint32_t)d % NACC;
+        mbar_wait(&acc_full_bar[buf], ((uint32_t)d / NACC) & 1u);
+        tc_fence_after();
+        uint32_t raw[NG][32];
+#pragma unroll
+        for (int h = 0; h < NG; ++h) tmem_ld_32x32(taddr + buf * BN + h * 32 * GS, raw[h]);
+        tmem_ld_wait();
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&acc_empty_bar[buf]);
+#pragma unroll
+        for (int h = 0; h < NG; ++h)
+#pragma unroll
+          for (int i = 0; i < 32; ++i) acc[h][i] += __uint_as_float(raw[h][i]);
+      }
+      if (aux.paired) {
+        mbar_wait(&acc_full_bar[2], 0);
+        tc_fence_after();
+        uint32_t raw[NG][32];
+#pragma unroll
+        for (int h = 0; h < NG; ++h) tmem_ld_32x32(taddr + NACC * BN + h * 32 * GS, raw[h]);
+        tmem_ld_wait();
+        tc_fence_before();
+#pragma unroll
+        for (int h = 0; h < NG; ++h)
+#pragma unroll
+          for (int i = 0; i < 32; ++i) acc[h][i] += __uint_as_float(raw[h][i]);
+      }
+    } else {
+      // One partial accumulator: every drain but the last is added here - group 0 into registers, the other groups into
+      // their stash boxes - and handed back to the MMA warp.  The last drain and the cross terms are added per group
+      // below, right before that group's epilogue, so at most 32 accumulator columns are live at a time.
+      const uint32_t stash = smem_u32(smem) + aux.off_stash;
+      for (int d = 0; !C::ONE_DRAIN && d + 1 < num_drains; ++d) {
+        mbar_wait(&acc_full_bar[0], (uint32_t)d & 1u);
+        tc_fence_after();
+        uint32_t raw[32];
+        tmem_ld_32x32(taddr, raw);
+        tmem_ld_wait();
+#pragma unroll
+        for (int i = 0; i < 32; ++i) acc[0][i] += __uint_as_float(raw[i]);
+#pragma unroll 1
+        for (int h = 1; h < NG; ++h) {
+          tmem_ld_32x32(taddr + h * 32, raw);
+          tmem_ld_wait();
+          const uint32_t sb = stash + (uint32_t)((h - 1) * BOX_BYTES);
+#pragma unroll
+          for (int u = 0; u < 8; ++u) {
+            float4 s = d == 0 ? make_float4(0.f, 0.f, 0.f, 0.f) : lds_f4(box_unit(sb, row, u));
+            s.x += __uint_as_float(raw[4 * u]);
+            s.y += __uint_as_float(raw[4 * u + 1]);
+            s.z += __uint_as_float(raw[4 * u + 2]);
+            s.w += __uint_as_float(raw[4 * u + 3]);
+            sts128(box_unit(sb, row, u), make_uint4(__float_as_uint(s.x), __float_as_uint(s.y), __float_as_uint(s.z), __float_as_uint(s.w)));
+          }
+        }
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&acc_empty_bar[0]);
+      }
+      mbar_wait(&acc_full_bar[0], (uint32_t)(num_drains - 1) & 1u);
+      if (aux.paired) mbar_wait(&acc_full_bar[2], 0);
       tc_fence_after();
-      uint32_t raw[NG][32];
-#pragma unroll
-      for (int h = 0; h < NG; ++h) tmem_ld_32x32(taddr + buf * BN + h * 64, raw[h]);
-      tmem_ld_wait();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&acc_empty_bar[buf]);
-#pragma unroll
-      for (int h = 0; h < NG; ++h)
-#pragma unroll
-        for (int i = 0; i < 32; ++i) acc[h][i] += __uint_as_float(raw[h][i]);
-    }
-    if (aux.paired) {
-      mbar_wait(&acc_full_bar[2], 0);
-      tc_fence_after();
-      uint32_t raw[NG][32];
-#pragma unroll
-      for (int h = 0; h < NG; ++h) tmem_ld_32x32(taddr + 2 * BN + h * 64, raw[h]);
-      tmem_ld_wait();
-      tc_fence_before();
-#pragma unroll
-      for (int h = 0; h < NG; ++h)
-#pragma unroll
-        for (int i = 0; i < 32; ++i) acc[h][i] += __uint_as_float(raw[h][i]);
     }
     if (any_in) mbar_wait(in_bar, 0);
 
@@ -620,13 +673,38 @@ bcosk_igemm_hp_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_c
 
 #pragma unroll
     for (int h = 0; h < NG; ++h) {
-      const int jj = j + 2 * h;                // 32-column group of the tile
+      const int jj = j + GS * h;               // 32-column group of the tile
       const int c0 = n0 + jj * 32;
+      float accs[C::SLIM ? 32 : 1];
+      if constexpr (C::SLIM) {
+        // (running sum or 0) + last drain + cross terms; tcgen05.ld is warp-wide, so before any lane leaves the loop
+        if (C::ONE_DRAIN || h == 0 || num_drains == 1) {
+#pragma unroll
+          for (int i = 0; i < 32; ++i) accs[i] = h == 0 ? acc[0][i] : 0.f;
+        } else {
+#pragma unroll
+          for (int u = 0; u < 8; ++u) {
+            const float4 s = lds_f4(box_unit(smem_u32(smem) + aux.off_stash + (uint32_t)((h - 1) * BOX_BYTES), row, u));
+            accs[4 * u] = s.x; accs[4 * u + 1] = s.y; accs[4 * u + 2] = s.z; accs[4 * u + 3] = s.w;
+          }
+        }
+        uint32_t raw[32];
+        tmem_ld_32x32(taddr + h * 32, raw);
+        tmem_ld_wait();
+#pragma unroll
+        for (int i = 0; i < 32; ++i) accs[i] += __uint_as_float(raw[i]);
+        if (aux.paired) {
+          tmem_ld_32x32(taddr + BN + h * 32, raw);
+          tmem_ld_wait();
+#pragma unroll
+          for (int i = 0; i < 32; ++i) accs[i] += __uint_as_float(raw[i]);
+        }
+      }
       if (!(ri.valid && c0 < p.n)) continue;
       const int ncols = min(32, p.n - c0);
-      const float (&accv)[32] = acc[h];
+      const float* accv = C::SLIM ? accs : acc[C::SLIM ? 0 : h];
       const uint32_t mb2 = mb2s[h];
-      if (aux.fast) {
+      if (C::SLIM || aux.fast) {
         if (MODE == BCOSK_MODE_FWD) {
           uint32_t mbits;
           hp_fwd_fast<T>(accv, inv_norm, smem_u32(s_alpha + jj * 32), aux.in16_planes ? r_in16 : 0u, r_out1,
@@ -824,10 +902,10 @@ bcosk_igemm_hp_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_c
       }
     }
     const bool want_sq = MODE == BCOSK_MODE_FWD && p.sq_out != nullptr;
-    if (want_sq && j == 1) s_sq[row] = sq_acc;
+    if (want_sq && j == 1) s_sq[row] = sq_acc;  // (GS = 2: the upper column half's sum goes to the warp of the lower one)
     // generic-proxy writes of the staged boxes -> visible to the async proxy, then one thread issues the bulk stores
     if (aux.out1_planes != 0 || aux.out2_kind != 0) fence_proxy_async_smem();
-    asm volatile("bar.sync 1, 256;" ::: "memory");
+    asm volatile("bar.sync 1, %0;" ::"n"(EPI_THREADS) : "memory");
     if ((aux.out1_planes != 0 || aux.out2_kind != 0) && et == 0) {
       for (int pl = 0; pl < aux.out1_planes; ++pl)
         for (int b = 0; b < boxes16; ++b)
@@ -844,7 +922,7 @@ bcosk_igemm_hp_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_c
       tma_store_commit_and_wait_read();
     }
     if (MODE == BCOSK_MODE_FWD && j == 0 && ri.valid) {
-      if (want_sq) p.sq_out[(size_t)tile_n * M + ri.m] = sq_acc + (n0 + 32 < p.n ? s_sq[row] : 0.f);
+      if (want_sq) p.sq_out[(size_t)tile_n * M + ri.m] = GS == 1 ? sq_acc : sq_acc + (n0 + 32 < p.n ? s_sq[row] : 0.f);
       if (p.inv_norm_out != nullptr && tile_n == 0) p.inv_norm_out[ri.m] = inv_norm;
     }
     tc_fence_before();
@@ -865,10 +943,12 @@ static int g_hp_xchunk = 0;      // experiment override of the cross-term accumu
 static int g_hp_stage_boxes = 1; // 0 = per-row epilogue I/O everywhere (A/B measurements)
 static int g_hp_early_iters = 4; // K loops of at most this many stages fetch their input boxes at kernel start
 
-template <int MODE, int BN_>
-static int launch_hp_mode(const bcosk_igemm_params& p, cudaStream_t st) {
+// The three- and four-CTA kernels (CTAS_ = 3, 4) set *declined and launches nothing where it does not apply (no packed epilogue, or its
+// boxes do not fit one paired stage): the caller then runs the two-CTA kernel, which gives the same bits.
+template <int MODE, int BN_, int CTAS_ = (BN_ == 64 ? 2 : 1)>
+static int launch_hp_mode(const bcosk_igemm_params& p, cudaStream_t st, bool* declined = nullptr, int32_t* info = nullptr) {
   using namespace hp;
-  using C = Cfg<BN_>;
+  using C = Cfg<BN_, CTAS_>;
   constexpr int BN = C::BN;
   constexpr int SLOT_BYTES = C::SLOT_BYTES, PAIR_BYTES = C::PAIR_BYTES, PLANE_BYTES = C::PLANE_BYTES, TAIL_BYTES = C::TAIL_BYTES;
   constexpr int MAX_SMEM = C::MAX_SMEM;
@@ -937,7 +1017,17 @@ static int launch_hp_mode(const bcosk_igemm_params& p, cudaStream_t st) {
   const int slot_b = aux.paired ? PAIR_BYTES : SLOT_BYTES;
   const int max_ring = aux.paired ? C::MAX_RING_PAIRED : C::MAX_RING;        // ring slots that fit the CTAs of one SM
   const int iters = aux.paired ? p.num_taps * p.chunks_per_tap : p.num_segs * p.num_taps * p.chunks_per_tap / (STAGE_K / p.kch);
-  const int early_iters = aux.paired ? (g_hp_early_iters + 2) / 3 : g_hp_early_iters;
+  // (three CTAs: input boxes always after the last MMA - the other CTAs of the SM hide the fetch)
+  const int early_iters = C::SLIM ? 0 : (aux.paired ? (g_hp_early_iters + 2) / 3 : g_hp_early_iters);
+  // three CTAs with more than one drain of the single partial accumulator: the running sums of the column groups after the
+  // first wait in a stash between the ring and the tail
+  int stash_b = 0;
+  if (C::SLIM) {
+    const int seg_iters = p.num_taps * p.chunks_per_tap / (STAGE_K / p.kch);
+    const int main_drains = (seg_iters + aux.chunk - 1) / aux.chunk;
+    const int num_drains = aux.paired ? main_drains : main_drains + (iters - seg_iters + aux.xchunk - 1) / aux.xchunk;
+    if (num_drains > 1) stash_b = (C::NG - 1) * BOX_BYTES;
+  }
   int stages = 0, extra = 0;
   auto place = [&]() -> bool {
     const int in16_b = aux.in16_planes * PLANE_BYTES, in32_b = aux.in32 ? (BN / 32) * BOX_BYTES : 0;
@@ -972,13 +1062,29 @@ static int launch_hp_mode(const bcosk_igemm_params& p, cudaStream_t st) {
     const int need = a_b + b_b + c_b;
     stages = (need + slot_b - 1) / slot_b;
     if (stages < max_ring) stages = max_ring;
-    if (stages > MAX_STAGES || stages * slot_b + tail_bytes > MAX_SMEM) return false;
+    // three CTAs: one paired stage, plus the stash box behind it.  fp32 gains (two boxes) may overrun the stage by exactly
+    // one box, the gain box of the second column group, which then shares the stash's place: each thread reads its row of
+    // the stash before it writes its row of that gain box.
+    int over = 0;
+    if (C::SLIM && stages > max_ring) {
+      over = need - max_ring * slot_b;
+      if (!(MODE == BCOSK_MODE_FWD && aux.out2_kind == 1 && over == BOX_BYTES)) return false;
+      stages = max_ring;
+    }
+    if (C::ONE_DRAIN && (stash_b != 0 || over != 0)) return false;   // four CTAs: the ring and the tail only
+    extra = stash_b > over ? stash_b : over;
+    if (stages > MAX_STAGES || stages * slot_b + extra + tail_bytes > MAX_SMEM) return false;
+    aux.off_stash = (uint32_t)(stages * slot_b);
     aux.off_in16 = 0;
     aux.off_out1 = 0;
     aux.off_in32 = (uint32_t)a_b;
     aux.off_out2 = MODE == BCOSK_MODE_FWD ? (uint32_t)a_b : (uint32_t)(a_b + b_b);
     return true;
   };
+  if (C::SLIM && !place()) {
+    *declined = true;
+    return BCOSK_OK;
+  }
   while (!place()) {
     if (MODE == BCOSK_MODE_EXPLAIN && aux.out2_kind == 2) aux.out2_kind = 0, aux.out2_planes = 0;
     else if (aux.in16_planes) aux.in16_planes = 0;
@@ -995,30 +1101,47 @@ static int launch_hp_mode(const bcosk_igemm_params& p, cudaStream_t st) {
     aux.fast = !p.y_f32 && p.y_planes == 2 && aux.out1_planes == 2 && (!p.add || aux.in16_planes == 2) && (!p.mul1 || aux.in32) &&
                (!p.out2 || (aux.out2_kind == 2 && aux.out2_planes == 2)) && (!p.mul2 || p.mul2_f32);
   if (g_hp_stage_boxes & 2) aux.fast = 0;      // A/B: generic epilogue arithmetic over the same boxes
+  if (C::SLIM && !aux.fast) {
+    *declined = true;
+    return BCOSK_OK;
+  }
   aux.stages = stages;
   aux.tail = (uint32_t)(stages * slot_b + extra);
   if (BN_ > 64 && !aux.fast)
     return set_error(BCOSK_EUNSUPPORTED, "igemm(hp): 128-wide tiles need the packed two-plane epilogue (two boxed planes, B = 2 or plain scale)");
   int smem = (int)aux.tail + tail_bytes;
   if (smem < C::MIN_SMEM) smem = C::MIN_SMEM;
-  auto kern = bcosk_igemm_hp_kernel<MODE, __nv_bfloat16, BN_>;
-  auto kern_h = bcosk_igemm_hp_kernel<MODE, __half, BN_>;
+  auto kern = bcosk_igemm_hp_kernel<MODE, __nv_bfloat16, BN_, CTAS_>;
+  auto kern_h = bcosk_igemm_hp_kernel<MODE, __half, BN_, CTAS_>;
   const void* fn = (p.dtype == BCOSK_DTYPE_BF16) ? (const void*)kern : (const void*)kern_h;
   BCOSK_CUDA_CHECK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, MAX_SMEM));
   BCOSK_CUDA_CHECK(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  if (info != nullptr) {        // bcosk_igemm_hp_config: report the configuration instead of launching
+    int blocks = 0;
+    BCOSK_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, fn, C::THREADS, (size_t)smem));
+    cudaFuncAttributes fa;
+    BCOSK_CUDA_CHECK(cudaFuncGetAttributes(&fa, fn));
+    info[0] = CTAS_;
+    info[1] = C::THREADS;
+    info[2] = smem;
+    info[3] = blocks;
+    info[4] = fa.numRegs;
+    info[5] = (int32_t)fa.localSizeBytes;
+    return BCOSK_OK;
+  }
   const long long m_tiles = (M + BM - 1) / BM;
   const long long n_tiles = (p.n + BN - 1) / BN;
   if (m_tiles * n_tiles > 0x7fffffffLL) return set_error(BCOSK_EUNSUPPORTED, "igemm(hp): grid too large");
   dim3 grid((unsigned)(m_tiles * n_tiles));
   if (p.dtype == BCOSK_DTYPE_BF16)
-    kern<<<grid, THREADS, smem, st>>>(ma, mb, min16, min32, mout1, mout2, p, aux);
+    kern<<<grid, C::THREADS, smem, st>>>(ma, mb, min16, min32, mout1, mout2, p, aux);
   else
-    kern_h<<<grid, THREADS, smem, st>>>(ma, mb, min16, min32, mout1, mout2, p, aux);
+    kern_h<<<grid, C::THREADS, smem, st>>>(ma, mb, min16, min32, mout1, mout2, p, aux);
   BCOSK_CUDA_CHECK(cudaGetLastError());
   return BCOSK_OK;
 }
 
-int launch_hp(const bcosk_igemm_params& p, cudaStream_t st) {
+static int dispatch_hp(const bcosk_igemm_params& p, cudaStream_t st, int32_t* info) {
   const int cps = hp::STAGE_K / p.kch;
   if ((p.num_taps * p.chunks_per_tap) % cps != 0)
     return set_error(BCOSK_EINVAL, "igemm(hp): a segment must be a whole number of K stages");
@@ -1026,12 +1149,32 @@ int launch_hp(const bcosk_igemm_params& p, cudaStream_t st) {
   if (p.mul1_sqrt_scale) return set_error(BCOSK_EUNSUPPORTED, "igemm(hp): recomputed gains (mul1_sqrt_scale) are a throughput-mode option");
   if (p.block_n == 128) {
     if (p.mode != BCOSK_MODE_FWD) return set_error(BCOSK_EUNSUPPORTED, "igemm(hp): 128-wide tiles are a forward-launch option");
-    return launch_hp_mode<BCOSK_MODE_FWD, 128>(p, st);
+    return launch_hp_mode<BCOSK_MODE_FWD, 128>(p, st, nullptr, info);
   }
-  return p.mode == BCOSK_MODE_FWD ? launch_hp_mode<BCOSK_MODE_FWD, 64>(p, st) : launch_hp_mode<BCOSK_MODE_EXPLAIN, 64>(p, st);
+  if (p.sched == 4 && p.mode == BCOSK_MODE_FWD) {
+    bool declined = false;
+    const int rc = launch_hp_mode<BCOSK_MODE_FWD, 64, 4>(p, st, &declined, info);
+    if (!declined) return rc;
+  }
+  if ((p.sched == 3 || p.sched == 4) && p.mode == BCOSK_MODE_FWD) {
+    bool declined = false;
+    const int rc = launch_hp_mode<BCOSK_MODE_FWD, 64, 3>(p, st, &declined, info);
+    if (!declined) return rc;
+  }
+  return p.mode == BCOSK_MODE_FWD ? launch_hp_mode<BCOSK_MODE_FWD, 64>(p, st, nullptr, info)
+                                  : launch_hp_mode<BCOSK_MODE_EXPLAIN, 64>(p, st, nullptr, info);
 }
 
+int launch_hp(const bcosk_igemm_params& p, cudaStream_t st) { return dispatch_hp(p, st, nullptr); }
+
 }  // namespace bcosk
+
+extern "C" int bcosk_igemm_hp_config(const bcosk_igemm_params* p, int32_t* info) {
+  if (!p || !info || !p->hp_accum) return bcosk::set_error(BCOSK_EINVAL, "igemm_hp_config: needs hp_accum params and info[6]");
+  bcosk_igemm_params q = *p;
+  if (q.block_n == 0) q.block_n = 64;
+  return bcosk::dispatch_hp(q, 0, info);
+}
 
 extern "C" int bcosk_set_hp_chunk(int32_t stages) {
   const int prev = bcosk::g_hp_chunk | (bcosk::g_hp_xchunk << 16);

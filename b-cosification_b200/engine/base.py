@@ -484,6 +484,8 @@ class PlanBase:
 
         The three schedules give bit-identical outputs (tests/test_kernels_gpu.py); which is fastest depends on N, K and
         the epilogue streams (measured: profiles/r01_schedule_ab.md), so it is decided per launch, once, before capture.
+        64-wide forward launches of the plane-aware kernel (hp_accum) choose between two (sched 1), three (sched 3) and four
+        (sched 4) CTAs per SM, which also give bit-identical outputs (tests/test_igemm_hp_ctas_gpu.py; profiles/r03_hp_three_ctas.md).
         Returns {launch name: (block_n, sched)}.
         """
         self._require_gpu()
@@ -506,24 +508,28 @@ class PlanBase:
             return sorted(ts)[len(ts) // 2]
 
         for op in self.fwd_ops + (self.bwd_ops if self.with_explain else []):
-            if not isinstance(op, O.IgemmOp) or op.hp_accum or op.flat:
+            if not isinstance(op, O.IgemmOp) or op.flat:
                 continue
-            # tile width: free to choose where no per-tile partial sums of squares are written (their layout follows it)
-            widths = [op.resolved_block_n()]
-            if op.sq_out is None and op.n >= 128 and widths[0] in (64, 128):
-                widths = [64, 128]
-            if widths == [128]:
-                continue
-            best, best_t = (widths[0], 1 if widths[0] == 64 else 0), float("inf")
-            for bn in widths:
-                op.block_n = bn
-                for sched in ((1, 2, 3) if bn == 64 else (0,)):
-                    if sched == 3 and op.n <= 64:
-                        continue                      # a single n tile: same as 2
-                    op.sched = sched
-                    t = timed(op)
-                    if t < best_t * 0.98:             # prefer the earlier (simpler) candidate on a tie
-                        best, best_t = (bn, sched), t
+            if op.hp_accum:
+                # plane-aware kernel: 64-wide forward launches run two (sched 1), three (sched 3) or four (sched 4) CTAs per SM
+                if op.mode != L.BCOSK_MODE_FWD or op.resolved_block_n() != 64:
+                    continue
+                cands = [(64, 1), (64, 3), (64, 4)]
+            else:
+                # tile width: free to choose where no per-tile partial sums of squares are written (their layout follows it)
+                widths = [op.resolved_block_n()]
+                if op.sq_out is None and op.n >= 128 and widths[0] in (64, 128):
+                    widths = [64, 128]
+                if widths == [128]:
+                    continue
+                cands = [(bn, sched) for bn in widths for sched in ((1, 2, 3) if bn == 64 else (0,))
+                         if not (sched == 3 and op.n <= 64)]   # a single n tile: 3 is the same as 2
+            best, best_t = cands[0], float("inf")
+            for bn, sched in cands:
+                op.block_n, op.sched = bn, sched
+                t = timed(op)
+                if t < best_t * 0.98:                 # prefer the earlier (simpler) candidate on a tie
+                    best, best_t = (bn, sched), t
             op.block_n, op.sched = best
             chosen[op.name] = best
             op.run()                                  # leave the tensors as the chosen configuration writes them
@@ -533,8 +539,8 @@ class PlanBase:
     def capture(self, autotune: Optional[bool] = None) -> None:
         """Capture forward and forward+explain as CUDA graphs (kernel parameters incl. TMA descriptors are baked in)."""
         self._require_gpu()
-        if (self.autotune_default if autotune is None else autotune) and not (self.hp_accum and self.bwd_hp):
-            self.autotune()      # parity-mode launches have one schedule: autotune skips them
+        if self.autotune_default if autotune is None else autotune:
+            self.autotune()
         s = torch.cuda.Stream()
         s.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(s):

@@ -129,11 +129,17 @@ typedef struct bcosk_igemm_params {
    *      (bcosk_set_hp_chunk, initially 2).  With fp16 planes the cross-term segments (a0 b1, a1 b0; each 2^-11 of the leading one) run back
    *      to back in ONE further accumulation; with bf16 planes they are chunked like the leading segment. */
   int32_t hp_chunk;
-  /* ---- schedule of a block_n == 64 launch (ignored otherwise and with hp_accum; results do not depend on it):
+  /* ---- schedule of a block_n == 64 launch (ignored otherwise; results do not depend on it):
    *      0 = library default (see bcosk_set_persistent / bcosk_set_light), 1 = one CTA per tile,
    *      2 = persistent CTAs, tiles strided over the grid, 3 = persistent CTAs, each walks all n tiles of one
    *      128-row block back to back (the segments of an output row reach L2 together).  The host plan measures the
-   *      three per launch once (engine/base.py PlanBase.autotune) - which wins depends on N/K and the epilogue streams. */
+   *      three per launch once (engine/base.py PlanBase.autotune) - which wins depends on N/K and the epilogue streams.
+   *      With hp_accum (forward launches only): 3 = three CTAs per SM (6 warps, 128 TMEM columns: one partial accumulator
+   *      of the leading segment, drained before the next chunk starts; one paired stage as the ring) where the packed
+   *      two-plane epilogue applies and its boxes fit that stage, else the same as 0; 4 = four CTAs per SM (the same kernel in
+   *      <= 56 KB of shared memory: launches whose leading segment is ONE accumulation, K stages <= hp_chunk, with 16-bit gains),
+   *      else the same as 3; any other value = two CTAs per SM (10 warps, two ping-pong partial accumulators).  All give
+   *      bit-identical y planes, gains, mask bits and sums of squares; the plan measures them per launch. */
   int32_t sched;
   /* ---- flat-window gather (a_flat = 1): `a` points at pixel (0,0) of a [a_nb, a_h, a_w, a_c] VIEW into a larger
    *      zero-bordered buffer whose rows are a_wp pixels and whose images are a_hp rows apart (borders at least as wide
@@ -198,6 +204,12 @@ int bcosk_set_hp_chunk(int32_t stages);
  * then a1 b0, instead of both per stage; with bf16 planes also in chunks), which moves the last bit of fp32 within the same error
  * bound (tests/test_contract_gemm_fp64_gpu.py). */
 int bcosk_set_hp_boxes(int32_t enabled);
+/* Parity-mode launch configuration, without launching: info[0] = CTAs per SM the chosen kernel is built for (2, 3 or 4 for
+ * 64-wide tiles, see `sched`; 1 for 128-wide), info[1] = threads per CTA, info[2] = dynamic shared memory bytes,
+ * info[3] = CTAs per SM cudaOccupancyMaxActiveBlocksPerMultiprocessor reports for that kernel at that size (measured on a
+ * B200 with CUDA 12.9: 1 for every instance of this kernel, also at 0 bytes, though registers, threads and shared memory admit
+ * 2, 3 or 4), info[4] = registers per thread, info[5] = local memory bytes per thread (spills).  Needs a current device. */
+int bcosk_igemm_hp_config(const bcosk_igemm_params* p, int32_t* info);
 
 /* Scheduling switch for A/B measurements: 1 = launches with block_n 64 (the bandwidth-bound ones) run on the persistent
  * one-CTA-per-SM kernel, 0 (default) = one CTA per tile everywhere.  Returns the previous setting.  Results are identical. */
