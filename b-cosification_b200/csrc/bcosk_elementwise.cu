@@ -478,6 +478,15 @@ avgpool_bwd_mul_rows_kernel(const T* __restrict__ gy, int h, int w, int c, int k
 // ------------------------------------------------------------------------------------------------
 // classifier tail: GAP + logit layer + argmax (one block per image)
 // ------------------------------------------------------------------------------------------------
+// torch.argmax order: NaN above every number, then the larger value, then the smaller index.  The starting candidate
+// (-inf, INT_MAX) loses to every class, so a row of -inf gives 0 and `pred` is always a class index.
+__device__ __forceinline__ bool argmax_before(float v, int i, float bv, int bi) {
+  const bool vn = v != v, bn = bv != bv;
+  if (vn != bn) return vn;
+  if (vn || v == bv) return i < bi;
+  return v > bv;
+}
+
 __global__ void gap_logits_kernel(const float* __restrict__ fc, int npix, int ncls, float inv_temp, float bias,
                                   float* __restrict__ logits, int* __restrict__ pred) {
   const int img = blockIdx.x;
@@ -490,15 +499,15 @@ __global__ void gap_logits_kernel(const float* __restrict__ fc, int npix, int nc
     for (int px = 0; px < npix; ++px) acc += __ldg(src + (size_t)px * ncls + cls);
     const float l = acc * invn * inv_temp + bias;
     logits[(size_t)img * ncls + cls] = l;
-    if (l > best) { best = l; best_i = cls; }
+    if (argmax_before(l, cls, best, best_i)) { best = l; best_i = cls; }
   }
-  // block arg-max, smallest index on ties
+  // block arg-max
   __shared__ float s_v[32];
   __shared__ int s_i[32];
   for (int o = 16; o > 0; o >>= 1) {
     const float ov = __shfl_xor_sync(0xffffffffu, best, o);
     const int oi = __shfl_xor_sync(0xffffffffu, best_i, o);
-    if (ov > best || (ov == best && oi < best_i)) { best = ov; best_i = oi; }
+    if (argmax_before(ov, oi, best, best_i)) { best = ov; best_i = oi; }
   }
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (lane == 0) { s_v[warp] = best; s_i[warp] = best_i; }
@@ -510,7 +519,7 @@ __global__ void gap_logits_kernel(const float* __restrict__ fc, int npix, int nc
     for (int o = 16; o > 0; o >>= 1) {
       const float ov = __shfl_xor_sync(0xffffffffu, best, o);
       const int oi = __shfl_xor_sync(0xffffffffu, best_i, o);
-      if (ov > best || (ov == best && oi < best_i)) { best = ov; best_i = oi; }
+      if (argmax_before(ov, oi, best, best_i)) { best = ov; best_i = oi; }
     }
     if (lane == 0 && pred != nullptr) pred[img] = best_i;
   }
@@ -798,6 +807,7 @@ extern "C" int bcosk_avgpool_bwd_mul(const void* gy, int32_t nb, int32_t h, int3
 extern "C" int bcosk_gap_logits(const float* fc, int32_t nb, int32_t npix, int32_t ncls, float inv_temp, float bias,
                                 float* logits, int32_t* pred, void* stream) {
   if (!fc || !logits) return set_error(BCOSK_EINVAL, "gap_logits: null pointer");
+  if (nb < 1 || npix < 1 || ncls < 1) return set_error(BCOSK_EINVAL, "gap_logits: bad shape");
   gap_logits_kernel<<<nb, 256, 0, S(stream)>>>(fc, npix, ncls, inv_temp, bias, logits, pred);
   BCOSK_CUDA_CHECK(cudaGetLastError());
   return BCOSK_OK;
@@ -821,6 +831,8 @@ template <typename SRC>
 static int contrib_map_impl(const float* g, const SRC* x, int32_t nb, int32_t h, int32_t w, int32_t cp,
                             const float* inv_std6, float out_scale, float* cmap, float* grad6, void* stream) {
   if (!g || !x || !cmap || !inv_std6 || cp < 24 || cp % 4) return set_error(BCOSK_EINVAL, "contrib_map: bad argument");
+  // one thread per 2x2 block, written with float2 stores: an odd size would leave the last row / column unwritten
+  if (h < 2 || w < 2 || h % 2 || w % 2) return set_error(BCOSK_EINVAL, "contrib_map: need even h, w (as input_prep)");
   InvStd6 is;
   for (int i = 0; i < 6; ++i) is.v[i] = inv_std6[i];
   if (nb < 1 || nb > 65535) return set_error(BCOSK_EINVAL, "contrib_map: batch must be in [1, 65535]");

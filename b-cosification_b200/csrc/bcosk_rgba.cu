@@ -16,7 +16,7 @@ __device__ __forceinline__ float x6_value(const float* x, size_t img, int c, siz
   return __ldg(x + (img * 6 + c) * plane + pix);
 }
 __device__ __forceinline__ float x6_value(const uint8_t* x, size_t img, int c, size_t plane, size_t pix) {
-  const float v = (float)__ldg(x + (img * 3 + (c % 3)) * plane + pix) * (1.0f / 255.0f);
+  const float v = (float)__ldg(x + (img * 3 + (c % 3)) * plane + pix) / 255.0f;
   return c < 3 ? v : 1.0f - v;                       // AddInverse (bcos/data/transforms.py:42-55)
 }
 
@@ -111,7 +111,8 @@ __global__ void rgba_finalize_kernel(const float* __restrict__ alpha, const floa
   const int pix = blockIdx.x * blockDim.x + threadIdx.x;
   if (pix >= plane) return;
   const float a = alpha[img * plane + pix] / qv[img];
-  out[(img * plane + pix) * 4 + 3] = fminf(fmaxf(a, 0.f), 1.f);
+  // torch.clamp keeps NaN: a zero quantile over zero alpha (an all-zero gradient image) is 0/0 in the reference too
+  out[(img * plane + pix) * 4 + 3] = a != a ? a : fminf(fmaxf(a, 0.f), 1.f);
 }
 
 template <typename SRC>

@@ -97,7 +97,7 @@ __global__ void vit_patchify_kernel(const X* __restrict__ x, int H, int W, int p
   if (sizeof(X) == 1) {
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
-      const float r = (float)x[(((size_t)img * 3 + c) * H + yy) * W + xx] * (1.0f / 255.0f);
+      const float r = (float)x[(((size_t)img * 3 + c) * H + yy) * W + xx] / 255.0f;
       v[c] = r;
       v[c + 3] = 1.0f - r;
     }
@@ -153,7 +153,7 @@ __global__ void vit_contrib_map_kernel(const float* __restrict__ g, const X* __r
   for (int c = 0; c < 6; ++c) {
     float xv;
     if (sizeof(X) == 1) {
-      const float r = (float)x[(((size_t)img * 3 + (c % 3)) * H + yy) * W + xx] * (1.0f / 255.0f);
+      const float r = (float)x[(((size_t)img * 3 + (c % 3)) * H + yy) * W + xx] / 255.0f;
       xv = c < 3 ? r : 1.0f - r;
     } else {
       xv = (float)x[(((size_t)img * 6 + c) * H + yy) * W + xx];

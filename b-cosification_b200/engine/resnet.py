@@ -270,6 +270,9 @@ class ResNetPlan(PlanBase):
         if targets.ndim == 1:
             targets = targets[None]
         assert targets.shape[1] == self.nb, (targets.shape, self.nb)
+        # the seed kernel indexes the classifier's weights with these: reject a bad class before anything is launched
+        if targets.numel() and (int(targets.min()) < 0 or int(targets.max()) >= self.ncls):
+            raise ValueError(f"targets must lie in [0, {self.ncls}), got [{int(targets.min())}, {int(targets.max())}]")
         if x6 is not None:
             self.load_input(x6)
         self.replay_forward()

@@ -332,7 +332,8 @@ int bcosk_gather_cast_multi(const float* src, const int64_t* table, int32_t npac
  * 16-bit layout change and the 2x2 space-to-depth that turns the 7x7/2 stem into a 4x4/1 conv:
  *   x    [nb, 6, h, w] fp32 (un-normalised [x, 1-x])
  *   out  [nb, h/2, w/2, planes * cp]   channel (dy*2+dx)*6 + c, zero padded to cp
- *   sq   [nb, h, w] fp32  sum_c xn^2 per ORIGINAL pixel (for the stem patch norm); may be NULL */
+ *   sq   [nb, h, w] fp32  sum_c xn^2 per ORIGINAL pixel (for the stem patch norm), summed over the STORED values (the sum
+ *        of the planes written for each channel, squared), so that the norm matches the operand the stem GEMM reads; may be NULL */
 int bcosk_input_prep_s2d(const float* x, int32_t nb, int32_t h, int32_t w, const float* mean6, const float* inv_std6,
                          void* out, int32_t cp, int32_t planes, int32_t dtype, float* sq, int32_t out_row_pitch,
                          int32_t out_img_pitch, void* stream);
@@ -369,7 +370,8 @@ int bcosk_avgpool_bwd_mul(const void* gy, int32_t nb, int32_t h, int32_t w, int3
  * sqrt(gain * gain_sqrt_scale[pixel]) (see bcosk_igemm_params.mul1_sqrt_scale); single 16-bit plane only. */
 
 /* ResNetBcos._forward_impl standard_models.py:50-52 tail + LogitLayer logitlayer.py:22-27:
- * logits[img, cls] = mean_pix fc[img, pix, cls] * inv_temp + bias; pred[img] = argmax (first max). */
+ * logits[img, cls] = mean_pix fc[img, pix, cls] * inv_temp + bias; pred[img] = argmax in torch.argmax's order: the first NaN,
+ * else the first maximum (a row of -inf gives 0), so pred is always in [0, ncls). */
 int bcosk_gap_logits(const float* fc, int32_t nb, int32_t npix, int32_t ncls, float inv_temp, float bias,
                      float* logits, int32_t* pred, void* stream);
 
@@ -383,7 +385,8 @@ int bcosk_fc_seed_dgrad(const int32_t* target, const void* gain_fc, int32_t gain
 
 /* (in_tensor * in_tensor.grad).sum(1) bcos/common.py:181, reading the stem dgrad in its space-to-depth
  * layout g [nb, h/2, w/2, cp] fp32 and the raw input x [nb,6,h,w] fp32:
- *   grad6[img,c,y,x] = g * inv_std6[c] * out_scale (optional output), cmap[img,y,x] = sum_c x * grad6 */
+ *   grad6[img,c,y,x] = g * inv_std6[c] * out_scale (optional output), cmap[img,y,x] = sum_c x * grad6
+ * h and w must be even (as for bcosk_input_prep_s2d). */
 int bcosk_contrib_map_s2d(const float* g, const float* x, int32_t nb, int32_t h, int32_t w, int32_t cp,
                           const float* inv_std6, float out_scale, float* cmap, float* grad6, void* stream);
 int bcosk_contrib_map_s2d_u8(const float* g, const uint8_t* x, int32_t nb, int32_t h, int32_t w, int32_t cp,
@@ -394,7 +397,9 @@ int bcosk_contrib_map_s2d_u8(const float* g, const uint8_t* x, int32_t nb, int32
  * x = the network input ([nb,6,h,w] fp32, or uint8 RGB [nb,3,h,w] with the inverse channels formed on the fly).
  * smooth = odd box-filter window of the alpha channel (15 in the reference, 0 = none), percentile in [0,100] (99.5):
  * alpha is divided by that per-image percentile (torch.quantile: linear interpolation of the two neighbouring order
- * statistics, found by radix select) and clipped to [0,1].  tmp: 2*nb*h*w + nb floats of scratch. */
+ * statistics, found by radix select) and clipped to [0,1] like torch.clamp, which keeps NaN: an image whose percentile is
+ * 0 gets NaN where its alpha is 0 (an all-zero gradient image: NaN everywhere), as the reference does.  The quantile's
+ * position q*(n-1) is formed in fp32.  tmp: 2*nb*h*w + nb floats of scratch. */
 int bcosk_explanation_rgba(const float* grad6, const float* x, int32_t nb, int32_t h, int32_t w, int32_t smooth,
                            float percentile, float* tmp, float* out, void* stream);
 int bcosk_explanation_rgba_u8(const float* grad6, const uint8_t* x, int32_t nb, int32_t h, int32_t w, int32_t smooth,
