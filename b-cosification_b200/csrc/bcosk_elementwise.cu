@@ -733,12 +733,15 @@ extern "C" int bcosk_avgpool_fwd(const void* x, int32_t nb, int32_t h, int32_t w
   const int lpp = lanes_per_pixel(c);
   if (!x || !y || lpp == 0) return set_error(BCOSK_EUNSUPPORTED, "avgpool_fwd: c must be a positive multiple of 8");
   if (nb > 65535) return set_error(BCOSK_EUNSUPPORTED, "avgpool_fwd: batch too large for the grid");
+  if (op < 1 || oq < 1) return set_error(BCOSK_EINVAL, "avgpool_fwd: empty output");
   {
     // row-staged kernel: <= 32 lanes per pixel, k full input rows (all planes) fit shared memory
     const size_t smem_row = (size_t)k * w * planes * c * 2;
     if (c / 8 <= 32 && (c / 8 & (c / 8 - 1)) == 0 && c % 8 == 0 && smem_row <= 100 * 1024 && op <= 32767) {
-      // long rows: two or three CTAs per output row (<= ~44 KB each: five CTAs per SM instead of two)
-      const int split = smem_row > 88 * 1024 ? 3 : (smem_row > 44 * 1024 ? 2 : 1);
+      // long rows: two or three CTAs per output row (<= ~44 KB each: five CTAs per SM instead of two); never more parts than
+      // output columns, or a part would own no column and stage a negative input range (a global 7 x 7 pool has oq = 1)
+      int split = smem_row > 88 * 1024 ? 3 : (smem_row > 44 * 1024 ? 2 : 1);
+      if (split > oq) split = oq;
       const int span = ((oq + split - 1) / split - 1) * stride + k + stride;          // input pixels one part reads (upper bound)
       size_t smem = (size_t)k * (span < w ? span : w) * planes * c * 2;
       if (smem > 48 * 1024) {

@@ -31,13 +31,9 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+import opsutil
 from bcos_b200 import _lib as L
-from bcos_b200.engine import CLIPViTPlan, DenseNetPlan, ResNetPlan, ViTPlan
 from bcos_b200.engine import ops as O
-from bcos_b200.engine.clip_rn import CLIPResNetPlan
-from bcos_b200.models import (clip_rn_state_shapes, clip_vit_state_shapes, densenet_state_shapes, resnet_state_shapes,
-                              vit_state_shapes)
-from bcos_b200.utils import synth
 
 U = 2.0 ** -24
 DT = {"fp16": torch.float16, "bf16": torch.bfloat16}
@@ -65,36 +61,8 @@ def _ratio(err, bound) -> float:
 # ---------------------------------------------------------------------------------------------------------------------
 # 16-bit planes
 # ---------------------------------------------------------------------------------------------------------------------
-def _store_rel(dtype: str, planes: int) -> float:
-    return 2.0 ** (-(11 if dtype == "fp16" else 8) * planes)
-
-
-def _store_floor(dtype: str, planes: int) -> float:
-    return planes * 2.0 ** -25 if dtype == "fp16" else 0.0
-
-
-def _planes(t, planes, c):
-    """[..., planes * c] 16-bit -> list of `planes` [..., c] views"""
-    return [t[..., p * c:(p + 1) * c] for p in range(planes)]
-
-
-def _joined(t, planes, c):
-    return sum(p.double() for p in _planes(t, planes, c))
-
-
-def _check_residual_planes(t, planes, c, what):
-    """every plane after the first is the round-to-nearest residual of the planes before it"""
-    ps = _planes(t, planes, c)
-    for i in range(planes - 1):
-        a = ps[i].abs()
-        ulp = (torch.nextafter(a, torch.full_like(a, math.inf)) - a).double()
-        bad = (ps[i + 1].double().abs() > ulp / 2).sum().item()
-        assert bad == 0, (what, f"plane {i + 1} is not the residual of plane {i}", bad)
-
-
-def _store_bound(v64, e, dtype, planes):
-    """bound of a stored value whose fp32 computation is within e of v64"""
-    return e + _store_rel(dtype, planes) * (v64.abs() + e) + _store_floor(dtype, planes)
+_store_rel, _store_floor, _planes, _joined = opsutil.store_rel, opsutil.store_floor, opsutil.split_planes, opsutil.joined
+_check_residual_planes, _store_bound = opsutil.check_residual_planes, opsutil.store_bound
 
 
 @functools.lru_cache(maxsize=None)
@@ -130,34 +98,7 @@ def _x_err(u8_input: bool) -> float:
 # ---------------------------------------------------------------------------------------------------------------------
 # geometries, from the plans
 # ---------------------------------------------------------------------------------------------------------------------
-@functools.lru_cache(maxsize=None)
-def _plan_ops():
-    """[(tag, op)] of the forward and explanation launches of the plans (built on the host at batch 1; only shapes are read)"""
-    out = []
-    sd50 = synth.synth_state_dict(resnet_state_shapes("resnet50"), 0)
-    for size in (224, 448):
-        for mode in ("parity", "throughput"):
-            for u8 in (False, True):
-                p = ResNetPlan("resnet50", sd50, 1, mode=mode, device="cpu", image_size=size, input_u8=u8, want_rgba=True)
-                out += [(f"resnet50@{size}/{mode}/{'u8' if u8 else 'f32'}", op) for op in p.fwd_ops + p.bwd_ops]
-    p = DenseNetPlan("densenet121", synth.synth_state_dict(densenet_state_shapes("densenet121"), 0), 1, mode="parity", device="cpu")
-    out += [("densenet121@224", op) for op in p.fwd_ops + p.bwd_ops]
-    csd = synth.synth_state_dict(clip_rn_state_shapes(), 0)
-    for fused in (True, False):
-        p = CLIPResNetPlan(csd, 1, mode="parity", device="cpu", fused_head=fused)
-        out += [(f"clip_rn50@224/{'fused' if fused else 'module'}_head", op) for op in p.fwd_ops + p.bwd_ops]
-    vsd = synth.synth_state_dict(vit_state_shapes("simple_vit_ti_patch16_224"), 0)
-    for size in (224, 256):
-        p = ViTPlan("simple_vit_ti_patch16_224", vsd, 1, mode="parity", device="cpu", image_size=size)
-        out += [(f"vit_ti@{size}", op) for op in p.fwd_ops + p.bwd_ops]
-    csd = synth.synth_state_dict(clip_vit_state_shapes(224, 32, 128, 2, 64), 0)
-    p = CLIPViTPlan(csd, 1, heads=2, mode="parity", device="cpu")
-    out += [("clip_vit_b32@224", op) for op in p.fwd_ops + p.bwd_ops]
-    return out
-
-
-def _ops_of(kind):
-    return [(tag, op) for tag, op in _plan_ops() if isinstance(op, kind)]
+_ops_of = opsutil.ops_of
 
 
 # =====================================================================================================================
