@@ -346,6 +346,16 @@ def sgemm_batched(trans_a, trans_b, m, n, k, a_ptr, lda, stride_a, b_ptr, ldb, s
                                      C.c_int64(stride_c), batch, C.c_float(alpha), _stream()), "bcosk_sgemm_batched")
 
 
+def sgemm_batched_acc(trans_a, trans_b, m, n, k, a_ptr, lda, stride_a, b_ptr, ldb, stride_b, c_ptr, ldc, stride_c, batch, alpha) -> None:
+    check(load().bcosk_sgemm_batched_acc(int(trans_a), int(trans_b), m, n, k, C.c_void_p(a_ptr), C.c_int64(lda), C.c_int64(stride_a),
+                                         C.c_void_p(b_ptr), C.c_int64(ldb), C.c_int64(stride_b), C.c_void_p(c_ptr), C.c_int64(ldc),
+                                         C.c_int64(stride_c), batch, C.c_float(alpha), _stream()), "bcosk_sgemm_batched_acc")
+
+
+def softmax_bwd(p, dp, rows, n, ds) -> None:
+    check(load().bcosk_softmax_bwd(_p(p), _p(dp), C.c_int64(rows), n, _p(ds), _stream()), "bcosk_softmax_bwd")
+
+
 def head_tokens(x, nb, npix, c, planes, dtype, tokens) -> None:
     check(load().bcosk_head_tokens(_p(x), nb, npix, c, planes, dtype, _p(tokens), _stream()), "bcosk_head_tokens")
 
@@ -497,6 +507,11 @@ def train_bwd_apply(ga, ga_f32, gb, xpost, tn, relu, out, out_f32, scale, alpha,
 
 def grad_combine(ga, gb, x, tn, rows, c, out, dtype) -> None:
     check(load().bcosk_grad_combine(_p(ga), _p(gb), _p(x), _p(tn), C.c_int64(rows), c, _p(out), dtype, _stream()), "bcosk_grad_combine")
+
+
+def pool_bwd_norm(ga, ga_f32, gb, xp, tn, nb, h, w, c, k, accumulate, gx, dtype) -> None:
+    check(load().bcosk_pool_bwd_norm(_p(ga), int(ga_f32), _p(gb), _p(xp), _p(tn), nb, h, w, c, k, int(accumulate), _p(gx), dtype, _stream()),
+          "bcosk_pool_bwd_norm")
 
 
 def sumpool_transpose(gnt, nb, h, w, k, stride, pad, op, oq, accumulate, tn) -> None:

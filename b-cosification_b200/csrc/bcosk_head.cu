@@ -21,7 +21,7 @@ static inline cudaStream_t SH(void* s) { return reinterpret_cast<cudaStream_t>(s
 template <bool TA, bool TB, int TM>
 __global__ void __launch_bounds__(256)
 sgemm_batched_kernel(int M, int N, int K, const float* __restrict__ A, long long lda, long long sA, const float* __restrict__ B, long long ldb,
-                     long long sB, float* __restrict__ C, long long ldc, long long sC, float alpha) {
+                     long long sB, float* __restrict__ C, long long ldc, long long sC, float alpha, int accumulate) {
   constexpr int R = TM / 16;                       // outputs per thread and dimension (4 for 64 x 64 tiles, 2 for 32 x 32)
   __shared__ float As[16][TM + 4];
   __shared__ float Bs[16][TM + 4];
@@ -71,7 +71,7 @@ sgemm_batched_kernel(int M, int N, int K, const float* __restrict__ A, long long
 #pragma unroll
     for (int j = 0; j < R; ++j) {
       const int n = n0 + tx * R + j;
-      if (n < N) C[(size_t)m * ldc + n] = alpha * acc[i][j];
+      if (n < N) C[(size_t)m * ldc + n] = accumulate ? C[(size_t)m * ldc + n] + alpha * acc[i][j] : alpha * acc[i][j];
     }
   }
 }
@@ -112,6 +112,20 @@ __global__ void row_softmax_kernel(float* __restrict__ s, long long rows, int n)
   sum = warp_sum(sum);
   const float inv = 1.0f / sum;
   for (int j = lane; j < n; j += 32) r[j] *= inv;
+}
+
+// softmax backward per row of n: ds = p * (dp - sum_j p_j dp_j) (one warp per row, fixed reduction order; ds may alias dp)
+__global__ void softmax_bwd_kernel(const float* __restrict__ p, const float* dp, long long rows, int n, float* ds) {
+  const long long row = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (row >= rows) return;
+  const int lane = threadIdx.x & 31;
+  const float* pr = p + row * n;
+  const float* dr = dp + row * n;
+  float dot = 0.f;
+  for (int j = lane; j < n; j += 32) dot = fmaf(__ldg(pr + j), dr[j], dot);
+  dot = warp_sum(dot);
+  float* out = ds + row * n;
+  for (int j = lane; j < n; j += 32) out[j] = __ldg(pr + j) * (dr[j] - dot);
 }
 
 // gradient wrt the trunk output pixels from the gradient wrt the tokens: g[img][pix][ch] = gt[img][pix + 1][ch] + gt[img][0][ch] / npix,
@@ -195,9 +209,9 @@ __global__ void seed_from_tokens_kernel(const float* __restrict__ gt, int nb, in
 
 using namespace bcosk;
 
-extern "C" int bcosk_sgemm_batched(int32_t trans_a, int32_t trans_b, int32_t m, int32_t n, int32_t k, const float* a, int64_t lda,
-                                   int64_t stride_a, const float* b, int64_t ldb, int64_t stride_b, float* c, int64_t ldc, int64_t stride_c,
-                                   int32_t batch, float alpha, void* stream) {
+static int sgemm_batched(int32_t trans_a, int32_t trans_b, int32_t m, int32_t n, int32_t k, const float* a, int64_t lda, int64_t stride_a,
+                         const float* b, int64_t ldb, int64_t stride_b, float* c, int64_t ldc, int64_t stride_c, int32_t batch, float alpha,
+                         int accumulate, void* stream) {
   if (!a || !b || !c || m < 1 || n < 1 || k < 1 || batch < 1 || batch > 65535) return set_error(BCOSK_EINVAL, "sgemm_batched: bad argument");
   // few 64 x 64 tiles (the projections of 512 mean tokens: 128-256 CTAs looping over K = 2048) leave SMs idle: 32 x 32 tiles then
   const long long tiles64 = (long long)((n + 63) / 64) * ((m + 63) / 64) * batch;
@@ -206,14 +220,26 @@ extern "C" int bcosk_sgemm_batched(int32_t trans_a, int32_t trans_b, int32_t m, 
   if (grid.y > 65535) return set_error(BCOSK_EUNSUPPORTED, "sgemm_batched: m too large for the grid");
 #define SG(TA_, TB_)                                                                                                                   \
   do {                                                                                                                                 \
-    if (tm == 32) sgemm_batched_kernel<TA_, TB_, 32><<<grid, 256, 0, SH(stream)>>>(m, n, k, a, lda, stride_a, b, ldb, stride_b, c, ldc, stride_c, alpha); \
-    else sgemm_batched_kernel<TA_, TB_, 64><<<grid, 256, 0, SH(stream)>>>(m, n, k, a, lda, stride_a, b, ldb, stride_b, c, ldc, stride_c, alpha);          \
+    if (tm == 32) sgemm_batched_kernel<TA_, TB_, 32><<<grid, 256, 0, SH(stream)>>>(m, n, k, a, lda, stride_a, b, ldb, stride_b, c, ldc, stride_c, alpha, accumulate); \
+    else sgemm_batched_kernel<TA_, TB_, 64><<<grid, 256, 0, SH(stream)>>>(m, n, k, a, lda, stride_a, b, ldb, stride_b, c, ldc, stride_c, alpha, accumulate);          \
   } while (0)
   if (trans_a) { if (trans_b) SG(true, true); else SG(true, false); }
   else { if (trans_b) SG(false, true); else SG(false, false); }
 #undef SG
   BCOSK_CUDA_CHECK(cudaGetLastError());
   return BCOSK_OK;
+}
+
+extern "C" int bcosk_sgemm_batched(int32_t trans_a, int32_t trans_b, int32_t m, int32_t n, int32_t k, const float* a, int64_t lda,
+                                   int64_t stride_a, const float* b, int64_t ldb, int64_t stride_b, float* c, int64_t ldc, int64_t stride_c,
+                                   int32_t batch, float alpha, void* stream) {
+  return sgemm_batched(trans_a, trans_b, m, n, k, a, lda, stride_a, b, ldb, stride_b, c, ldc, stride_c, batch, alpha, 0, stream);
+}
+
+extern "C" int bcosk_sgemm_batched_acc(int32_t trans_a, int32_t trans_b, int32_t m, int32_t n, int32_t k, const float* a, int64_t lda,
+                                       int64_t stride_a, const float* b, int64_t ldb, int64_t stride_b, float* c, int64_t ldc, int64_t stride_c,
+                                       int32_t batch, float alpha, void* stream) {
+  return sgemm_batched(trans_a, trans_b, m, n, k, a, lda, stride_a, b, ldb, stride_b, c, ldc, stride_c, batch, alpha, 1, stream);
 }
 
 extern "C" int bcosk_head_tokens(const void* x, int32_t nb, int32_t npix, int32_t c, int32_t planes, int32_t dtype, float* tokens, void* stream) {
@@ -229,6 +255,13 @@ extern "C" int bcosk_head_tokens(const void* x, int32_t nb, int32_t npix, int32_
 extern "C" int bcosk_row_softmax(float* s, int64_t rows, int32_t n, void* stream) {
   if (!s || rows < 1 || n < 1) return set_error(BCOSK_EINVAL, "row_softmax: bad argument");
   row_softmax_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, SH(stream)>>>(s, rows, n);
+  BCOSK_CUDA_CHECK(cudaGetLastError());
+  return BCOSK_OK;
+}
+
+extern "C" int bcosk_softmax_bwd(const float* p, const float* dp, int64_t rows, int32_t n, float* ds, void* stream) {
+  if (!p || !dp || !ds || rows < 1 || n < 1) return set_error(BCOSK_EINVAL, "softmax_bwd: bad argument");
+  softmax_bwd_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, SH(stream)>>>(p, dp, rows, n, ds);
   BCOSK_CUDA_CHECK(cudaGetLastError());
   return BCOSK_OK;
 }

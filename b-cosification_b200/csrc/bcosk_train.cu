@@ -296,6 +296,40 @@ __global__ void grad_combine_kernel(const T* __restrict__ gA, const T* __restric
   *reinterpret_cast<uint4*>(out + row * C + g * 8) = pack8<T>(f);
 }
 
+// Backward of AvgPool2d(k) (stride k, no padding: the anti-aliasing pools of the CLIP ResNets) fused with the consumers' terms
+// at the pooled resolution: gx[img, y, x, :] (+)= (gA + gB + xp * T)[img, y / k, x / k, :] / k^2.  One thread per input pixel and
+// 8 channels; pixels past the last full window get zero.  Every output element is written by one thread (no atomics).
+template <typename T>
+__global__ void pool_bwd_norm_kernel(const void* __restrict__ gA, int ga_f32, const T* __restrict__ gB, const T* __restrict__ xp,
+                                     const float* __restrict__ Tn, int nb, int h, int w, int C, int k, int accumulate, T* __restrict__ gx) {
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  const int G = C >> 3;
+  if (idx >= (long long)nb * h * w * G) return;
+  const long long pix = idx / G;
+  const int g = (int)(idx - pix * G);
+  const int x = (int)(pix % w), y = (int)((pix / w) % h), img = (int)(pix / ((long long)w * h));
+  const int op = h / k, oq = w / k;
+  float f[8];
+  if (y / k < op && x / k < oq) {
+    const size_t row = ((size_t)img * op + y / k) * oq + x / k;
+    grad_in8<T>(gA, ga_f32 != 0, gB, xp, Tn, 0, row, C, g * 8, f);
+    const float inv = 1.0f / (float)(k * k);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) f[i] *= inv;
+  } else {
+#pragma unroll
+    for (int i = 0; i < 8; ++i) f[i] = 0.f;
+  }
+  uint4* dst = reinterpret_cast<uint4*>(gx + (size_t)pix * C + g * 8);
+  if (accumulate) {
+    float o[8];
+    unpack8<T>(*dst, o);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) f[i] += o[i];
+  }
+  *dst = pack8<T>(f);
+}
+
 // T[img, y, x] (+)= sum over the output pixels (p, q) whose k x k window (stride, pad) covers (y, x) of gnT[img, p, q]
 __global__ void sumpool_transpose_kernel(const float* __restrict__ gnT, int nb, int h, int w, int k, int stride, int pad, int op, int oq,
                                          int accumulate, float* __restrict__ Tn) {
@@ -573,6 +607,17 @@ extern "C" int bcosk_grad_combine(const void* ga, const void* gb, const void* x,
   BCOSK_T_SWITCH(dtype, grad_combine_kernel<T><<<grid_for(rows * (c / 8), 256), 256, 0, S_(stream)>>>(
       reinterpret_cast<const T*>(ga), reinterpret_cast<const T*>(gb), reinterpret_cast<const T*>(x), tn, rows, c,
       reinterpret_cast<T*>(out));)
+  BCOSK_CUDA_CHECK(cudaGetLastError());
+  return BCOSK_OK;
+}
+
+extern "C" int bcosk_pool_bwd_norm(const void* ga, int32_t ga_f32, const void* gb, const void* x, const float* tn, int32_t nb, int32_t h,
+                                   int32_t w, int32_t c, int32_t k, int32_t accumulate, void* gx, int32_t dtype, void* stream) {
+  if (!ga || !gx || nb < 1 || h < k || w < k || k < 1 || c < 8 || c % 8 != 0 || (tn && !x))
+    return set_error(BCOSK_EINVAL, "pool_bwd_norm: bad argument");
+  const long long n = (long long)nb * h * w * (c / 8);
+  BCOSK_T_SWITCH(dtype, pool_bwd_norm_kernel<T><<<grid_for(n, 256), 256, 0, S_(stream)>>>(
+      ga, ga_f32, reinterpret_cast<const T*>(gb), reinterpret_cast<const T*>(x), tn, nb, h, w, c, k, accumulate, reinterpret_cast<T*>(gx));)
   BCOSK_CUDA_CHECK(cudaGetLastError());
   return BCOSK_OK;
 }

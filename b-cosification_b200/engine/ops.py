@@ -677,9 +677,10 @@ class SgemmOp:
     stride_c: int
     batch: int
     alpha: float = 1.0
+    accumulate: bool = False     # C += alpha * op(A) op(B)
 
     def run(self) -> None:
-        L.sgemm_batched(self.trans_a, self.trans_b, self.m, self.n, self.k, self.a.data_ptr() + 4 * self.a_off, self.lda, self.stride_a,
+        (L.sgemm_batched_acc if self.accumulate else L.sgemm_batched)(self.trans_a, self.trans_b, self.m, self.n, self.k, self.a.data_ptr() + 4 * self.a_off, self.lda, self.stride_a,
                         self.b.data_ptr() + 4 * self.b_off, self.ldb, self.stride_b, self.c.data_ptr() + 4 * self.c_off, self.ldc,
                         self.stride_c, self.batch, self.alpha)
 

@@ -1,6 +1,7 @@
 """Fine-tuning step of a B-cosified ResNet or DenseNet (SURVEY 8f row 2, BASELINE config 5): forward in train mode, loss, full
 backward, gradient all-reduce, adaptive gradient clipping + AdamW - one process per GPU, batch sharded, NCCL for the gradients.
-`ResNetTrainPlan` and `DenseNetTrainPlan` share `TrainPlanBase`; the DenseNet's own kernels are described at its class.
+`ResNetTrainPlan`, `DenseNetTrainPlan` and `CLIPResNetTrainPlan` (engine/clip_train.py) share `TrainPlanBase`; the DenseNet's own
+kernels are described at its class.
 
 Reference: `training_step` bcos/training/trainer.py:666-784 (outputs = model(images); loss = criterion(outputs, labels)),
 autograd backward through `BcosifyConv2d.forward_impl` (bcosifyconv2d.py:50-102, scale NOT detached) and
@@ -141,6 +142,7 @@ class TrainPlanBase(PlanBase):
         self._cur_w_off = 0
         self._w_items: List[Tuple[str, Tensor, int]] = []     # (state-dict key, fp32 tensor, offset)
         self.norm_units: List[Tuple[int, int, int]] = []      # (master offset, gradient offset, c) of BN weights not owned by a TrainLayer
+        self.row_units: List[Tuple[int, int, int, int]] = []  # (master offset, gradient offset, rows, cols) of fp32 matrices used unpacked
         self.opt_ops: List = []
         self.running_var: Dict[str, Tensor] = {}
         self.w_flat = None                    # allocated after all weights are registered (closures read self.w_flat late)
@@ -377,6 +379,8 @@ class TrainPlanBase(PlanBase):
                 gidx[lay.bnw_off:lay.bnw_off + o] = lay.gbn_off + torch.arange(o)
         for w_off, g_off, c in self.norm_units:
             gidx[w_off:w_off + c] = g_off + torch.arange(c)
+        for w_off, g_off, rows, cols in self.row_units:
+            gidx[w_off:w_off + rows * cols] = g_off + torch.arange(rows * cols)
         assert int((gidx < 0).sum()) == 0, "a master weight without a gradient slot"
         self.gidx = gidx.to(torch.int32).to(self.device)
         # ---- AGC + AdamW of the WHOLE model in one launch: one unit = one output row of a conv / the whole BN weight vector
@@ -393,6 +397,9 @@ class TrainPlanBase(PlanBase):
         for w_off, _, c in self.norm_units:
             u_off.append(w_off)
             u_cols.append(c)
+        for w_off, _, rows, cols in self.row_units:
+            u_off += [w_off + i * cols for i in range(rows)]
+            u_cols += [cols] * rows
         self.unit_off = torch.tensor(u_off, dtype=torch.int64, device=self.device)
         self.unit_cols = torch.tensor(u_cols, dtype=torch.int32, device=self.device)
         self.adam_state = self._zeros(3, dtype=torch.float32)          # {step, 1 - beta1^step, 1 - beta2^step}

@@ -299,6 +299,14 @@ int bcosk_train_bwd_apply(const void* ga, int32_t ga_f32, const void* gb, const 
 /* out = ga + gb + x * tn[row] (16-bit rows; gb / tn optional): gradient of a tensor that is not a norm layer's output */
 int bcosk_grad_combine(const void* ga, const void* gb, const void* x, const float* tn, int64_t rows, int32_t c, void* out,
                        int32_t dtype, void* stream);
+/* Backward of AvgPool2d(k) (stride k, no padding; CLIP/clip/model.py:10-55 Bottleneck.avgpool and the downsample's AvgPool2d,
+ * model.py:140-145 the stem's AvgPool2d(2)) fused with the consumers' terms at the pooled resolution, which the pool's output
+ * receives like any conv input (ga + gb + x * tn, see bcosk_train_bwd_reduce):
+ *   gx[img, y, x, :] (+)= (ga + gb + xp * tn[row])[img, y / k, x / k, :] / k^2        (pixels past the last full window: 0)
+ * ga [nb*op*oq, c] 16-bit or fp32 (ga_f32), gb / xp 16-bit (optional), tn fp32 [nb*op*oq] (optional, needs xp), op = h / k,
+ * oq = w / k; gx [nb, h, w, c] 16-bit, added to when accumulate.  One writer per element: bit-reproducible. */
+int bcosk_pool_bwd_norm(const void* ga, int32_t ga_f32, const void* gb, const void* xp, const float* tn, int32_t nb, int32_t h,
+                        int32_t w, int32_t c, int32_t k, int32_t accumulate, void* gx, int32_t dtype, void* stream);
 /* tn[img, y, x] (+)= sum of gnt over the output pixels whose k x k window (stride, pad) covers input pixel (y, x) */
 int bcosk_sumpool_transpose(const float* gnt, int32_t nb, int32_t h, int32_t w, int32_t k, int32_t stride, int32_t pad,
                             int32_t op, int32_t oq, int32_t accumulate, float* tn, void* stream);
@@ -561,13 +569,20 @@ int bcosk_dense_slice_bwd(const float* G, const void* F, int32_t ld, int32_t col
 int bcosk_sgemm_batched(int32_t trans_a, int32_t trans_b, int32_t m, int32_t n, int32_t k, const float* a, int64_t lda, int64_t stride_a,
                         const float* b, int64_t ldb, int64_t stride_b, float* c, int64_t ldc, int64_t stride_c, int32_t batch, float alpha,
                         void* stream);
+/* The same, adding into C: C[i] += alpha * op(A[i]) * op(B[i]). */
+int bcosk_sgemm_batched_acc(int32_t trans_a, int32_t trans_b, int32_t m, int32_t n, int32_t k, const float* a, int64_t lda,
+                            int64_t stride_a, const float* b, int64_t ldb, int64_t stride_b, float* c, int64_t ldc, int64_t stride_c,
+                            int32_t batch, float alpha, void* stream);
 /* tokens [nb][npix + 1][c] fp32 from the trunk output planes x [nb][npix][planes * c]: token 0 = mean over the pixels
  * (bcosattnpool.py:37-38: cat([x.mean(0), x])), token j + 1 = pixel j. */
 int bcosk_head_tokens(const void* x, int32_t nb, int32_t npix, int32_t c, int32_t planes, int32_t dtype, float* tokens, void* stream);
 /* in-place softmax over rows of n fp32 values */
 int bcosk_row_softmax(float* s, int64_t rows, int32_t n, void* stream);
+/* Backward of the row softmax (the attention weights p = softmax(s), bcosattnpool.py:48-50 through F.multi_head_attention_forward,
+ * with q and k in the graph as in training): ds = p * (dp - sum_j p_j dp_j) per row of n fp32 values; ds may alias dp. */
+int bcosk_softmax_bwd(const float* p, const float* dp, int64_t rows, int32_t n, float* ds, void* stream);
 /* Gradient wrt the tokens g_tokens [nb][npix + 1][c] fp32 -> the last trunk block's gradient tensors (see bcosk_seed_from_nchw):
- * g[pix] = g_tokens[pix + 1] + g_tokens[0] / npix;  out1 = planes(g * scale * mul1), out2 = planes(g * scale [* mul2]) under mask2. */
+ * g[pix] = g_tokens[pix + 1] + g_tokens[0] / npix;  out1 = planes(g * scale * mul1) (mul1 NULL: 1), out2 = planes(g * scale [* mul2]) under mask2. */
 int bcosk_seed_from_tokens(const float* g_tokens, int32_t nb, int32_t npix, int32_t c, float scale, const void* mul1, int32_t mul1_f32,
                            void* out1, const uint32_t* mask2, const void* mul2, int32_t mul2_f32, void* out2, int32_t planes,
                            int32_t dtype, void* stream);
