@@ -62,7 +62,7 @@ def _file_digest(path: str, extra: str) -> str:
 def build(force: bool = False, verbose: bool = False) -> str:
     """Compile libbcosk.so if sources changed; returns the library path.  Every translation unit is compiled to its own
     object (in parallel, only those whose source or headers changed), then linked.
-    $BCOSK_EXTRA_NVCC_FLAGS (e.g. -DBCOSK_TIMING, experiments only) is appended to the nvcc command line."""
+    $BCOSK_EXTRA_NVCC_FLAGS (experiments only) is appended to the nvcc command line."""
     from concurrent.futures import ThreadPoolExecutor
     extra = os.environ.get("BCOSK_EXTRA_NVCC_FLAGS", "").split()
     dig = _digest() + "|" + " ".join(extra)

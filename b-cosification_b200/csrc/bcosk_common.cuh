@@ -84,15 +84,6 @@ __device__ __forceinline__ void tma_load_4d(void* smem_dst, const void* desc, ui
       ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(desc)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
       : "memory");
 }
-// Same, delivered to the same shared-memory offset (and signalled on the same barrier offset) of every CTA in `mask`.
-__device__ __forceinline__ void tma_load_2d_mc(void* smem_dst, const void* desc, uint64_t* bar, int32_t c0, int32_t c1,
-                                               uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-      " [%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(desc)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
 // 4-D im2col load over an NHWC tensor described as (C, W, H, N); (off_w, off_h) = filter tap offset
 __device__ __forceinline__ void tma_load_im2col_4d(void* smem_dst, const void* desc, uint64_t* bar, int32_t c,
                                                    int32_t w, int32_t h, int32_t n, uint16_t off_w, uint16_t off_h) {
@@ -168,82 +159,6 @@ __device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t desc_a, uint6
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
                : "memory");
-}
-// Same, arriving on the barrier at this offset in every CTA of `mask` (thread-block cluster).
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                   smem_u32(bar)),
-               "h"(mask)
-               : "memory");
-}
-// ---- CTA pair (cta_group::2): two CTAs of a cluster on the two SMs of a TPC run ONE 256-row MMA; each holds its 128
-// rows of A and half of the B rows in its own shared memory, the leader (rank 0) issues, D lands in both TMEMs.
-__device__ __forceinline__ void tmem_alloc_2cta(uint32_t* smem_dst, uint32_t ncols) {   // one warp in EACH CTA, same dst offset
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_dst)), "r"(ncols)
-               : "memory");
-}
-__device__ __forceinline__ void tmem_relinquish_2cta() {
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_2cta(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void umma_f16_2cta(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                              uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
-      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit_2cta(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                   smem_u32(bar)),
-               "h"(mask)
-               : "memory");
-}
-// shared::cluster address of the same offset in CTA `rank` of the cluster
-__device__ __forceinline__ uint32_t mapa_u32(uint32_t smem_addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// pair loads: data into THIS CTA's shared memory, bytes counted on the barrier at `bar_cluster_addr` (the leader's)
-__device__ __forceinline__ void tma_load_2d_2cta(void* smem_dst, const void* desc, uint32_t bar_cluster_addr, int32_t c0,
-                                                 int32_t c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(desc)), "r"(bar_cluster_addr), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_im2col_4d_2cta(void* smem_dst, const void* desc, uint32_t bar_cluster_addr, int32_t c,
-                                                        int32_t w, int32_t h, int32_t n, uint16_t off_w, uint16_t off_h) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.im2col.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes"
-      " [%0], [%1, {%3, %4, %5, %6}], [%2], {%7, %8};"
-      ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(desc)), "r"(bar_cluster_addr), "r"(c), "r"(w), "r"(h),
-      "r"(n), "h"(off_w), "h"(off_h)
-      : "memory");
-}
-// Programmatic dependent launch: a grid launched with the programmatic-serialization attribute may start while its
-// predecessor is still draining; grid_dependency_wait() blocks until the predecessor has completed and its writes are
-// visible (no-op without the attribute), grid_launch_dependents() lets the successor's CTAs be scheduled as soon as every
-// CTA of this grid has started.
-__device__ __forceinline__ void grid_dependency_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void grid_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-// all threads of all CTAs of the cluster
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
 // TMEM -> registers: this warp's 32 lanes x 32 consecutive fp32 columns (thread i <- lane base+i).
 __device__ __forceinline__ void tmem_ld_32x32(uint32_t taddr, uint32_t (&r)[32]) {

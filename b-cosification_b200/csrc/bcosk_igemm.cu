@@ -35,10 +35,6 @@ constexpr int NUM_THREADS = 192;
 #define BCOSK_BN128_STAGES 2
 #define BCOSK_BN128_BLOCKS 3
 #endif
-#ifndef BCOSK_BN256_STAGES
-#define BCOSK_BN256_STAGES 4   // 256-wide per-tile kernel (experiment knobs; the plans do not pick 256-wide tiles)
-#define BCOSK_BN256_BLOCKS 1
-#endif
 #ifndef BCOSK_LIGHT2_BLOCKS
 #define BCOSK_LIGHT2_BLOCKS 4   // CTAs per SM of the single-stage forward variant (5 spills ~200 B per thread)
 #endif
@@ -48,62 +44,25 @@ constexpr int NUM_THREADS = 192;
 // LIGHT = 2: two slots and 4 CTAs per SM for forward launches whose K loop is ONE stage (K = 64).  Slot 0 is the stage and
 // afterwards the y tile; slot 1 holds the residual tile and the gain tile is staged over it - every thread reads its own
 // residual words before it writes the same words of the gain tile, so the alias is safe.
-#ifndef BCOSK_HP_CHUNK
-#define BCOSK_HP_CHUNK 1   // pipeline stages (64 K-elements each) accumulated by the tensor core before the epilogue warps drain them
-#endif
-template <int BN, bool HP = false, int LIGHT = 0> struct TileCfg {
-  static constexpr int kStages = LIGHT == 2 ? 2 : (LIGHT ? 3 : ((BN == 128) ? BCOSK_BN128_STAGES : (BN == 256 ? BCOSK_BN256_STAGES : 4)));   // pipeline slots; the last may hold the input tile
-  static constexpr int kMinBlocks = LIGHT == 2 ? BCOSK_LIGHT2_BLOCKS : (LIGHT ? 3 : (BN == 128 ? BCOSK_BN128_BLOCKS : ((BN < 128) ? 2 : BCOSK_BN256_BLOCKS)));
+template <int BN, int LIGHT = 0> struct TileCfg {
+  static constexpr int kStages = LIGHT == 2 ? 2 : (LIGHT ? 3 : (BN == 128 ? BCOSK_BN128_STAGES : 4));   // pipeline slots; the last may hold the input tile
+  static constexpr int kMinBlocks = LIGHT == 2 ? BCOSK_LIGHT2_BLOCKS : (LIGHT ? 3 : (BN == 128 ? BCOSK_BN128_BLOCKS : 2));
   static constexpr int kBStageBytes = BN * STAGE_K * 2;
   static constexpr int kSlotBytes = A_STAGE_BYTES + kBStageBytes;   // A stage followed by its B stage
   static constexpr int kTileBytes = BM * BN * 2;                    // one 16-bit epilogue tile (BN/64 boxes of 16 KB)
-  static constexpr bool kTmaEpilogue = !HP && (BN == 64 || BN == 128);
-  // HP (high-precision accumulation): two TMEM accumulators that the epilogue warps drain every pipeline stage
-  static constexpr int kTmemCols = (BN < 32 ? 32 : BN) * (HP ? 2 : 1);
+  static constexpr bool kTmaEpilogue = BN == 64 || BN == 128;
+  static constexpr int kTmemCols = BN;                              // one fp32 accumulator column per tile column
   static constexpr int kBarOffset = kStages * (A_STAGE_BYTES + kBStageBytes);
   // stages + 1 KB alignment slack + barriers/params
   static constexpr int kSmemBytes = kBarOffset + 1024 + 256 + 2 * BN * 4;
 };
 
-#ifdef BCOSK_TIMING2
-#define BCOSK_TIMING
-#endif
-#ifdef BCOSK_TIMING
-// Experiment-only instrumentation (never in the shipped library): per-CTA clock64 stamps of the per-tile kernel.
-__device__ unsigned long long* g_timing_buf = nullptr;
-__device__ int g_timing_cap = 0;
-#ifdef BCOSK_TIMING2
-#define BCOSK_STAMP(slot) do { } while (0)
-#else
-#define BCOSK_STAMP(slot)                                                                                  \
-  do {                                                                                                     \
-    if (g_timing_buf != nullptr && (int)blockIdx.x < g_timing_cap) g_timing_buf[blockIdx.x * 8 + (slot)] = clock64(); \
-  } while (0)
-#endif
-// accumulate a duration into slot `slot` of this CTA (each slot has one writer thread)
-#define BCOSK_TACC_BEGIN() const long long _tacc0 = clock64()
-#define BCOSK_TACC(slot)                                                                                      \
-  do {                                                                                                        \
-    if (g_timing_buf != nullptr && (int)blockIdx.x < g_timing_cap) g_timing_buf[blockIdx.x * 8 + (slot)] += clock64() - _tacc0; \
-  } while (0)
-#else
-#define BCOSK_STAMP(slot) do { } while (0)
-#define BCOSK_TACC_BEGIN() do { } while (0)
-#define BCOSK_TACC(slot) do { } while (0)
-#endif
-#ifdef BCOSK_TIMING2
-#define BCOSK_TACC2_BEGIN() BCOSK_TACC_BEGIN()
-#define BCOSK_TACC2(slot) BCOSK_TACC(slot)
-#else
-#define BCOSK_TACC2_BEGIN() do { } while (0)
-#define BCOSK_TACC2(slot) do { } while (0)
-#endif
-
-
 // One 32-column slice of one output row: everything after the accumulator is in registers.
-// Generic (scalar) form: any scale mode, precision planes, fp32 side tensors.
+// Generic (scalar) form: any scale mode, precision planes, fp32 side tensors.  An out-of-line call, because in the
+// kernels it serves only as the fallback of the fast form and would otherwise cost them their register budget; the
+// arrays passed by reference live in local memory there.
 template <int MODE, typename T>
-__device__ __forceinline__ void epilogue_chunk_generic_inl(const bcosk_igemm_params& p, const RowInfo& ri, int64_t yrow, float inv_norm,
+__device__ __noinline__ void epilogue_chunk_generic(const bcosk_igemm_params& p, const RowInfo& ri, int64_t yrow, float inv_norm,
                                                int64_t add_row, const float* s_alpha, const float* s_beta, int j, int c0,
                                                int ncols, float (&v)[32], float& sq_acc, const EpiTiles& tl, int row) {
   T* y16 = reinterpret_cast<T*>(p.y);
@@ -221,17 +180,6 @@ __device__ __forceinline__ void epilogue_chunk_generic_inl(const bcosk_igemm_par
       store32_planes<T>(y16 + (size_t)yrow * p.y_ld + c0, p.y_planes, p.y_plane_stride, ncols, v);
     }
   }
-}
-
-
-// Out-of-line copy for the kernels where the generic form is only the fallback (keeps their register budget); the arrays
-// passed by reference live in local memory there.  The parity-mode (HP) kernels call the inline form: ncu showed more
-// local-memory than global-memory sectors in their launches (profiles/r01_parity_mode_ncu.md).
-template <int MODE, typename T>
-__device__ __noinline__ void epilogue_chunk_generic(const bcosk_igemm_params& p, const RowInfo& ri, int64_t yrow, float inv_norm,
-                                               int64_t add_row, const float* s_alpha, const float* s_beta, int j, int c0,
-                                               int ncols, float (&v)[32], float& sq_acc, const EpiTiles& tl, int row) {
-  epilogue_chunk_generic_inl<MODE, T>(p, ri, yrow, inv_norm, add_row, s_alpha, s_beta, j, c0, ncols, v, sq_acc, tl, row);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -482,13 +430,13 @@ __device__ __forceinline__ void epilogue_chunk(const bcosk_igemm_params& p, cons
   }
 }
 
-template <int BN, int MODE, typename T, bool HP, int LIGHT = 0, bool PAIR = false>
-__global__ void __launch_bounds__(NUM_THREADS, TileCfg<BN, HP, LIGHT>::kMinBlocks)
+template <int BN, int MODE, typename T, int LIGHT = 0>
+__global__ void __launch_bounds__(NUM_THREADS, TileCfg<BN, LIGHT>::kMinBlocks)
 bcosk_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                    const __grid_constant__ CUtensorMap tmap_in, const __grid_constant__ CUtensorMap tmap_in2,
                    const __grid_constant__ CUtensorMap tmap_out1, const __grid_constant__ CUtensorMap tmap_out2,
                    const __grid_constant__ bcosk_igemm_params p, const IgemmAux aux) {
-  using Cfg = TileCfg<BN, HP, LIGHT>;
+  using Cfg = TileCfg<BN, LIGHT>;
   constexpr int kSlots = Cfg::kStages;
   extern __shared__ uint8_t smem_raw[];
   // 1024-byte alignment required by the 128B swizzle atoms
@@ -497,10 +445,8 @@ bcosk_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
   // epilogue input tile is prefetched it owns the last slot (the ring then has kSlots-1 stages)
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + Cfg::kBarOffset);
   uint64_t* empty_bar = full_bar + kSlots;
-  uint64_t* tmem_full_bar = empty_bar + kSlots;    // non-HP: accumulator complete
-  uint64_t* acc_full_bar = tmem_full_bar + 1;      // HP: [2] partial accumulator ready
-  uint64_t* acc_empty_bar = acc_full_bar + 2;      // HP: [2] partial accumulator drained
-  uint64_t* in_bar = acc_empty_bar + 2;            // epilogue input tile landed
+  uint64_t* tmem_full_bar = empty_bar + kSlots;    // accumulator complete
+  uint64_t* in_bar = tmem_full_bar + 1;            // epilogue input tile landed
   uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(in_bar + 1);
   float* s_alpha = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(full_bar) + 256);
   float* s_beta = s_alpha + BN;
@@ -508,13 +454,9 @@ bcosk_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int n_tiles = (p.n + BN - 1) / BN;
-  const int cl = aux.cluster > 1 ? aux.cluster : 1;
-  constexpr bool pair = PAIR;                                      // own instantiation (cta_group::2 code needs a cluster launch); implies cl == 2
-  const int cl_rank = (int)(blockIdx.x % (unsigned)cl);            // == %cluster_ctarank for (cl,1,1) clusters
-  const int cl_id = blockIdx.x / cl;
-  const int tile_n = cl_id % n_tiles;
-  const int tile_m = (cl_id / n_tiles) * cl + cl_rank;
-  const uint16_t cl_mask = (uint16_t)((1u << cl) - 1u);
+  const int tile = blockIdx.x;
+  const int tile_n = tile % n_tiles;
+  const int tile_m = tile / n_tiles;
   const int M = p.a_nb * p.op * p.oq;
   const int m0 = tile_m * BM;
   const int n0 = tile_n * BN;
@@ -526,42 +468,26 @@ bcosk_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
   const bool use_in2_tile = use_in_tile && aux.tma_in2 != 0;   // host guarantees >= 2 ring stages remain
   const bool late_in = use_in_tile && !use_in2_tile && aux.late_in != 0;
   const int num_stages = kSlots - ((use_in_tile && !late_in) ? 1 : 0) - (use_in2_tile ? 1 : 0);
-  if (threadIdx.x == 64) BCOSK_STAMP(0);
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmap_a);
     tma_prefetch_desc(&tmap_b);
     for (int s = 0; s < kSlots; ++s) {
-      // pair: the leader's barrier counts both producers' arrivals and both CTAs' bytes; one multicast commit frees a slot
-      mbar_init(&full_bar[s], pair ? 2 : 1);
-      mbar_init(&empty_bar[s], pair ? 1 : cl);   // multicast: free when every CTA that receives this slot's data consumed it
+      mbar_init(&full_bar[s], 1);
+      mbar_init(&empty_bar[s], 1);
     }
     mbar_init(tmem_full_bar, 1);
-    for (int s = 0; s < 2; ++s) {
-      mbar_init(&acc_full_bar[s], 1);
-      mbar_init(&acc_empty_bar[s], 4);  // one arrival per epilogue warp
-    }
     mbar_init(in_bar, 1);
     fence_barrier_init();
   }
   if (warp == 1) {
-    if constexpr (PAIR) {
-      tmem_alloc_2cta(tmem_ptr_smem, Cfg::kTmemCols);
-      tmem_relinquish_2cta();
-    } else {
-      tmem_alloc(tmem_ptr_smem, Cfg::kTmemCols);
-      tmem_relinquish();
-    }
+    tmem_alloc(tmem_ptr_smem, Cfg::kTmemCols);
+    tmem_relinquish();
   }
   tc_fence_before();
   __syncthreads();
-  if (cl > 1) cluster_sync_all();        // peers' barriers exist before any multicast data or remote arrival reaches them
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
-  // everything above touched only parameters, shared memory and TMEM: it may overlap the previous launch's tail
-  grid_launch_dependents();
-  grid_dependency_wait();
-  if (threadIdx.x == 64) BCOSK_STAMP(1);
 
   if (warp == 0) {
     // ===================== TMA producer =====================
@@ -591,43 +517,13 @@ bcosk_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
       int seg = 0, tap = 0, kc = 0;
       for (int it = 0; it < num_iters; ++it) {
         uint8_t* slot = smem + stage * Cfg::kSlotBytes;
-        {
-          BCOSK_TACC2_BEGIN();
-          mbar_wait(&empty_bar[stage], phase ^ 1);
-          BCOSK_TACC2(0);
-        }
-        if constexpr (PAIR) {
-          // both CTAs' stages are counted on the LEADER's barrier (it alone issues the pair MMA)
-          const uint32_t lead_bar = mapa_u32(smem_u32(&full_bar[stage]), 0);
-          if (cl_rank == 0) mbar_arrive_expect_tx(&full_bar[stage], 2 * (A_STAGE_BYTES + (BN / 2) * STAGE_K * 2));
-          else mbar_arrive_remote(lead_bar);
-          const uint32_t b_half_chunk = (BN / 2) * p.kch * 2;
-          for (int j = 0; j < chunks_per_stage; ++j) {
-            const int ci = it * chunks_per_stage + j;
-            tma_load_im2col_4d_2cta(slot + j * a_chunk_bytes, &tmap_a, lead_bar, p.seg_a_choff[seg] + kc * p.kch, base_w,
-                                    base_h, img, p.tap_off_w[tap], p.tap_off_h[tap]);
-            tma_load_2d_2cta(slot + A_STAGE_BYTES + j * b_half_chunk, &tmap_b, lead_bar, ci * p.kch, n0 + cl_rank * (BN / 2));
-            if (++kc == p.chunks_per_tap) {
-              kc = 0;
-              if (++tap == p.num_taps) { tap = 0; ++seg; }
-            }
-          }
-          if (++stage == num_stages) { stage = 0; phase ^= 1; }
-          continue;
-        }
+        mbar_wait(&empty_bar[stage], phase ^ 1);
         mbar_arrive_expect_tx(&full_bar[stage], Cfg::kSlotBytes);
         for (int j = 0; j < chunks_per_stage; ++j) {
           const int ci = it * chunks_per_stage + j;
           tma_load_im2col_4d(slot + j * a_chunk_bytes, &tmap_a, &full_bar[stage], p.seg_a_choff[seg] + kc * p.kch, base_w,
                              base_h, img, p.tap_off_w[tap], p.tap_off_h[tap]);
-          if (cl > 1) {
-            // this CTA's share of the weight tile, delivered to every CTA of the cluster
-            const int rows = BN / cl;
-            tma_load_2d_mc(slot + A_STAGE_BYTES + j * b_chunk_bytes + cl_rank * rows * p.kch * 2, &tmap_b, &full_bar[stage],
-                           ci * p.kch, n0 + cl_rank * rows, cl_mask);
-          } else {
-            tma_load_2d(slot + A_STAGE_BYTES + j * b_chunk_bytes, &tmap_b, &full_bar[stage], ci * p.kch, n0);
-          }
+          tma_load_2d(slot + A_STAGE_BYTES + j * b_chunk_bytes, &tmap_b, &full_bar[stage], ci * p.kch, n0);
           if (++kc == p.chunks_per_tap) {
             kc = 0;
             if (++tap == p.num_taps) { tap = 0; ++seg; }
@@ -648,51 +544,7 @@ bcosk_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
     }
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
-    if constexpr (PAIR) {
-      // CTA pair: the leader issues one 256 x BN MMA per K step over both CTAs' stages; commits reach both CTAs
-      if (lane == 0 && cl_rank == 0) {
-        const uint32_t idesc = umma_idesc_f16((uint32_t)p.dtype, 2 * BM, BN);
-        const uint32_t row_bytes = p.kch * 2;
-        const uint32_t a_chunk_bytes = BM * p.kch * 2;
-        const uint32_t b_half_chunk = (BN / 2) * p.kch * 2;
-        const int mma_per_chunk = p.kch / 16;
-        int stage = 0;
-        uint32_t phase = 0;
-        uint32_t accumulate = 0;
-        for (int it = 0; it < num_iters; ++it) {
-          uint8_t* slot = smem + stage * Cfg::kSlotBytes;
-          {
-            BCOSK_TACC2_BEGIN();
-            mbar_wait(&full_bar[stage], phase);
-            BCOSK_TACC2(1);
-          }
-          tc_fence_after();
-          BCOSK_TACC2_BEGIN();
-          if (chunks_per_stage == 1) {
-            const uint64_t da = umma_smem_desc_kmajor(smem_u32(smem), 128) + (uint64_t)stage * (Cfg::kSlotBytes >> 4);
-            const uint64_t db = da + (A_STAGE_BYTES >> 4);
-            umma_f16_2cta(tmem_base, da, db, idesc, accumulate);
-            umma_f16_2cta(tmem_base, da + 2, db + 2, idesc, 1);
-            umma_f16_2cta(tmem_base, da + 4, db + 4, idesc, 1);
-            umma_f16_2cta(tmem_base, da + 6, db + 6, idesc, 1);
-            accumulate = 1;
-          } else {
-            for (int j = 0; j < chunks_per_stage; ++j) {
-              const uint64_t da = umma_smem_desc_kmajor(smem_u32(slot + j * a_chunk_bytes), row_bytes);
-              const uint64_t db = umma_smem_desc_kmajor(smem_u32(slot + A_STAGE_BYTES + j * b_half_chunk), row_bytes);
-              for (int k = 0; k < mma_per_chunk; ++k) {
-                umma_f16_2cta(tmem_base, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), idesc, accumulate);
-                accumulate = 1;
-              }
-            }
-          }
-          umma_commit_2cta(&empty_bar[stage], 0x3);
-          BCOSK_TACC2(3);
-          if (++stage == num_stages) { stage = 0; phase ^= 1; }
-        }
-        umma_commit_2cta(tmem_full_bar, 0x3);
-      }
-    } else if (lane == 0) {
+    if (lane == 0) {
       const uint32_t idesc = umma_idesc_f16((uint32_t)p.dtype, BM, BN);
       const uint32_t row_bytes = p.kch * 2;
       const uint32_t a_chunk_bytes = BM * p.kch * 2;
@@ -704,35 +556,18 @@ bcosk_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
       uint32_t phase = 0;
       uint32_t accumulate = 0;
       for (int it = 0; it < num_iters; ++it) {
-        uint32_t tmem_d = tmem_base;
-        if (HP) {
-          // fresh accumulator per stage: the tensor core truncates when it aligns addends to a large running sum,
-          // so long dot products are summed in registers (round-to-nearest fp32) by the epilogue warps instead
-          // (BCOSK_HP_CHUNK consecutive stages may share one accumulator: experiment knob, 1 in the shipped library)
-          const int d = it / BCOSK_HP_CHUNK, buf = d & 1;
-          if (it % BCOSK_HP_CHUNK == 0) {
-            mbar_wait(&acc_empty_bar[buf], (((uint32_t)d >> 1) & 1u) ^ 1u);
-            accumulate = 0;
-          }
-          tmem_d = tmem_base + (uint32_t)(buf * BN);
-        }
         uint8_t* slot = smem + stage * Cfg::kSlotBytes;
-        {
-          BCOSK_TACC2_BEGIN();
-          mbar_wait(&full_bar[stage], phase);
-          BCOSK_TACC2(1);
-        }
+        mbar_wait(&full_bar[stage], phase);
         tc_fence_after();
-        BCOSK_TACC2_BEGIN();
         if (chunks_per_stage == 1) {
           // 64-channel chunks: four K steps per stage, descriptors differ by constants only (the issuing thread must
           // stay below the 64 cycles a 128 x 128 x 16 MMA takes; the generic loop below costs ~170 per MMA)
           const uint64_t da = da_stage0 + (uint64_t)stage * slot16;
           const uint64_t db = da + (A_STAGE_BYTES >> 4);
-          umma_f16(tmem_d, da, db, idesc, accumulate);
-          umma_f16(tmem_d, da + 2, db + 2, idesc, 1);
-          umma_f16(tmem_d, da + 4, db + 4, idesc, 1);
-          umma_f16(tmem_d, da + 6, db + 6, idesc, 1);
+          umma_f16(tmem_base, da, db, idesc, accumulate);
+          umma_f16(tmem_base, da + 2, db + 2, idesc, 1);
+          umma_f16(tmem_base, da + 4, db + 4, idesc, 1);
+          umma_f16(tmem_base, da + 6, db + 6, idesc, 1);
           accumulate = 1;
         } else {
           for (int j = 0; j < chunks_per_stage; ++j) {
@@ -740,20 +575,15 @@ bcosk_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
             const uint64_t db = umma_smem_desc_kmajor(smem_u32(slot + A_STAGE_BYTES + j * b_chunk_bytes), row_bytes);
             for (int k = 0; k < mma_per_chunk; ++k) {
               // advance 16 K-elements = 32 bytes inside the swizzle atom: +2 in the (addr >> 4) field
-              umma_f16(tmem_d, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), idesc, accumulate);
+              umma_f16(tmem_base, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), idesc, accumulate);
               accumulate = 1;
             }
           }
         }
-        // frees the smem slot once these MMAs have read it (in every CTA of the cluster: their multicasts land here too)
-        if (cl > 1) umma_commit_mc(&empty_bar[stage], cl_mask);
-        else umma_commit(&empty_bar[stage]);
-        BCOSK_TACC2(3);
-        if (HP && (it % BCOSK_HP_CHUNK == BCOSK_HP_CHUNK - 1 || it == num_iters - 1))
-          umma_commit(&acc_full_bar[(it / BCOSK_HP_CHUNK) & 1]);
+        umma_commit(&empty_bar[stage]);   // frees the smem slot once these MMAs have read it
         if (++stage == num_stages) { stage = 0; phase ^= 1; }
       }
-      if (!HP) umma_commit(tmem_full_bar);  // accumulator complete
+      umma_commit(tmem_full_bar);  // accumulator complete
     }
   } else {
     // ===================== epilogue (warps 2..5) =====================
@@ -815,7 +645,6 @@ bcosk_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
     }
     float sq_acc = 0.f;
     const uint32_t lane_base = (uint32_t)(quad * 32) << 16;
-    if (et == 0) BCOSK_STAMP(2);   // setup + patch norm done
     EpiTiles tl;
     tl.in = use_in_tile ? smem_u32(smem + (kSlots - 1) * Cfg::kSlotBytes) : 0u;
     tl.in2 = use_in2_tile ? smem_u32(smem + (kSlots - 2) * Cfg::kSlotBytes) : 0u;
@@ -826,111 +655,44 @@ bcosk_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
     tl.out1 = (Cfg::kTmaEpilogue && aux.tma_out1) ? smem_u32(smem + (kSwapOut ? Cfg::kSlotBytes : 0)) : 0u;
     tl.out2 = (Cfg::kTmaEpilogue && aux.tma_out2) ? smem_u32(smem + (kSwapOut ? 0 : Cfg::kSlotBytes)) : 0u;
 
-    if constexpr (HP) {
-      // The generic epilogue reads this row's side tensors (residual / extra gradient / gains) with plain loads after the
-      // last drain; with 12 warps per SM nothing hides their DRAM latency (ncu: long-scoreboard stalls).  Pull the lines
-      // into L2 now, while the K loop runs.
-      if (ri.valid) {
-        const int tile_cols = min(BN, p.n - n0);
-        auto prefetch_row = [&](const void* base, size_t elem_off, int elem_bytes) {
-          const char* b = reinterpret_cast<const char*>(base) + elem_off * (size_t)elem_bytes;
-          const char* e = b + (size_t)tile_cols * elem_bytes;
-          for (const char* q = reinterpret_cast<const char*>(reinterpret_cast<uintptr_t>(b) & ~(uintptr_t)127); q < e; q += 128)
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(q));
-        };
-        if (MODE == BCOSK_MODE_FWD) {
-          if (p.res != nullptr && tl.in == 0)
-            for (int pl = 0; pl < p.res_planes; ++pl)
-              prefetch_row(p.res, (size_t)ri.m * p.res_ld + n0 + (size_t)pl * p.res_plane_stride, 2);
-        } else {
-          if (add_row >= 0)
-            for (int pl = 0; pl < p.add_planes; ++pl)
-              prefetch_row(p.add, (size_t)add_row * p.add_ld + n0 + (size_t)pl * p.add_plane_stride, 2);
-          if (p.mul1 != nullptr && tl.in == 0) prefetch_row(p.mul1, (size_t)ri.m * p.mul1_ld + n0, p.mul1_f32 ? 4 : 2);
-          if (p.out2 != nullptr && p.mul2 != nullptr) prefetch_row(p.mul2, (size_t)ri.m * p.mul2_ld + n0, p.mul2_f32 ? 4 : 2);
-        }
-      }
-      float acc[BN];
+    const bool fast = epilogue_fast_ok<MODE>(p);
+    // explain: the previous block's ReLU mask words of this row (one per 32 columns), fetched before any waiting
+    uint32_t mb_pre[BN / 32];
 #pragma unroll
-      for (int i = 0; i < BN; ++i) acc[i] = 0.f;
-      const int num_drains = (num_iters + BCOSK_HP_CHUNK - 1) / BCOSK_HP_CHUNK;
-      for (int it = 0; it < num_drains; ++it) {
-        const int buf = it & 1;
-        mbar_wait(&acc_full_bar[buf], ((uint32_t)it >> 1) & 1u);
-        tc_fence_after();
-#pragma unroll
-        for (int j = 0; j < BN / 32; ++j) {
-          uint32_t raw[32];
-          tmem_ld_32x32(tmem_base + lane_base + (uint32_t)(buf * BN + j * 32), raw);
-          tmem_ld_wait();
-#pragma unroll
-          for (int i = 0; i < 32; ++i) acc[j * 32 + i] += __uint_as_float(raw[i]);
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&acc_empty_bar[buf]);
-      }
-#pragma unroll
-      for (int j = 0; j < BN / 32; ++j) {
-        const int c0 = n0 + j * 32;
-        if (c0 < p.n && ri.valid) {
-          float v[32];
-#pragma unroll
-          for (int i = 0; i < 32; ++i) v[i] = acc[j * 32 + i];
-          epilogue_chunk_generic_inl<MODE, T>(p, ri, yrow, inv_norm, add_row, s_alpha, s_beta, j, c0, min(32, p.n - c0), v,
-                                              sq_acc, tl, row);
-        }
-      }
-    } else {
-      const bool fast = epilogue_fast_ok<MODE>(p);
-      // explain: the previous block's ReLU mask words of this row (one per 32 columns), fetched before any waiting
-      uint32_t mb_pre[BN / 32];
-#pragma unroll
-      for (int j = 0; j < BN / 32; ++j) {
-        mb_pre[j] = 0xffffffffu;
-        if (MODE == BCOSK_MODE_EXPLAIN && p.mask2 != nullptr && ri.valid && n0 + j * 32 < p.n)
-          mb_pre[j] = __ldg(p.mask2 + (size_t)ri.m * p.mask2_ld + ((n0 + j * 32) >> 5));
-      }
-      if (use_in_tile) mbar_wait(in_bar, 0);
-      if (et == 0) BCOSK_STAMP(3);   // input tile landed
-      {
-        BCOSK_TACC2_BEGIN();
-        mbar_wait(tmem_full_bar, 0);  // all MMAs done: accumulator complete AND every pipeline slot is drained
-        if (et == 0) { BCOSK_TACC2(4); }
-      }
-      tc_fence_after();
-      BCOSK_TACC2_BEGIN();
-      if (et == 0) BCOSK_STAMP(4);   // accumulator ready
+    for (int j = 0; j < BN / 32; ++j) {
+      mb_pre[j] = 0xffffffffu;
+      if (MODE == BCOSK_MODE_EXPLAIN && p.mask2 != nullptr && ri.valid && n0 + j * 32 < p.n)
+        mb_pre[j] = __ldg(p.mask2 + (size_t)ri.m * p.mask2_ld + ((n0 + j * 32) >> 5));
+    }
+    if (use_in_tile) mbar_wait(in_bar, 0);
+    mbar_wait(tmem_full_bar, 0);  // all MMAs done: accumulator complete AND every pipeline slot is drained
+    tc_fence_after();
 #pragma unroll 1
-      for (int j = 0; j < BN / 32; ++j) {
-        const int c0 = n0 + j * 32;
-        if (c0 >= p.n) break;  // warp-uniform
-        uint32_t raw[32];
-        tmem_ld_32x32(tmem_base + lane_base + (uint32_t)(j * 32), raw);
-        tmem_ld_wait();
-        if (!ri.valid) continue;
-        float v[32];
+    for (int j = 0; j < BN / 32; ++j) {
+      const int c0 = n0 + j * 32;
+      if (c0 >= p.n) break;  // warp-uniform
+      uint32_t raw[32];
+      tmem_ld_32x32(tmem_base + lane_base + (uint32_t)(j * 32), raw);
+      tmem_ld_wait();
+      if (!ri.valid) continue;
+      float v[32];
 #pragma unroll
-        for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(raw[i]);
-        epilogue_chunk<MODE, T>(p, ri, yrow, inv_norm, add_row, s_alpha, s_beta, j, c0, min(32, p.n - c0), v, sq_acc, tl,
-                                row, fast, pick_word<BN / 32>(mb_pre, j));
-      }
-      if (et == 0) BCOSK_STAMP(5);   // epilogue math done
-      if (et == 0) { BCOSK_TACC2(5); }
-      if (tl.out1 != 0 || tl.out2 != 0) {
-        // generic-proxy smem writes -> visible to the async proxy, then one thread issues the bulk tensor stores
-        fence_proxy_async_smem();
-        asm volatile("bar.sync 1, 128;" ::: "memory");
-        if (et == 0) {
-          for (int b = 0; b < BN / 64; ++b) {
-            const int c = n0 + b * 64;
-            if (c >= p.n) break;
-            if (tl.out1 != 0) tma_store_2d_addr(&tmap_out1, tl.out1 + b * 16384, c, m0);
-            if (tl.out2 != 0) tma_store_2d_addr(&tmap_out2, tl.out2 + b * 16384, c, m0);
-          }
-          tma_store_commit_and_wait_read();
-          BCOSK_STAMP(6);   // TMA stores have read their shared-memory tiles
+      for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(raw[i]);
+      epilogue_chunk<MODE, T>(p, ri, yrow, inv_norm, add_row, s_alpha, s_beta, j, c0, min(32, p.n - c0), v, sq_acc, tl,
+                              row, fast, pick_word<BN / 32>(mb_pre, j));
+    }
+    if (tl.out1 != 0 || tl.out2 != 0) {
+      // generic-proxy smem writes -> visible to the async proxy, then one thread issues the bulk tensor stores
+      fence_proxy_async_smem();
+      asm volatile("bar.sync 1, 128;" ::: "memory");
+      if (et == 0) {
+        for (int b = 0; b < BN / 64; ++b) {
+          const int c = n0 + b * 64;
+          if (c >= p.n) break;
+          if (tl.out1 != 0) tma_store_2d_addr(&tmap_out1, tl.out1 + b * 16384, c, m0);
+          if (tl.out2 != 0) tma_store_2d_addr(&tmap_out2, tl.out2 + b * 16384, c, m0);
         }
+        tma_store_commit_and_wait_read();
       }
     }
     if (MODE == BCOSK_MODE_FWD) {
@@ -941,13 +703,10 @@ bcosk_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
   }
 
   __syncthreads();
-  if (cl > 1) cluster_sync_all();        // no CTA leaves while a peer's commit may still arrive on its barriers
   if (warp == 1) {
     tc_fence_after();
-    if constexpr (PAIR) tmem_dealloc_2cta(tmem_base, Cfg::kTmemCols);
-    else tmem_dealloc(tmem_base, Cfg::kTmemCols);
+    tmem_dealloc(tmem_base, Cfg::kTmemCols);
   }
-  if (threadIdx.x == 64) BCOSK_STAMP(7);
 }
 
 // =================================================================================================
@@ -1053,8 +812,6 @@ bcosk_igemm_persistent_kernel(const __grid_constant__ CUtensorMap tmap_a, const 
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
-  grid_launch_dependents();     // prologue done: it may overlap the previous launch's tail
-  grid_dependency_wait();       // from here on global memory written by the previous launch is read
 
   if (warp == 0) {
     // ===================== A/B producer =====================
@@ -1075,11 +832,7 @@ bcosk_igemm_persistent_kernel(const __grid_constant__ CUtensorMap tmap_a, const 
         int seg = 0, tap = 0, kc = 0;
         for (int it = 0; it < num_iters; ++it) {
           uint8_t* slot = smem + stage * Cfg::kSlotBytes;
-          {
-            BCOSK_TACC2_BEGIN();
-            mbar_wait(&empty_bar[stage], phase ^ 1);
-            BCOSK_TACC2(0);
-          }
+          mbar_wait(&empty_bar[stage], phase ^ 1);
           mbar_arrive_expect_tx(&full_bar[stage], Cfg::kSlotBytes);
           for (int j = 0; j < chunks_per_stage; ++j) {
             const int ci = it * chunks_per_stage + j;
@@ -1108,21 +861,13 @@ bcosk_igemm_persistent_kernel(const __grid_constant__ CUtensorMap tmap_a, const 
       uint32_t i = 0;
       for (int t; (t = persist_tile((int)i, n_tiles, m_tiles, aux.order)) >= 0; ++i) {
         const uint32_t buf = i & 1u;
-        {
-          BCOSK_TACC2_BEGIN();
-          mbar_wait(&acc_empty_bar[buf], ((i >> 1) & 1u) ^ 1u);   // epilogue has drained this accumulator
-          BCOSK_TACC2(2);
-        }
+        mbar_wait(&acc_empty_bar[buf], ((i >> 1) & 1u) ^ 1u);   // epilogue has drained this accumulator
         tc_fence_after();
         const uint32_t tmem_d = tmem_base + buf * BN;
         uint32_t accumulate = 0;
         for (int it = 0; it < num_iters; ++it) {
           uint8_t* slot = smem + stage * Cfg::kSlotBytes;
-          {
-            BCOSK_TACC2_BEGIN();
-            mbar_wait(&full_bar[stage], phase);
-            BCOSK_TACC2(1);
-          }
+          mbar_wait(&full_bar[stage], phase);
           tc_fence_after();
           for (int j = 0; j < chunks_per_stage; ++j) {
             const uint64_t da = umma_smem_desc_kmajor(smem_u32(slot + j * a_chunk_bytes), row_bytes);
@@ -1145,11 +890,7 @@ bcosk_igemm_persistent_kernel(const __grid_constant__ CUtensorMap tmap_a, const 
       for (int t; (t = persist_tile((int)i, n_tiles, m_tiles, aux.order)) >= 0; ++i) {
         const uint32_t buf = i & 1u;
         const int m0 = (t / n_tiles) * BM, n0 = (t % n_tiles) * BN;
-        {
-          BCOSK_TACC2_BEGIN();
-          mbar_wait(&in_empty_bar[buf], ((i >> 1) & 1u) ^ 1u);
-          BCOSK_TACC2(3);
-        }
+        mbar_wait(&in_empty_bar[buf], ((i >> 1) & 1u) ^ 1u);
         mbar_arrive_expect_tx(&in_full_bar[buf], Cfg::kTileBytes * (use_in2_tile ? 2 : 1));
         tma_load_2d(in_tile + buf * Cfg::kTileBytes, &tmap_in, &in_full_bar[buf], n0, m0);
         if (use_in2_tile) tma_load_2d(in2_tile + buf * Cfg::kTileBytes, &tmap_in2, &in_full_bar[buf], n0, m0);
@@ -1283,22 +1024,13 @@ bcosk_igemm_persistent_kernel(const __grid_constant__ CUtensorMap tmap_a, const 
       tl.out1 = aux.tma_out1 ? smem_u32(out1_tile + buf * Cfg::kTileBytes) : 0u;
       tl.out2 = aux.tma_out2 ? smem_u32(out2_tile + buf * Cfg::kTileBytes) : 0u;
 
-#ifdef BCOSK_TIMING2
-      const long long _t0 = clock64();
-#endif
       mbar_wait(&side_full_bar[buf], par);
       const uint32_t side0 = s_side[buf * (BM * 2) + row * 2];
       const uint32_t side1 = s_side[buf * (BM * 2) + row * 2 + 1];
       const float inv_norm = (MODE == BCOSK_MODE_FWD) ? __uint_as_float(side0) : 1.f;
       const uint32_t mb = (MODE == BCOSK_MODE_EXPLAIN) ? (half ? side1 : side0) : 0xffffffffu;
       if (use_in_tile) mbar_wait(&in_full_bar[buf], par);
-#ifdef BCOSK_TIMING2
-      const long long _t1 = clock64();
-#endif
       mbar_wait(&acc_full_bar[buf], par);
-#ifdef BCOSK_TIMING2
-      const long long _t2 = clock64();
-#endif
       tc_fence_after();
 
       float sq_acc = 0.f;
@@ -1340,15 +1072,6 @@ bcosk_igemm_persistent_kernel(const __grid_constant__ CUtensorMap tmap_a, const 
         p.sq_out[(size_t)tile_n * M + ri.m] = s_sq[(buf * 2) * BM + row] + s_sq[(buf * 2 + 1) * BM + row];
       if (MODE == BCOSK_MODE_FWD && p.inv_norm_out != nullptr && tile_n == 0 && half == 0 && ri.valid)
         p.inv_norm_out[ri.m] = inv_norm;
-#ifdef BCOSK_TIMING2
-      if (et == 0 && g_timing_buf != nullptr && (int)blockIdx.x < g_timing_cap) {
-        const long long _t3 = clock64();
-        g_timing_buf[blockIdx.x * 8 + 4] += _t1 - _t0;
-        g_timing_buf[blockIdx.x * 8 + 5] += _t2 - _t1;
-        g_timing_buf[blockIdx.x * 8 + 6] += _t3 - _t2;
-        g_timing_buf[blockIdx.x * 8 + 7] += 1;
-      }
-#endif
     }
     if (any_out_tile && et == 0) tma_store_wait_read();
     tc_fence_before();
@@ -1454,8 +1177,6 @@ bcosk_igemm_flat_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
-  grid_launch_dependents();     // prologue done: it may overlap the previous launch's tail
-  grid_dependency_wait();       // from here on global memory written by the previous launch is read
 
   if (warp == 0) {
     // ===================== producer =====================
@@ -1467,11 +1188,7 @@ bcosk_igemm_flat_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
         const uint32_t buf = i & 1u, par = (i >> 1) & 1u;
         const int img = t / geo.tiles_img;
         const int m0 = (t - img * geo.tiles_img) * BM;
-        {
-          BCOSK_TACC_BEGIN();
-          mbar_wait(&win_empty_bar[buf], par ^ 1u);
-          BCOSK_TACC(0);
-        }
+        mbar_wait(&win_empty_bar[buf], par ^ 1u);
         mbar_arrive_expect_tx(&win_full_bar[buf], win_bytes);
         if (geo.dense) {
           // input rows p0 + lo_h .. of this image, pixels lo_w .. lo_w + pitch - 1: borders arrive as zeros
@@ -1494,18 +1211,9 @@ bcosk_igemm_flat_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
       uint32_t i = 0;
       for (int t = blockIdx.x; t < total_tiles; t += gridDim.x, ++i) {
         const uint32_t buf = i & 1u, par = (i >> 1) & 1u;
-        {
-          BCOSK_TACC_BEGIN();
-          mbar_wait(&acc_empty_bar[buf], par ^ 1u);
-          BCOSK_TACC(2);
-        }
-        {
-          BCOSK_TACC_BEGIN();
-          mbar_wait(&win_full_bar[buf], par);
-          BCOSK_TACC(1);
-        }
+        mbar_wait(&acc_empty_bar[buf], par ^ 1u);
+        mbar_wait(&win_full_bar[buf], par);
         tc_fence_after();
-        BCOSK_TACC_BEGIN();
         // one LDS + two 64-bit adds per tap, then the K steps unrolled: the issuing thread must stay well under the
         // ~48 cycles a 128 x 64 x 16 MMA takes (measured: scripts/exp/mma_rate.cu), a naive loop costs ~240 per MMA
         uint64_t da0 = umma_smem_desc_kmajor(smem_u32(s_win + buf * win_stride), row_bytes);
@@ -1537,7 +1245,6 @@ bcosk_igemm_flat_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
         }
         umma_commit(&win_empty_bar[buf]);
         umma_commit(&acc_full_bar[buf]);
-        BCOSK_TACC(3);
       }
     }
   } else {
@@ -1584,13 +1291,7 @@ bcosk_igemm_flat_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
       tl.out1 = aux.tma_out1 ? smem_u32(s_out + (buf * 2) * Cfg::kTileBytes) : 0u;
       tl.out2 = aux.tma_out2 ? smem_u32(s_out + (buf * 2 + 1) * Cfg::kTileBytes) : 0u;
 
-#ifdef BCOSK_TIMING
-      const long long _t_a = clock64();
-#endif
       mbar_wait(&acc_full_bar[buf], par);
-#ifdef BCOSK_TIMING
-      const long long _t_b = clock64();
-#endif
       tc_fence_after();
       float sq_acc = 0.f;
       if (c0 < p.n) {
@@ -1610,9 +1311,6 @@ bcosk_igemm_flat_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
       if (lane == 0) mbar_arrive(&acc_empty_bar[buf]);
       float* sq_buf = s_sq + buf * (BN / 32) * BM;
       if (want_sq) sq_buf[j * BM + row] = sq_acc;
-#ifdef BCOSK_TIMING
-      const long long _t_c = clock64();
-#endif
       if (any_out_tile && geo.tma_store) {
         fence_proxy_async_smem();
         if (et == 0) tma_store_wait_read();           // tile i-1's stores have read the other staging buffer
@@ -1655,15 +1353,6 @@ bcosk_igemm_flat_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
         p.sq_out[ri.m] = s;
       }
       if (MODE == BCOSK_MODE_FWD && p.inv_norm_out != nullptr && j == 0 && ri.valid) p.inv_norm_out[ri.m] = inv_norm;
-#ifdef BCOSK_TIMING
-      if (et == 0 && g_timing_buf != nullptr && (int)blockIdx.x < g_timing_cap) {
-        const long long _t_d = clock64();
-        g_timing_buf[blockIdx.x * 8 + 4] += _t_b - _t_a;   // waiting for the accumulator
-        g_timing_buf[blockIdx.x * 8 + 5] += _t_c - _t_b;   // TMEM load + epilogue math + staging
-        g_timing_buf[blockIdx.x * 8 + 6] += _t_d - _t_c;   // barrier + copy-out
-        g_timing_buf[blockIdx.x * 8 + 7] += 1;             // tiles
-      }
-#endif
     }
     if (any_out_tile && geo.tma_store && et == 0) tma_store_wait_read();
     tc_fence_before();
@@ -1721,30 +1410,11 @@ struct LaunchMaps {
   CUtensorMap a, b, in, in2, out1, out2;
 };
 
-static int g_pdl_enabled = 0;          // programmatic dependent launch of the tensor-core kernels (prologue overlaps the previous
-                                       // tail): measured 13.77 -> 13.73 ms / step, not worth a default
-
-// kernel<<<grid, block, smem, stream>>>(args...) with the programmatic-serialization attribute when enabled
-template <typename Kern, typename... Args>
-static cudaError_t launch_pdl(Kern kern, dim3 grid, int threads, size_t smem, cudaStream_t st, Args... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = dim3(threads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = g_pdl_enabled ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kern, args...);
-}
-
-template <int BN, int MODE, bool HP, int LIGHT = 0, bool PAIR = false>
+template <int BN, int MODE, int LIGHT = 0>
 static int launch_igemm(const LaunchMaps& mp, const bcosk_igemm_params& p, const IgemmAux& aux, cudaStream_t st) {
-  using Cfg = TileCfg<BN, HP, LIGHT>;
-  auto kern = bcosk_igemm_kernel<BN, MODE, __nv_bfloat16, HP, LIGHT, PAIR>;
-  auto kern_h = bcosk_igemm_kernel<BN, MODE, __half, HP, LIGHT, PAIR>;
+  using Cfg = TileCfg<BN, LIGHT>;
+  auto kern = bcosk_igemm_kernel<BN, MODE, __nv_bfloat16, LIGHT>;
+  auto kern_h = bcosk_igemm_kernel<BN, MODE, __half, LIGHT>;
   const void* fn = (p.dtype == BCOSK_DTYPE_BF16) ? (const void*)kern : (const void*)kern_h;
   // per launch: the attribute belongs to (function, device); a process may drive several GPUs and threads
   BCOSK_CUDA_CHECK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
@@ -1753,39 +1423,16 @@ static int launch_igemm(const LaunchMaps& mp, const bcosk_igemm_params& p, const
   const long long n_tiles = (p.n + BN - 1) / BN;
   if (m_tiles * n_tiles > 0x7fffffffLL) return set_error(BCOSK_EUNSUPPORTED, "igemm: grid too large");
   dim3 grid((unsigned)(m_tiles * n_tiles));
-  if (aux.cluster > 1) {
-    if (m_tiles % aux.cluster != 0) return set_error(BCOSK_EINVAL, "igemm: cluster size must divide the row blocks");
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = dim3(NUM_THREADS);
-    cfg.dynamicSmemBytes = Cfg::kSmemBytes;
-    cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = (unsigned)aux.cluster;
-    at[0].val.clusterDim.y = 1;
-    at[0].val.clusterDim.z = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
-    if (p.dtype == BCOSK_DTYPE_BF16)
-      BCOSK_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kern, mp.a, mp.b, mp.in, mp.in2, mp.out1, mp.out2, p, aux));
-    else
-      BCOSK_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kern_h, mp.a, mp.b, mp.in, mp.in2, mp.out1, mp.out2, p, aux));
-    return BCOSK_OK;
-  }
   if (p.dtype == BCOSK_DTYPE_BF16)
-    BCOSK_CUDA_CHECK(launch_pdl(kern, grid, NUM_THREADS, Cfg::kSmemBytes, st, mp.a, mp.b, mp.in, mp.in2, mp.out1, mp.out2, p, aux));
+    kern<<<grid, NUM_THREADS, Cfg::kSmemBytes, st>>>(mp.a, mp.b, mp.in, mp.in2, mp.out1, mp.out2, p, aux);
   else
-    BCOSK_CUDA_CHECK(launch_pdl(kern_h, grid, NUM_THREADS, Cfg::kSmemBytes, st, mp.a, mp.b, mp.in, mp.in2, mp.out1, mp.out2, p, aux));
+    kern_h<<<grid, NUM_THREADS, Cfg::kSmemBytes, st>>>(mp.a, mp.b, mp.in, mp.in2, mp.out1, mp.out2, p, aux);
+  BCOSK_CUDA_CHECK(cudaGetLastError());
   return BCOSK_OK;
 }
 
 static int g_num_sms = 0;             // refreshed per launch from the current device (a process may drive several GPUs)
 static int g_late_in_iters = 2;        // K stages from which the epilogue input tile is fetched after the main loop (0 = never)
-static int g_cluster = 1;              // 1 none; 2/4 weight-tile multicast across row blocks; 3 = CTA pairs (cta_group::2)
-// Measured on B200 (profiles/r01_schedule_ab.md): per-tile + 3 CTAs/SM and the persistent kernel reach the same
-// ~4 TB/s on the bandwidth-bound launches; the per-tile schedule is the default.
-static int g_persistent_enabled = 0;   // 0 off, 1 tiles strided over the grid, 2 row-block order
 static bool g_light_enabled = true;
 static bool g_light4_enabled = true;
 static int g_light4_max_iters = 4;
@@ -1808,9 +1455,10 @@ static int launch_persistent(const LaunchMaps& mp, const bcosk_igemm_params& p, 
   if (tiles > 0x7fffffffLL) return set_error(BCOSK_EUNSUPPORTED, "igemm: too many tiles");
   dim3 grid((unsigned)(tiles < g_num_sms ? tiles : g_num_sms));
   if (p.dtype == BCOSK_DTYPE_BF16)
-    BCOSK_CUDA_CHECK(launch_pdl(kern, grid, P_THREADS, Cfg::kSmemBytes, st, mp.a, mp.b, mp.in, mp.in2, mp.out1, mp.out2, p, aux));
+    kern<<<grid, P_THREADS, Cfg::kSmemBytes, st>>>(mp.a, mp.b, mp.in, mp.in2, mp.out1, mp.out2, p, aux);
   else
-    BCOSK_CUDA_CHECK(launch_pdl(kern_h, grid, P_THREADS, Cfg::kSmemBytes, st, mp.a, mp.b, mp.in, mp.in2, mp.out1, mp.out2, p, aux));
+    kern_h<<<grid, P_THREADS, Cfg::kSmemBytes, st>>>(mp.a, mp.b, mp.in, mp.in2, mp.out1, mp.out2, p, aux);
+  BCOSK_CUDA_CHECK(cudaGetLastError());
   return BCOSK_OK;
 }
 
@@ -1904,9 +1552,10 @@ static int launch_flat_bn(const bcosk_igemm_params& p, cudaStream_t st) {
   if (tiles > 0x7fffffffLL || (long long)p.a_nb * hp * wp > 0x7fffffffLL) return set_error(BCOSK_EUNSUPPORTED, "igemm(flat): too large");
   dim3 grid((unsigned)(tiles < g_num_sms ? tiles : g_num_sms));
   if (p.dtype == BCOSK_DTYPE_BF16)
-    BCOSK_CUDA_CHECK(launch_pdl(kern, grid, Cfg::kThreads, (size_t)smem, st, mp.a, mp.b, mp.out1, mp.out2, p, aux, geo));
+    kern<<<grid, Cfg::kThreads, (size_t)smem, st>>>(mp.a, mp.b, mp.out1, mp.out2, p, aux, geo);
   else
-    BCOSK_CUDA_CHECK(launch_pdl(kern_h, grid, Cfg::kThreads, (size_t)smem, st, mp.a, mp.b, mp.out1, mp.out2, p, aux, geo));
+    kern_h<<<grid, Cfg::kThreads, (size_t)smem, st>>>(mp.a, mp.b, mp.out1, mp.out2, p, aux, geo);
+  BCOSK_CUDA_CHECK(cudaGetLastError());
   return BCOSK_OK;
 }
 
@@ -1969,18 +1618,18 @@ static int validate(const bcosk_igemm_params& p) {
   return BCOSK_OK;
 }
 
-static int make_maps(const bcosk_igemm_params& p, int bn, int cluster, LaunchMaps* mp, IgemmAux* aux) {
+static int make_maps(const bcosk_igemm_params& p, int bn, LaunchMaps* mp, IgemmAux* aux) {
   memset(mp, 0, sizeof(*mp));
   memset(aux, 0, sizeof(*aux));
   int rc = make_im2col_map_nhwc(&mp->a, p.a, p.a_nb, p.a_h, p.a_w, p.a_c, p.lo_w, p.lo_h, p.up_w, p.up_h, p.stride_w,
                                 p.stride_h, p.kch, BM, p.kch == 64 ? 128 : 64);
   if (rc) return rc;
   const long long ktot = (long long)p.num_segs * p.num_taps * p.chunks_per_tap * p.kch;
-  rc = make_tiled_map_2d(&mp->b, p.b, ktot, p.n, p.kch, bn / cluster, p.kch == 64 ? 128 : 64);   // each CTA fetches its share
+  rc = make_tiled_map_2d(&mp->b, p.b, ktot, p.n, p.kch, bn, p.kch == 64 ? 128 : 64);
   if (rc) return rc;
   // ---- TMA epilogue (throughput mode): 16-bit single-plane tensors addressed densely by output row
   const long long M = (long long)p.a_nb * p.op * p.oq;
-  const bool tile_ok = !p.hp_accum && (bn == 64 || bn == 128) && p.max_out <= 1;   // MaxOut rows leave with per-row stores
+  const bool tile_ok = (bn == 64 || bn == 128) && p.max_out <= 1;   // MaxOut rows leave with per-row stores
   const bool dense_out = p.os_0 == 0 && p.os_q == 1 && p.os_p == p.oq && p.os_n == (long long)p.op * p.oq;
   auto map16 = [&](CUtensorMap* m, const void* base, int ld) -> bool {
     if ((reinterpret_cast<uintptr_t>(base) & 15) != 0 || ld % 8 != 0) return false;
@@ -2014,43 +1663,27 @@ extern "C" int bcosk_igemm(const bcosk_igemm_params* pp, void* stream) {
   if (rc) return rc;
   int bn = p.block_n;
   if (bn == 0) bn = p.n <= 32 ? 32 : ((p.n <= 64 || p.hp_accum) ? 64 : 128);
-  if (bn != 32 && bn != 64 && bn != 128 && bn != 256) return set_error(BCOSK_EINVAL, "igemm: block_n");
-  if (p.hp_accum && bn > 128) return set_error(BCOSK_EINVAL, "igemm: hp_accum needs block_n <= 128");
+  if (bn != 32 && bn != 64 && bn != 128) return set_error(BCOSK_EINVAL, "igemm: block_n");
   p.block_n = bn;
   if (p.max_out > 1) p.sched = 1;        // MaxOut: the per-tile kernel (generic epilogue, per-row stores)
   if (p.a_flat) return launch_flat(p, reinterpret_cast<cudaStream_t>(stream));
   if (p.hp_accum) return launch_hp(p, reinterpret_cast<cudaStream_t>(stream));   // parity mode: bcosk_igemm_hp.cu
-  // weight-tile multicast: 128-wide tiles with a long K loop are bound by L2 -> shared-memory traffic (A and B stages
-  // of every tile come from L2: ~13 TB/s at 800 TFLOP/s, the L2 limit); CTAs of neighbouring row blocks share B
-  int cluster = 1;
-  {
-    const long long m_tiles = ((long long)p.a_nb * p.op * p.oq + BM - 1) / BM;
-    const int iters = p.num_segs * p.num_taps * p.chunks_per_tap / (STAGE_K / p.kch);
-    const int persistent_req = p.sched == 0 ? g_persistent_enabled : p.sched - 1;
-    const int want = g_cluster == 3 ? 2 : g_cluster;
-    if (want > 1 && !p.hp_accum && bn == 128 && p.n % bn == 0 && iters >= 8 && m_tiles % want == 0 &&
-        !(persistent_req && bn == 64))
-      cluster = want;
-  }
   LaunchMaps mp;
   IgemmAux aux{};
-  rc = make_maps(p, bn, cluster, &mp, &aux);
+  rc = make_maps(p, bn, &mp, &aux);
   if (rc) return rc;
-  aux.cluster = cluster;
   {
     const int iters = p.num_segs * p.num_taps * p.chunks_per_tap / (STAGE_K / p.kch);
     aux.late_in = (g_late_in_iters > 0 && bn == 128 && iters >= g_late_in_iters) ? 1 : 0;
   }
-  aux.pair = (cluster == 2 && g_cluster == 3) ? 1 : 0;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
 #define BCOSK_DISPATCH(BN_)                                                                         \
   case BN_:                                                                                         \
-    return p.mode == BCOSK_MODE_FWD ? launch_igemm<BN_, BCOSK_MODE_FWD, false>(mp, p, aux, st)      \
-                                    : launch_igemm<BN_, BCOSK_MODE_EXPLAIN, false>(mp, p, aux, st);
+    return p.mode == BCOSK_MODE_FWD ? launch_igemm<BN_, BCOSK_MODE_FWD>(mp, p, aux, st)             \
+                                    : launch_igemm<BN_, BCOSK_MODE_EXPLAIN>(mp, p, aux, st);
   if (p.sched < 0 || p.sched > 3) return set_error(BCOSK_EINVAL, "igemm: sched must be 0..3");
-  const int persistent = p.sched == 0 ? g_persistent_enabled : p.sched - 1;   // 0 per tile, 1 strided, 2 row blocks
-  if (!p.hp_accum && persistent && bn == 64) {
-    aux.order = persistent == 2 ? 1 : 0;
+  if (p.sched >= 2 && bn == 64) {   // 0 / 1 one CTA per tile, 2 persistent strided, 3 persistent in row-block order
+    aux.order = p.sched == 3 ? 1 : 0;
     return p.mode == BCOSK_MODE_FWD ? launch_persistent<BCOSK_MODE_FWD>(mp, p, aux, st)
                                     : launch_persistent<BCOSK_MODE_EXPLAIN>(mp, p, aux, st);
   }
@@ -2061,7 +1694,7 @@ extern "C" int bcosk_igemm(const bcosk_igemm_params* pp, void* stream) {
     const int iters = p.num_segs * p.num_taps * p.chunks_per_tap / (STAGE_K / p.kch);
     if (bn == 64 && g_light_enabled && aux.tma_in2 && iters == 1 && p.mode == BCOSK_MODE_EXPLAIN && aux.tma_in &&
         aux.tma_out1 && (aux.tma_out2 || !p.out2) && !p.y_f32 && p.y_planes == 1 && !p.mul2_f32)
-      return launch_igemm<64, BCOSK_MODE_EXPLAIN, false, 1>(mp, p, aux, st);
+      return launch_igemm<64, BCOSK_MODE_EXPLAIN, 1>(mp, p, aux, st);
   }
   if (bn == 64 && g_light_enabled && !aux.tma_in2) {
     // short K loop (<= 4 stages): the 3-CTA/SM variant
@@ -2071,56 +1704,25 @@ extern "C" int bcosk_igemm(const bcosk_igemm_params* pp, void* stream) {
     const bool out_tiles = aux.tma_out1 && (aux.tma_out2 || !(p.mode == BCOSK_MODE_FWD ? p.gain : p.out2));
     if (iters <= g_light4_max_iters && g_light4_enabled && out_tiles) {
       aux.late_in = (aux.tma_in && iters >= 2) ? 1 : 0;
-      return p.mode == BCOSK_MODE_FWD ? launch_igemm<64, BCOSK_MODE_FWD, false, 2>(mp, p, aux, st)
-                                      : launch_igemm<64, BCOSK_MODE_EXPLAIN, false, 2>(mp, p, aux, st);
+      return p.mode == BCOSK_MODE_FWD ? launch_igemm<64, BCOSK_MODE_FWD, 2>(mp, p, aux, st)
+                                      : launch_igemm<64, BCOSK_MODE_EXPLAIN, 2>(mp, p, aux, st);
     }
     if (iters <= 4)
-      return p.mode == BCOSK_MODE_FWD ? launch_igemm<64, BCOSK_MODE_FWD, false, 1>(mp, p, aux, st)
-                                      : launch_igemm<64, BCOSK_MODE_EXPLAIN, false, 1>(mp, p, aux, st);
+      return p.mode == BCOSK_MODE_FWD ? launch_igemm<64, BCOSK_MODE_FWD, 1>(mp, p, aux, st)
+                                      : launch_igemm<64, BCOSK_MODE_EXPLAIN, 1>(mp, p, aux, st);
   }
-  if (aux.pair && bn == 128)
-    return p.mode == BCOSK_MODE_FWD ? launch_igemm<128, BCOSK_MODE_FWD, false, false, true>(mp, p, aux, st)
-                                    : launch_igemm<128, BCOSK_MODE_EXPLAIN, false, false, true>(mp, p, aux, st);
   switch (bn) {
     BCOSK_DISPATCH(32)
     BCOSK_DISPATCH(64)
     BCOSK_DISPATCH(128)
-    BCOSK_DISPATCH(256)
   }
 #undef BCOSK_DISPATCH
   return set_error(BCOSK_EINVAL, "igemm: unreachable");
 }
 
-extern "C" int bcosk_set_persistent(int32_t enabled) {
-  const int prev = g_persistent_enabled;
-  g_persistent_enabled = enabled;
-  return prev;
-}
-
-#ifdef BCOSK_TIMING
-extern "C" int bcosk_debug_set_timing(void* buf, int32_t capacity_ctas) {
-  unsigned long long* b = reinterpret_cast<unsigned long long*>(buf);
-  BCOSK_CUDA_CHECK(cudaMemcpyToSymbol(g_timing_buf, &b, sizeof(b)));
-  BCOSK_CUDA_CHECK(cudaMemcpyToSymbol(g_timing_cap, &capacity_ctas, sizeof(int)));
-  return BCOSK_OK;
-}
-#endif
-
-extern "C" int bcosk_set_pdl(int32_t enabled) {
-  const int prev = g_pdl_enabled;
-  g_pdl_enabled = enabled != 0;
-  return prev;
-}
-
 extern "C" int bcosk_set_late_input(int32_t min_k_stages) {
   const int prev = g_late_in_iters;
   g_late_in_iters = min_k_stages;
-  return prev;
-}
-
-extern "C" int bcosk_set_cluster(int32_t size) {
-  const int prev = g_cluster;
-  if (size >= 1 && size <= 4) g_cluster = size;
   return prev;
 }
 

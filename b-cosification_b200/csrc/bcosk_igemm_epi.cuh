@@ -145,12 +145,8 @@ struct IgemmAux {
   int tma_out1;  // primary output y staged in slot 0 and written with TMA
   int tma_out2;  // forward: gain, explain: out2 - staged in slot 1 and written with TMA
   int order;     // persistent kernel: 0 = tiles strided over the grid, 1 = a CTA walks all n tiles of one row block
-  int cluster;   // per-tile kernel: CTAs of `cluster` consecutive row blocks (same n tile) form a thread-block cluster;
-                 // each fetches 1/cluster of the weight tile and multicasts it to the others (0/1 = no cluster)
   int late_in;   // long K loops: fetch the epilogue input tile AFTER the main loop (into the last slot, once its final
                  // stage is consumed) so that the ring keeps all its stages while the MMAs run
-  int pair;      // cluster == 2 run as a CTA pair: one cta_group::2 MMA over both row blocks, each CTA keeps only its half
-                 // of the weight tile (no multicast: the tensor core reads the other half from the peer's shared memory)
 };
 
 // Shared-memory tiles of the TMA epilogue: [BN/64 boxes][128 rows][128 bytes], 16-byte units XOR-swizzled by row

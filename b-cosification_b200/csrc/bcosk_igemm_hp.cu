@@ -323,8 +323,6 @@ bcosk_igemm_hp_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_c
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
-  grid_launch_dependents();
-  grid_dependency_wait();
 
   if (warp == 0) {
     // ===================== TMA producer =====================

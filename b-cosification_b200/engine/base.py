@@ -132,7 +132,6 @@ class PlanBase:
     # launches whose K loop has at most this many 64-deep stages are bandwidth bound: they use 64-wide tiles, which
     # the library runs with 3 CTAs per SM (more bytes in flight); 0 disables
     light_k_iters = 3
-    wide_k_iters = 0
     parity_dgrad = True              # strided k x k data gradients as stride^2 parity-class launches (no zero insertion)
     # do not store gains that are sqrt(y / ||patch||) of a stored ReLU output.  Measured: the forward launches save 0.20 ms
     # of gain writes per step and the consumers pay 0.21 ms for the square roots (MUFU, 16 per cycle per SM): off.
@@ -151,8 +150,6 @@ class PlanBase:
             return 32
         if n <= 64 or hp or k_iters <= self.light_k_iters:
             return 64
-        if self.wide_k_iters and n >= 256 and k_iters >= self.wide_k_iters:
-            return 256                    # experiment: 256-wide tiles for long K loops (off: wide_k_iters = 0)
         return 128
 
     @staticmethod

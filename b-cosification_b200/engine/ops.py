@@ -71,7 +71,7 @@ class IgemmOp:
     a_dense_frac: float = 1.0
     hp_accum: bool = False           # per-stage TMEM accumulators summed in registers (parity mode)
     hp_chunk: int = 0                # include/bcosk.h `hp_chunk`: K stages per TMEM accumulation of the leading segment (0 = default)
-    sched: int = 0                   # include/bcosk.h `sched`: 0 default, 1 per tile, 2 persistent, 3 persistent row blocks
+    sched: int = 0                   # include/bcosk.h `sched`: 0 / 1 per tile, 2 persistent, 3 persistent row blocks
                                      # (hp_accum forward launches: 3 / 4 = three / four CTAs per SM, else two)
     flat: bool = False               # include/bcosk.h `a_flat`: `a` is the interior view of a zero-bordered buffer
     side_mapped: bool = False        # include/bcosk.h `side_mapped`: mul1 / out2 / ... follow the mapped output row

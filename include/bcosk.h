@@ -80,7 +80,7 @@ typedef struct bcosk_igemm_params {
   const void* b;
   int32_t n;
   int32_t dtype;   /* BCOSK_DTYPE_* of a, b, and all 16-bit epilogue tensors */
-  int32_t block_n; /* CTA tile N: 32, 64, 128, 256; 0 = choose */
+  int32_t block_n; /* CTA tile N: 32, 64, 128; 0 = choose */
   int32_t mode;    /* BCOSK_MODE_* */
   /* ---- forward epilogue */
   int32_t scale_mode; /* BCOSK_SCALE_* */
@@ -120,7 +120,8 @@ typedef struct bcosk_igemm_params {
   const uint32_t* mask2;
   int32_t mask2_ld;
   /* ---- accumulation: 0 = one fp32 TMEM accumulator over all of K (throughput mode); 1 = a fresh TMEM accumulator
-   *      per 64-deep K stage, summed in registers with round-to-nearest fp32 adds (parity mode; block_n <= 64).
+   *      per 64-deep K stage, summed in registers with round-to-nearest fp32 adds (parity mode: 64-wide tiles, or 128-wide
+   *      for forward launches with block_n = 128).
    *      The tensor core truncates when aligning addends to a large running sum (measured: relative error ~K*2^-26,
    *      biased), which random-init deep B-cos nets amplify 10^2-10^3 x. */
   int32_t hp_accum;
@@ -130,9 +131,9 @@ typedef struct bcosk_igemm_params {
    *      to back in ONE further accumulation; with bf16 planes they are chunked like the leading segment. */
   int32_t hp_chunk;
   /* ---- schedule of a block_n == 64 launch (ignored otherwise; results do not depend on it):
-   *      0 = library default (see bcosk_set_persistent / bcosk_set_light), 1 = one CTA per tile,
-   *      2 = persistent CTAs, tiles strided over the grid, 3 = persistent CTAs, each walks all n tiles of one
-   *      128-row block back to back (the segments of an output row reach L2 together).  The host plan measures the
+   *      0 and 1 = one CTA per tile (the variant follows bcosk_set_light), 2 = persistent CTAs, tiles strided over the
+   *      grid, 3 = persistent CTAs, each walks all n tiles of one 128-row block back to back (the segments of an output
+   *      row reach L2 together).  The host plan measures the
    *      three per launch once (engine/base.py PlanBase.autotune) - which wins depends on N/K and the epilogue streams.
    *      With hp_accum (forward launches only): 3 = three CTAs per SM (6 warps, 128 TMEM columns: one partial accumulator
    *      of the leading segment, drained before the next chunk starts; one paired stage as the ring) where the packed
@@ -211,25 +212,10 @@ int bcosk_set_hp_boxes(int32_t enabled);
  * 2, 3 or 4), info[4] = registers per thread, info[5] = local memory bytes per thread (spills).  Needs a current device. */
 int bcosk_igemm_hp_config(const bcosk_igemm_params* p, int32_t* info);
 
-/* Scheduling switch for A/B measurements: 1 = launches with block_n 64 (the bandwidth-bound ones) run on the persistent
- * one-CTA-per-SM kernel, 0 (default) = one CTA per tile everywhere.  Returns the previous setting.  Results are identical. */
-int bcosk_set_persistent(int32_t enabled);
-/* 1 = the tensor-core kernels are launched with programmatic stream serialization (default 0: measured gain 0.3 %): their prologue (barrier
- * init, TMEM allocation, descriptor prefetch) overlaps the previous launch's tail and `griddepcontrol.wait` orders every
- * global-memory access after the previous launch's completion.  Returns the previous setting.  Results are identical. */
-int bcosk_set_pdl(int32_t enabled);
-
 /* 128-wide launches whose K loop has at least `min_k_stages` 64-deep stages fetch their epilogue input tile (residual /
  * producer gain) after the main loop instead of parking it in a ring slot, so the MMAs run on 3 stages instead of 2
  * (0 = never).  Returns the previous setting.  Results are identical. */
 int bcosk_set_late_input(int32_t min_k_stages);
-
-/* Cluster mode of the 128-wide launches with >= 8 K stages.  1 = none.  2 / 4 = the CTAs of that many neighbouring
- * 128-row blocks each fetch a share of the weight tile and multicast it (TMA .multicast::cluster).  3 = CTA pairs:
- * two row blocks run ONE tcgen05.mma.cta_group::2 (256 x 128) issued by the leader CTA, each CTA keeps only its half of
- * the weight tile in shared memory (25 % fewer bytes into each SM per FLOP).  Returns the previous setting.  Results are
- * identical in every mode (tests/test_kernels_gpu.py). */
-int bcosk_set_cluster(int32_t size);
 
 /* Bit 0: launches with block_n 64 and a K loop of <= 4 stages use the 3-CTA-per-SM variant.  Bit 1: forward launches with
  * a single K stage use the 4-CTA-per-SM variant (the gain tile is staged over the consumed residual tile).  Default 3.

@@ -18,13 +18,8 @@ ap.add_argument("--only", default="")
 ap.add_argument("--mode", default=None, help="engine/resnet.py PRECISION_MODES name (default: parity); overrides --planes / --dtype")
 ap.add_argument("--planes", type=int, default=None)
 ap.add_argument("--dtype", default=None, choices=["bf16", "fp16"])
-ap.add_argument("--persistent", type=int, default=0)
-ap.add_argument("--cluster", type=int, default=1)
 ap.add_argument("--autotune", type=int, default=0, help="pick per-launch schedules first (as capture() does); use with ncu --profile-from-start off")
 a = ap.parse_args()
-from bcos_b200 import _lib
-_lib.load().bcosk_set_persistent(a.persistent)
-_lib.load().bcosk_set_cluster(a.cluster)
 if a.planes is None and a.dtype is None:
     plan = synthetic_resnet_plan(a.arch, a.batch, mode=a.mode or "parity", device="cuda", input_u8=True)
 else:

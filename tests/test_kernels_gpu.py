@@ -446,29 +446,28 @@ def test_a_tile_im2col(bcosk_lib):
                 assert torch.equal(out.float().cpu(), exp), (h, cin, k, stride, kch, tile_m, chunk)
 
 
-def test_persistent_and_per_tile_schedules_agree(bcosk_lib):
-    """same launches through the persistent (TMEM double-buffered) and the one-CTA-per-tile kernels"""
-    g = torch.Generator().manual_seed(21)
+def test_persistent_sched_matches_per_tile(bcosk_lib):
+    """same launch through the persistent (TMEM double-buffered) and the one-CTA-per-tile kernels"""
     nb, h, cin, cout = 4, 28, 128, 256
     outs = []
-    for persistent in (2, 1, 0):    # 2 = row-block tile order, 1 = tiles strided over the grid, 0 = one CTA per tile
-        prev = bcosk_lib.bcosk_set_persistent(persistent)
-        try:
-            gg = torch.Generator().manual_seed(21)
-            plan = _mini_plan(nb, 1)
-            x = _rand_act(gg, nb, h, h, cin, 1)
-            w = torch.randn(cout, cin, 3, 3, generator=gg) / math.sqrt(cin * 9)
-            plan.sd = {"bn.running_var": torch.rand(cout, generator=gg) + 0.5, "bn.weight": torch.rand(cout, generator=gg) + 0.5}
-            res = _rand_act(gg, nb, h, h, cout, 1)
-            y, rec = plan._conv_fwd("p", x, w, 1, 1, 1, bn="bn", relu=True, res=res, want_mask=True)
-            memo = {}
-            dops = [U.to_device(o, "cuda", memo) for o in plan.fwd_ops]
-            for o in dops:
-                o.run()
-            torch.cuda.synchronize()
-            outs.append([t.cpu() for t in (dops[-1].y, dops[-1].gain, dops[-1].maskbits, dops[-1].sq_out)])
-        finally:
-            bcosk_lib.bcosk_set_persistent(prev)
+    for sched in (3, 2, 1):         # persistent in row-block order, persistent with tiles strided over the grid, one CTA per tile
+        gg = torch.Generator().manual_seed(21)
+        plan = _mini_plan(nb, 1)
+        plan.light_k_iters = 18     # 18 K stages: 64-wide tiles (four column tiles), the only width with a persistent kernel
+        x = _rand_act(gg, nb, h, h, cin, 1)
+        w = torch.randn(cout, cin, 3, 3, generator=gg) / math.sqrt(cin * 9)
+        plan.sd = {"bn.running_var": torch.rand(cout, generator=gg) + 0.5, "bn.weight": torch.rand(cout, generator=gg) + 0.5}
+        res = _rand_act(gg, nb, h, h, cout, 1)
+        y, rec = plan._conv_fwd("p", x, w, 1, 1, 1, bn="bn", relu=True, res=res, want_mask=True)
+        op = plan.fwd_ops[-1]
+        assert op.resolved_block_n() == 64
+        op.sched = sched
+        memo = {}
+        dops = [U.to_device(o, "cuda", memo) for o in plan.fwd_ops]
+        for o in dops:
+            o.run()
+        torch.cuda.synchronize()
+        outs.append([t.cpu() for t in (dops[-1].y, dops[-1].gain, dops[-1].maskbits, dops[-1].sq_out)])
     for other in outs[:-1]:
         for k, (a, b) in enumerate(zip(other, outs[-1])):
             if k == 3:      # sums of squares: the persistent kernel adds two half-row partials (different rounding order)
@@ -477,49 +476,9 @@ def test_persistent_and_per_tile_schedules_agree(bcosk_lib):
                 assert torch.equal(a, b)
 
 
-def test_cluster_multicast_matches_single_cta(bcosk_lib):
-    """128-wide, K-heavy launches with the weight tile multicast across a cluster of 2 / 4 row blocks == no cluster"""
-    outs = {}
-    for cl in (1, 2, 4, 3):                         # 3 = CTA pairs (cta_group::2)
-        prev = bcosk_lib.bcosk_set_cluster(cl)
-        try:
-            g = torch.Generator().manual_seed(33)
-            nb, h, cin, cout = 4, 16, 64, 256          # M = 1024 -> 8 row blocks, K = 576 -> 9 stages, two n tiles
-            plan = _mini_plan(nb, 1)
-            x = _rand_act(g, nb, h, h, cin, 1)
-            w = torch.randn(cout, cin, 3, 3, generator=g) / math.sqrt(cin * 9)
-            plan.sd = {"bn.running_var": torch.rand(cout, generator=g) + 0.5, "bn.weight": torch.rand(cout, generator=g) + 0.5}
-            res = _rand_act(g, nb, h, h, cout, 1)
-            y, rec = plan._conv_fwd("c", x, w, 1, 1, 1, bn="bn", relu=True, res=res, want_mask=True)
-            assert plan.fwd_ops[-1].resolved_block_n() == 128
-            # its data gradient: K = 9 * 256
-            plan._alloc_ghat(rec)
-            rec.ghat.copy_(torch.randn(nb, h, h, cout, generator=g).to(plan.dt))
-            yb = torch.zeros(nb, h, h, 128, dtype=plan.dt)
-            w2 = torch.randn(cout, 128, 3, 3, generator=g) / 48
-            rec2 = type(rec)("d", w2, 1, 1, 1, (h, h), (h, h), 128)
-            rec2.ghat, rec2.ghat_map, rec2.algo_flops = rec.ghat, None, 0.0
-            plan._dgrad(rec2, y=yb, mul1=(torch.rand(nb * h * h, 128, generator=g) + 0.5).to(plan.gain_dt))
-            assert plan.bwd_ops[-1].resolved_block_n() == 128
-            ops = plan.fwd_ops + plan.bwd_ops
-            if cl == 1:
-                print(_run_and_compare(ops))
-            memo = {}
-            dops = [U.to_device(o, "cuda", memo) for o in ops]
-            for o in dops:
-                o.run()
-            torch.cuda.synchronize()
-            outs[cl] = [t.cpu() for t in (dops[0].y, dops[0].gain, dops[0].maskbits, dops[0].sq_out, dops[1].y)]
-        finally:
-            bcosk_lib.bcosk_set_cluster(prev)
-    for cl in (2, 4, 3):
-        for a, b in zip(outs[cl], outs[1]):
-            assert torch.equal(a, b), cl
-
-
-def test_launch_variants_are_bit_identical(bcosk_lib):
-    """the scheduling switches (CTAs per SM / ring slots, late input tile, programmatic dependent launch) only change
-    how tiles are scheduled: every output must be bit-identical"""
+def test_light_and_late_input_variants_are_bit_identical(bcosk_lib):
+    """the scheduling switches (CTAs per SM / ring slots, late input tile) only change how tiles are scheduled: every
+    output must be bit-identical"""
     def build():
         g = torch.Generator().manual_seed(91)
         nb, h = 4, 16
@@ -558,8 +517,8 @@ def test_launch_variants_are_bit_identical(bcosk_lib):
         plan._dgrad(rec3, y=torch.zeros(nb, h, h, 128, dtype=plan.dt), mul1=(torch.rand(M, 128, generator=g) + 0.5).to(plan.gain_dt))
         return ops + list(plan.bwd_ops)
 
-    def run(light, late, pdl):
-        prev = (bcosk_lib.bcosk_set_light(light), bcosk_lib.bcosk_set_late_input(late), bcosk_lib.bcosk_set_pdl(pdl))
+    def run(light, late):
+        prev = (bcosk_lib.bcosk_set_light(light), bcosk_lib.bcosk_set_late_input(late))
         try:
             memo = {}
             dops = [U.to_device(o, "cuda", memo) for o in build()]
@@ -571,12 +530,12 @@ def test_launch_variants_are_bit_identical(bcosk_lib):
                 outs += [t.cpu() for t in (o.y, o.gain, o.maskbits, o.sq_out, o.out2) if t is not None]
             return outs
         finally:
-            bcosk_lib.bcosk_set_light(prev[0]); bcosk_lib.bcosk_set_late_input(prev[1]); bcosk_lib.bcosk_set_pdl(prev[2])
+            bcosk_lib.bcosk_set_light(prev[0]); bcosk_lib.bcosk_set_late_input(prev[1])
 
     ref_ops = build()
     print(_run_and_compare(ref_ops))                 # default switches against the emulator
-    base = run(0, 0, 0)                              # 2 CTAs / SM everywhere, input tile parked in a ring slot
-    for cfg in ((1, 0, 0), (3, 2, 0), (3, 2, 1), (11, 2, 0), (7, 1, 0)):
+    base = run(0, 0)                                 # 2 CTAs / SM everywhere, input tile parked in a ring slot
+    for cfg in ((1, 0), (3, 2), (11, 2), (7, 1)):
         outs = run(*cfg)
         assert len(outs) == len(base)
         for a, b in zip(outs, base):
